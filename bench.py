@@ -43,6 +43,9 @@ VALID_ONLY = True
 # PRE_ROLL untimed env steps after reset() bring the batch to the stationary mix of episode phases (episodes last
 # ~5.6 steps under random play) before the W warm-up and K timed steps.
 PRE_ROLL = 32
+# --dump-outputs writes a fixed, seeded sample of the envs (all their outputs), at most this many and DUMP_BYTES in all
+DUMP_ENVS = 4096
+DUMP_BYTES = 56 << 20
 
 
 def set_workload(name: str, envs):
@@ -237,10 +240,26 @@ def run_reference_arm(args, rank: int, world: int):
 
 
 # ----------------------------------------------------------------------------- CUDA arm
-def time_env_steps(torch, m, dev, rank, world, barrier, board, n_envs, K, Wm, ring, valid_only=True):
+def dump_outputs(torch, out_dir, step_out, actions):
+    """--dump-outputs: what one step returned to its caller (obs, action mask, rewards, dones and the actions the
+    built-in policy drew) for a fixed, seeded sample of the envs, as float32 .npy files; env_index.npy (float64)
+    names the sampled envs."""
+    n = actions.shape[0]
+    per_env = 4 * (step_out.obs[0].numel() + step_out.action_mask[0].numel() + 3) + 8
+    rows = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_ENVS, DUMP_BYTES // per_env), replace=False))
+    idx = torch.from_numpy(rows).to(actions.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), rows.astype(np.float64))
+    for name, t in (("obs", step_out.obs), ("action_mask", step_out.action_mask), ("rewards", step_out.rewards),
+                    ("dones", step_out.dones), ("actions", actions)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(0, idx).float().cpu().numpy())
+
+
+def time_env_steps(torch, m, dev, rank, world, barrier, board, n_envs, K, Wm, ring, valid_only=True, dump_dir=None):
     """The device-timed leg for one board/env-count: PRE_ROLL + W untimed and K timed fused step launches (built-in
     synthetic policy), CUDA events around the K launches only; then a separate replay that measures the per-launch
     kernel time for the roofline (back to back between one event pair, and with an event pair around each launch).
+    With `dump_dir`, the outputs of the last timed step are written there (dump_outputs) before the replay.
     Returns (ms of the K timed launches, kernel ms back to back, clocks, kernel ms bracketed)."""
     h, w, mines = board
     cfg = m.EnvConfig(H=h, W=w, mine_count=mines, guarantee_safe_neighborhood=True, step_penalty=1e-4)
@@ -267,6 +286,8 @@ def time_env_steps(torch, m, dev, rank, world, barrier, board, n_envs, K, Wm, ri
     clocks = sampler.finish()          # sampled while the last launches are still executing
     barrier()
     ms_total = ev0.elapsed_time(ev1)
+    if dump_dir is not None:
+        dump_outputs(torch, dump_dir, slots[(K - 1) % ring], scratch)
     # Per-launch kernel time for the roofline, from a separate replay after the timed region: Kk launches back to back
     # between ONE event pair (launches of one stream do not overlap, so elapsed / Kk bounds the mean kernel duration
     # from above), after 5 launches that absorb the restart after the barrier.  An event pair around EACH launch adds
@@ -349,7 +370,8 @@ def run_cuda_arm(args, rank: int, world: int, local_rank: int):
 
     Ke = min(K, 400)                           # steps replayed by the e2e legs
     ms_total, ms_kernel, clocks, ms_kernel_bracketed = time_env_steps(torch, m, dev, rank, world, barrier, (H, W, MINES),
-                                                                      N, K, Wm, ring, VALID_ONLY)
+                                                                      N, K, Wm, ring, VALID_ONLY,
+                                                                      args.dump_outputs if rank == 0 else None)
     # The actions the e2e legs replay are recorded in a separate untimed pass over the same deterministic trajectory
     # (recording inside the timed launches costs 3 us per launch: 65,536 four-byte stores into a row of device memory
     # that is cold every step, against a scratch row that stays in L2).
@@ -731,7 +753,11 @@ def main():
     ap.add_argument("--no-rollout", action="store_true")
     ap.add_argument("--no-c4", action="store_true")
     ap.add_argument("--no-train", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (a fixed, seeded sample of the envs) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     set_workload(args.workload, args.envs)
     global VALID_ONLY

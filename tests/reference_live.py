@@ -33,12 +33,13 @@ def available() -> bool:
     return os.path.isfile(os.path.join(REF_DIR, "minesweeper", "env.py"))
 
 
+SKIP_REASON = (f"the reference is not installed at {REF_DIR} (tools/install_reference.sh <checkout>); "
+               "it is not part of this repository")
+
+
 def require():
-    """The live-reference tests fail loudly (they do not skip) when the install is missing."""
     if not available():
-        raise RuntimeError(
-            f"{REF_DIR} is missing: run tools/install_reference.sh in the authoring container (it is run by "
-            "__graft_entry__.build()); baseline/_ref is git-ignored but ships to the GPU box with the tree")
+        raise RuntimeError(f"{REF_DIR} is missing: install the reference with tools/install_reference.sh <checkout>")
 
 
 def load() -> Dict[str, object]:

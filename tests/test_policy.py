@@ -1,13 +1,14 @@
 """The policy modules stay PyTorch (SURVEY section 2); this only checks that they are
 state_dict-compatible with, and numerically identical to, the reference modules when the
-reference tree is present (authoring container)."""
-import os
+reference is installed (tools/install_reference.sh)."""
 import sys
 
 import pytest
 import torch
 
-REF = "/root/reference"
+import reference_live as RL
+
+REF = RL.REF_DIR
 
 
 def test_build_model_shapes_and_param_count():
@@ -21,7 +22,7 @@ def test_build_model_shapes_and_param_count():
         m.build_model("nope", obs_shape=(10, 8, 8))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present on this box")
+@pytest.mark.skipif(not RL.available(), reason=RL.SKIP_REASON)
 @pytest.mark.parametrize("name,cfg,shape", [
     ("cnn_residual", dict(stem_channels=96, blocks=5, dropout=0.05, value_hidden=256), (10, 16, 16)),
     ("cnn", dict(hidden=64), (10, 8, 8)),

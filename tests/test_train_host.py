@@ -12,9 +12,10 @@ import torch.multiprocessing as mp
 
 from minesweeper_ppo_b200 import train as T
 from minesweeper_ppo_b200.policy import build_model
+import reference_live as RL
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = RL.REF_DIR
 
 
 def test_load_config_medium_yaml():
@@ -39,7 +40,7 @@ def _batch(n=64, seed=0):
         mine_valid=torch.rand((n, 8, 8), generator=g) < 0.7)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present on this box")
+@pytest.mark.skipif(not RL.available(), reason=RL.SKIP_REASON)
 def test_ppo_update_matches_reference_cpu():
     sys.path.insert(0, REF)
     try:
