@@ -226,6 +226,65 @@ int msw_masked_sample(const void *logits, int32_t logits_dtype, uint8_t *mask,
                       const uint32_t *epoch, int64_t row_id_base, int64_t *actions64,
                       int32_t *actions32, float *logp, void *stream);
 
+/* Greedy action of the evaluator (eval.py:330-340): actions[r] = the argmax of
+ * logits.masked_fill(~mask, -1e9) over row r of fp32 logits [n][A], exactly as
+ * torch's argmax picks it -- masked cells compete at -1e9, ties go to the first
+ * index, a NaN wins (the first NaN).  `mask` (bool [n][A]) is in/out for one
+ * case only: a row without any legal action is made all-legal first (the guard
+ * of eval.py:336-338).  One warp per row. */
+int msw_masked_argmax(const float *logits, uint8_t *mask, int64_t n, int32_t A,
+                      int32_t *actions, void *stream);
+
+/* Episode accounting of eval.evaluate_vec (eval.py:350-428) on the device, as
+ * two launches around msw_step.  `counters` is int64 [MSW_EVAL_COUNTERS]
+ * (zero, except MSW_EVAL_ERROR_KEY = INT64_MAX, at the start of an evaluation);
+ * updates are integer atomics, so the totals do not depend on the order. */
+enum {
+    /* msw_eval_pre_step */
+    MSW_EVAL_INVALID = 0,              /* picks outside the mask, over all n envs */
+    MSW_EVAL_FORCED_STEPS, MSW_EVAL_FORCED_CORRECT,      /* chosen cell in subset_reveal */
+    MSW_EVAL_GUESS_ATTEMPTS, MSW_EVAL_GUESS_SUCCESS,     /* chosen cell not in it */
+    MSW_EVAL_REVEAL_TOTAL,             /* analysed envs with first_click_done */
+    MSW_EVAL_FORCED_GUESS_TOTAL, MSW_EVAL_FORCED_GUESS_SUCCESS,
+    MSW_EVAL_SAFE_OPTION_TOTAL, MSW_EVAL_SAFE_OPTION_HITS, MSW_EVAL_SAFE_OPTION_MISSES,
+    MSW_EVAL_SAFE_CELLS,               /* sum of count_forced_safe_cells */
+    MSW_EVAL_COMP_SIZE_SUM, MSW_EVAL_COMP_COUNT,         /* component_sizes */
+    MSW_EVAL_CHOSEN_SIZE_SUM, MSW_EVAL_CHOSEN_COUNT,     /* chosen_component_size */
+    MSW_EVAL_PRE_COUNTERS,
+    /* msw_eval_post_step */
+    MSW_EVAL_WINS = MSW_EVAL_PRE_COUNTERS, MSW_EVAL_TOTAL_STEPS,
+    MSW_EVAL_NEW_REVEALS,              /* sum of last_new_reveals of uncounted envs */
+    MSW_EVAL_FORCED_GUESS_EPISODES,
+    /* smallest step_index * n + env of an analysed env whose msw_avoidability
+     * flag bit 3 (search budget exceeded) was set; INT64_MAX if none */
+    MSW_EVAL_ERROR_KEY,
+    MSW_EVAL_COUNTERS
+};
+
+/* Before msw_step, on the state the actions were chosen on: for every env, an
+ * invalid pick (mask[i][actions[i]] == 0) is counted; envs with counted[i] == 0
+ * and i < batch_size are analysed -- the `safe` test on the mines, subset-rule
+ * hit or guess from msw_forced_subset's subset_bits, and, when
+ * first_click_done, the avoidability bookkeeping of avoidability.py:41-49 from
+ * msw_avoidability's arrays (safe_bits, comp_of_cell, comp_size, avoid_flags),
+ * which sets ep_unavoidable[i] for a forced guess.  belief_sel (nullable, u8
+ * [n][H*W]) is rewritten whole: 1 + mine for each unknown (not revealed, not
+ * flagged) cell of an analysed env, 0 elsewhere. */
+int msw_eval_pre_step(const msw_env_desc *desc, const msw_state *st, int64_t n, int64_t batch_size,
+                      const int32_t *actions, const uint8_t *mask, const uint32_t *subset_bits,
+                      const uint32_t *safe_bits, const int16_t *comp_of_cell, const int16_t *comp_size,
+                      const uint8_t *avoid_flags, const uint8_t *counted, uint8_t *ep_unavoidable,
+                      uint8_t *belief_sel, int64_t *counters, int64_t step_index, void *stream);
+
+/* After msw_step, over all n envs (eval.py:405-428): step_counter[i] += 1; an
+ * uncounted env adds its last_new_reveals; an uncounted env that is done (or,
+ * when max_steps > 0, has reached max_steps) adds its steps (and, if done, its
+ * win and ep_unavoidable), resets its step counter, becomes counted and adds 1
+ * to *finished. */
+int msw_eval_post_step(int64_t n, const uint8_t *done, const int8_t *outcome, const int32_t *new_reveals,
+                       uint8_t *counted, int32_t *step_counter, const uint8_t *ep_unavoidable,
+                       int32_t max_steps, int64_t *counters, int32_t *finished, void *stream);
+
 /* Fused GroupNorm + (fp32 residual add) + ReLU + Dropout2d between the cuDNN
  * convolutions of the rollout forward (SURVEY section 8 row f4; replaces the
  * eager norm/act/dropout/add/cast kernels of cnn_residual.py:17-27, 50-54

@@ -87,7 +87,19 @@ SIGNATURES = {
     "msw_forced_subset": (C.c_int, [_P(EnvDesc), _P(State), C.c_int64, C.c_void_p, C.c_void_p]),
     "msw_avoidability": (C.c_int, [_P(EnvDesc), _P(State), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_uint32, C.c_void_p]),
+    "msw_masked_argmax": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
+    "msw_eval_pre_step": (C.c_int, [_P(EnvDesc), _P(State), C.c_int64, C.c_int64] + [C.c_void_p] * 11
+                          + [C.c_int64, C.c_void_p]),
+    "msw_eval_post_step": (C.c_int, [C.c_int64] + [C.c_void_p] * 6 + [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
 }
+
+# int64 counter slots of msw_eval_pre_step / msw_eval_post_step (enum in include/msw_b200.h)
+EVAL_COUNTERS = (
+    "invalid", "forced_steps", "forced_correct", "guess_attempts", "guess_success", "reveal_total",
+    "forced_guess_total", "forced_guess_success", "safe_option_total", "safe_option_hits", "safe_option_misses",
+    "safe_cells", "comp_size_sum", "comp_count", "chosen_size_sum", "chosen_count",
+    "wins", "total_steps", "new_reveals", "forced_guess_episodes", "error_key",
+)
 
 _lib = None
 

@@ -461,9 +461,7 @@ class VecMinesweeper:
         u = self._unpacked()
         if "subset" not in u:
             bits = torch.empty((self.num_envs, self.wpb), dtype=torch.int32, device=self.device)
-            with torch.cuda.device(self.device):
-                _lib.check(self._L.msw_forced_subset(C.byref(self._desc), C.byref(self._state), self.num_envs,
-                                                     bits.data_ptr(), self._stream()), "msw_forced_subset")
+            self._launch_forced_subset(bits)
             raw = bits.cpu().numpy().view(np.uint8).reshape(self.num_envs, -1)
             u["subset"] = np.unpackbits(raw, axis=1, count=self.HW, bitorder="little").astype(bool)
         return u["subset"]
@@ -479,14 +477,32 @@ class VecMinesweeper:
             coc = torch.empty((n, HW), dtype=torch.int16, device=dev)
             cs = torch.empty((n, HW), dtype=torch.int16, device=dev)
             fl = torch.empty((n,), dtype=torch.uint8, device=dev)
-            with torch.cuda.device(dev):
-                _lib.check(self._L.msw_avoidability(C.byref(self._desc), C.byref(self._state), n, bits.data_ptr(),
-                                                    coc.data_ptr(), cs.data_ptr(), fl.data_ptr(),
-                                                    int(search_budget) & 0xFFFFFFFF, self._stream()), "msw_avoidability")
+            self._launch_avoidability(bits, coc, cs, fl, search_budget)
             raw = bits.cpu().numpy().view(np.uint8).reshape(n, -1)
             u["avoid"] = {"safe": np.unpackbits(raw, axis=1, count=HW, bitorder="little").astype(bool),
                           "comp_of_cell": coc.cpu().numpy(), "comp_size": cs.cpu().numpy(), "flags": fl.cpu().numpy()}
         return u["avoid"]
+
+    # device halves of forced_subset() / avoidability(): fill caller-owned device buffers, no host copy, no cache
+    def _launch_forced_subset(self, bits: torch.Tensor) -> None:
+        """msw_forced_subset into int32 [n, wpb] `bits`."""
+        self._check(bits, (self.num_envs, self.wpb), torch.int32, "subset bits")
+        with torch.cuda.device(self.device):
+            _lib.check(self._L.msw_forced_subset(C.byref(self._desc), C.byref(self._state), self.num_envs,
+                                                 bits.data_ptr(), self._stream()), "msw_forced_subset")
+
+    def _launch_avoidability(self, bits: torch.Tensor, coc: torch.Tensor, cs: torch.Tensor, fl: torch.Tensor,
+                             search_budget: int = 0) -> None:
+        """msw_avoidability into int32 [n, wpb] `bits`, int16 [n, HW] `coc` / `cs` and uint8 [n] `fl`."""
+        n, HW = self.num_envs, self.HW
+        self._check(bits, (n, self.wpb), torch.int32, "safe bits")
+        self._check(coc, (n, HW), torch.int16, "comp_of_cell")
+        self._check(cs, (n, HW), torch.int16, "comp_size")
+        self._check(fl, (n,), torch.uint8, "avoid flags")
+        with torch.cuda.device(self.device):
+            _lib.check(self._L.msw_avoidability(C.byref(self._desc), C.byref(self._state), n, bits.data_ptr(),
+                                                coc.data_ptr(), cs.data_ptr(), fl.data_ptr(),
+                                                int(search_budget) & 0xFFFFFFFF, self._stream()), "msw_avoidability")
 
     def random_actions(self, step_index: int, valid_only: bool = True, seed: int = 1,
                        out: Optional[torch.Tensor] = None) -> torch.Tensor:

@@ -11,16 +11,22 @@ with the reference's episode accounting (only the first finished episode per env
 eval.py:411-428).  Returns the reference's metric dict, key for key.  `tests/golden/c1_eval.npz` holds
 the dict the unmodified reference produced for a scripted policy; `test_eval_matches_reference_metrics`
 replays the same mine layouts through this function on the CUDA env and compares.
+
+`evaluate_vec_device` returns the same dict with nothing per env crossing the bus: greedy action
+(msw_masked_argmax), both analytics and the episode accounting (msw_eval_pre_step / msw_eval_post_step) run
+on the device, and one 4-byte `finished` count is read back per step (DESIGN.md section 4.9).
 """
 from __future__ import annotations
 
+import ctypes as C
 from typing import Callable, Dict, List, Optional
 
 import numpy as np
 import torch
 
+from . import _lib
 from .avoidability import analyze_avoidability
-from .env import EnvConfig, VecMinesweeper
+from .env import EnvConfig, StepOut, VecMinesweeper
 from .rules import analyze_forced_modules
 
 
@@ -175,4 +181,201 @@ def evaluate_vec(model: torch.nn.Module, env_cfg: EnvConfig, episodes: int = 100
         "forced_step_rate": forced_steps / max(1, forced_steps + guess_attempts),
         "forced_step_accuracy": forced_correct / max(1, forced_steps),
         "guess_success_rate": guess_success / max(1, guess_attempts),
+    }
+
+
+def masked_argmax(logits: torch.Tensor, mask: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """int32 `logits.masked_fill(~mask, -1e9).argmax(-1)` of fp32 [n, A] logits in one launch (msw_masked_argmax),
+    torch's tie and NaN rules included.  A row of `mask` without a legal action is made all-legal in place first."""
+    if logits.device.type != "cuda":
+        raise RuntimeError("masked_argmax runs on CUDA only (no CPU fallback in this package)")
+    n, A = logits.shape
+    if logits.dtype != torch.float32 or not logits.is_contiguous():
+        raise ValueError("masked_argmax: logits must be a contiguous float32 [n, A] tensor")
+    if mask.dtype != torch.bool or tuple(mask.shape) != (n, A) or not mask.is_contiguous() or mask.device != logits.device:
+        raise ValueError("masked_argmax: mask must be a contiguous bool [n, A] tensor on the logits device")
+    if out is None:
+        out = torch.empty((n,), dtype=torch.int32, device=logits.device)
+    if out.dtype != torch.int32 or tuple(out.shape) != (n,) or not out.is_contiguous() or out.device != logits.device:
+        raise ValueError("masked_argmax: out must be a contiguous int32 [n] tensor on the logits device")
+    with torch.cuda.device(logits.device):
+        _lib.check(_lib.load().msw_masked_argmax(logits.data_ptr(), mask.data_ptr(), n, A, out.data_ptr(),
+                                                 torch.cuda.current_stream().cuda_stream), "msw_masked_argmax")
+    return out
+
+
+_K = {name: k for k, name in enumerate(_lib.EVAL_COUNTERS)}
+_INT64_MAX = (1 << 63) - 1
+
+
+class _DeviceEvaluator:
+    """State and per-step phases of `evaluate_vec_device`; every buffer is allocated once.  The phases are methods
+    so that tools/eval_probe.py can time them one by one with CUDA events."""
+
+    def __init__(self, model: torch.nn.Module, vec: VecMinesweeper, search_budget: int, max_steps: int):
+        self.model, self.vec = model, vec
+        self.search_budget, self.max_steps = int(search_budget), int(max_steps)
+        n, HW, wpb, dev = vec.num_envs, vec.HW, vec.wpb, vec.device
+        z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=dev)
+        self.out = StepOut(obs=z((n, _lib.OBS_CHANNELS, vec.H, vec.W), torch.float32), action_mask=z((n, HW), torch.bool),
+                           rewards=z((n,), torch.float32), dones=z((n,), torch.bool))
+        self.actions = z((n,), torch.int32)
+        self.subset = z((n, wpb), torch.int32)
+        self.safe, self.coc, self.cs = z((n, wpb), torch.int32), z((n, HW), torch.int16), z((n, HW), torch.int16)
+        self.avoid_flags = z((n,), torch.uint8)
+        self.counted, self.ep_unavoidable = z((n,), torch.uint8), z((n,), torch.uint8)
+        self.step_counter = z((n,), torch.int32)
+        self.sel, self.sel_mask = z((n, HW), torch.uint8), z((n, HW), torch.bool)
+        self.prob: Optional[torch.Tensor] = None
+        self.counters = z((len(_lib.EVAL_COUNTERS),), torch.int64)
+        self.counters[_K["error_key"]] = _INT64_MAX
+        self.finished = z((1,), torch.int32)
+        self.finished_host = torch.zeros((1,), dtype=torch.int32).pin_memory()
+        self.probs: List[torch.Tensor] = []
+        self.labels: List[torch.Tensor] = []
+        self.step_index = 0
+        self.infos: Dict[str, torch.Tensor] = {}
+        self.mine_logits: Optional[torch.Tensor] = None
+        self.logits: Optional[torch.Tensor] = None
+        vec.reset(out=self.out)
+
+    def new_batch(self) -> None:
+        for t in (self.counted, self.ep_unavoidable, self.step_counter, self.finished):
+            t.zero_()
+
+    def forward(self) -> None:
+        logits, _, mine_logits = self.model(self.out.obs, return_mine=True)   # fp32, no autocast (eval.py:333)
+        n, HW = self.vec.num_envs, self.vec.HW
+        assert logits.shape[1] == self.out.action_mask.shape[1] == HW          # eval.py:22-27
+        if logits.dtype != torch.float32:
+            raise TypeError(f"evaluate_vec_device: the policy returned {logits.dtype} logits; it needs an fp32 forward")
+        self.logits, self.mine_logits = logits.contiguous(), mine_logits
+
+    def act(self) -> None:
+        masked_argmax(self.logits, self.out.action_mask, out=self.actions)
+
+    def analytics(self) -> None:
+        self.vec._launch_forced_subset(self.subset)
+        self.vec._launch_avoidability(self.safe, self.coc, self.cs, self.avoid_flags, self.search_budget)
+
+    def account_pre(self, batch_size: int) -> None:
+        vec, n, HW = self.vec, self.vec.num_envs, self.vec.HW
+        belief = self.mine_logits is not None
+        if belief:
+            if self.prob is None:
+                self.prob = torch.empty((n, HW), dtype=torch.float32, device=vec.device)
+            torch.sigmoid(self.mine_logits.reshape(n, HW), out=self.prob)
+        with torch.cuda.device(vec.device):
+            _lib.check(vec._L.msw_eval_pre_step(
+                C.byref(vec._desc), C.byref(vec._state), n, int(batch_size), self.actions.data_ptr(),
+                self.out.action_mask.data_ptr(), self.subset.data_ptr(), self.safe.data_ptr(), self.coc.data_ptr(),
+                self.cs.data_ptr(), self.avoid_flags.data_ptr(), self.counted.data_ptr(), self.ep_unavoidable.data_ptr(),
+                self.sel.data_ptr() if belief else None, self.counters.data_ptr(), self.step_index, vec._stream()),
+                "msw_eval_pre_step")
+        if belief:      # the reference's order: step, env, cell in row-major order (eval.py:352-358)
+            torch.ne(self.sel, 0, out=self.sel_mask)
+            self.probs.append(self.prob.masked_select(self.sel_mask))
+            self.labels.append(self.sel.masked_select(self.sel_mask))
+
+    def step(self) -> None:
+        _, _, _, self.infos = self.vec.step(self.actions, out=self.out, want_infos=True)
+
+    def account_post(self) -> int:
+        vec, it = self.vec, self.infos
+        with torch.cuda.device(vec.device):
+            _lib.check(vec._L.msw_eval_post_step(
+                vec.num_envs, self.out.dones.data_ptr(), it["outcome_code"].data_ptr(), it["last_new_reveals"].data_ptr(),
+                self.counted.data_ptr(), self.step_counter.data_ptr(), self.ep_unavoidable.data_ptr(), self.max_steps,
+                self.counters.data_ptr(), self.finished.data_ptr(), vec._stream()), "msw_eval_post_step")
+        self.step_index += 1
+        self.finished_host.copy_(self.finished, non_blocking=True)
+        torch.cuda.current_stream(vec.device).synchronize()
+        return int(self.finished_host[0])
+
+    def run_step(self, batch_size: int) -> int:
+        self.forward()
+        self.act()
+        self.analytics()
+        self.account_pre(batch_size)
+        self.step()
+        return self.account_post()
+
+    def check_budget(self) -> None:
+        key = int(self.counters[_K["error_key"]])
+        if key != _INT64_MAX:
+            n = self.vec.num_envs
+            raise RuntimeError(f"evaluate_vec_device: exact search of env {key % n} exceeded its step budget at "
+                               f"evaluation step {key // n}; pass a larger search_budget")
+
+    def belief_pairs(self):
+        """(probabilities f32, labels f32) of every belief pair, copied to the host once."""
+        if not self.probs:
+            return np.zeros(0), np.zeros(0)
+        p = torch.cat(self.probs).cpu().numpy()
+        y = (torch.cat(self.labels) - 1).cpu().numpy().astype(np.float32)
+        return p, y
+
+
+@torch.no_grad()
+def evaluate_vec_device(model: torch.nn.Module, env_cfg: EnvConfig, episodes: int = 1000, seed: int = 0,
+                        num_envs: int = 256, max_steps_per_episode: int = 512,
+                        vec_factory: Optional[Callable[..., VecMinesweeper]] = None,
+                        search_budget: int = 0) -> Dict[str, float]:
+    """`evaluate_vec` with the per-env work on the device: the same metric dict, key for key.
+
+    `vec_factory(num_envs=, cfg=, seed=, api="torch")` builds the env (default VecMinesweeper); `search_budget` is
+    msw_avoidability's per-lane step budget (0 = its default), and an analysed env that exceeds it raises
+    RuntimeError, as `analyze_avoidability` does.  `avg_progress` agrees with `evaluate_vec` to float64 summation
+    order (DESIGN.md section 4.9); every other key is equal."""
+    device = next(model.parameters()).device
+    was_training = model.training
+    model.eval()                                                          # eval.py:278-279
+    vec = (vec_factory or VecMinesweeper)(num_envs=num_envs, cfg=env_cfg, seed=seed, api="torch")
+    if vec.device != device:
+        raise ValueError(f"evaluate_vec_device: model on {device}, env on {vec.device}")
+    ev = _DeviceEvaluator(model, vec, search_budget, max_steps_per_episode)
+    remaining = episodes
+    try:
+        while remaining > 0:
+            batch_size = min(vec.num_envs, remaining)
+            ev.new_batch()
+            finished = 0
+            while finished < batch_size:
+                finished = ev.run_step(batch_size)
+            ev.check_budget()
+            remaining -= batch_size
+    finally:
+        if was_training:
+            model.train()
+    c = {k: int(v) for k, v in zip(_lib.EVAL_COUNTERS, ev.counters.cpu().tolist())}
+    p, y = ev.belief_pairs()
+    return _device_metrics(c, p, y, episodes, vec.HW)
+
+
+def _device_metrics(c: Dict[str, int], p: np.ndarray, y: np.ndarray, episodes: int, HW: int) -> Dict[str, float]:
+    """The dict of evaluate_vec (eval.py:490-510) from the device counters and the belief pairs."""
+    wins, total_steps = c["wins"], c["total_steps"]
+    ci_low, ci_high = _wilson(wins, max(1, episodes))
+    reveal_den = float(max(1, c["reveal_total"]))
+    forced_steps, guess_attempts = c["forced_steps"], c["guess_attempts"]
+    return {
+        "win_rate": wins / max(1, episodes), "win_ci_low": ci_low, "win_ci_high": ci_high,
+        "avg_steps": total_steps / max(1, episodes),
+        "avg_progress": c["new_reveals"] / float(HW) / max(1, episodes),
+        "invalid_rate": c["invalid"] / max(1, total_steps),
+        "forced_guess_rate": c["forced_guess_total"] / reveal_den,
+        "forced_guess_success_rate": _ratio(c["forced_guess_success"], c["forced_guess_total"]),
+        "forced_guess_episode_rate": c["forced_guess_episodes"] / float(max(1, episodes)),
+        "safe_option_rate": c["safe_option_total"] / reveal_den,
+        "safe_option_miss_rate": _ratio(c["safe_option_misses"], c["safe_option_total"]),
+        "safe_option_pick_rate": _ratio(c["safe_option_hits"], c["safe_option_total"]),
+        "avg_safe_options_per_turn": _ratio(c["safe_cells"], c["safe_option_total"]),
+        "avg_frontier_component_size": _ratio(float(c["comp_size_sum"]), c["comp_count"]),
+        "avg_selected_component_size": _ratio(float(c["chosen_size_sum"]), c["chosen_count"]),
+        "belief_auroc": _auroc(y, p) if len(p) else float("nan"),
+        "belief_ece": _ece(p, y) if len(p) else float("nan"),
+        "wins": float(wins), "episodes": float(episodes),
+        "forced_step_rate": forced_steps / max(1, forced_steps + guess_attempts),
+        "forced_step_accuracy": c["forced_correct"] / max(1, forced_steps),
+        "guess_success_rate": c["guess_success"] / max(1, guess_attempts),
     }
