@@ -1,6 +1,8 @@
-// msw_capi.cu -- version / error entry points of the C ABI (include/msw_b200.h).
+// msw_capi.cu -- version / error entry points of the C ABI (include/msw_b200.h), and the host helpers the
+// kernels' launchers share (SM count, tensor-map encoder).
 #include "../../include/msw_b200.h"
 #include "msw_error.h"
+#include "msw_sm100.cuh"
 
 #include <execinfo.h>
 #include <signal.h>
@@ -40,6 +42,36 @@ int sm_count()
         cached_sms = sms;
     }
     return cached_sms;
+}
+
+typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
+                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+static EncodeTiledFn encode_tiled_fn()
+{
+    static const EncodeTiledFn fn = [] {
+        void *p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
+            q != cudaDriverEntryPointSuccess)
+            p = nullptr;
+        return reinterpret_cast<EncodeTiledFn>(p);
+    }();
+    return fn;
+}
+
+bool tensor_map_encoder_available() { return encode_tiled_fn() != nullptr; }
+
+CUresult encode_tiled(CUtensorMap *map, CUtensorMapDataType dtype, cuuint32_t rank, const void *base,
+                      const cuuint64_t *dims, const cuuint64_t *strides, const cuuint32_t *box,
+                      CUtensorMapSwizzle swizzle)
+{
+    static const cuuint32_t elem_strides[5] = {1, 1, 1, 1, 1};     // rank <= 5
+    const EncodeTiledFn fn = encode_tiled_fn();
+    if (!fn) return CUDA_ERROR_NOT_SUPPORTED;
+    return fn(map, dtype, rank, const_cast<void *>(base), dims, strides, box, elem_strides, CU_TENSOR_MAP_INTERLEAVE_NONE,
+              swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
 }
 
 }  // namespace msw

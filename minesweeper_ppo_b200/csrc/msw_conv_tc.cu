@@ -19,10 +19,12 @@
 // the activation streams through a 2-stage ring.  K = 96 = one 64-channel block (128-byte swizzle) + one
 // 32-channel block (64-byte swizzle).  Roles: warp 0 TMA producer, warp 1 MMA issuer (54 tcgen05.mma of
 // 128 x 96 x 16 per tile into a ring of four 96-column accumulators), warp 2 TMEM allocation, warps 4-15
-// epilogue (thread = pixel, each warpgroup a third of the channels).
+// epilogue (thread = pixel, each warpgroup a third of the channels).  The mbarrier / TMA / tcgen05 wrappers are in
+// msw_sm100.cuh.
 #include "../../include/msw_b200.h"
 #include "msw_common.cuh"
 #include "msw_error.h"
+#include "msw_sm100.cuh"
 
 #include <cuda.h>
 #include <cuda_fp16.h>
@@ -92,75 +94,6 @@ __device__ __forceinline__ long long cv_p8(long long board, int half, int third,
     return ((((board * 2 + half) * 3 + third) * 4 + c4) * 128 + pp) * 8;
 }
 
-__device__ __forceinline__ unsigned cv_smem(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void cv_bar_init(unsigned bar, unsigned count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(bar), "r"(count));
-}
-__device__ __forceinline__ void cv_bar_expect(unsigned bar, unsigned bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void cv_bar_arrive(unsigned bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(bar) : "memory");
-}
-__device__ __forceinline__ void cv_bar_wait(unsigned bar, unsigned parity)
-{
-    unsigned done = 0;
-    while (!done)
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void cv_tma_2d(unsigned dst, const CUtensorMap *map, int c0, int c1, unsigned bar)
-{
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                 :: "r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void cv_tma_4d(unsigned dst, const CUtensorMap *map, int c0, int c1, int c2, int c3, unsigned bar)
-{
-    asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
-                 :: "r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(bar) : "memory");
-}
-// One lane of a converged warp.  ptxas knows that code guarded by elect.sync runs on exactly one thread, so the
-// tcgen05 / TMA instructions inside take their uniform-register operands directly; guarded by `lane == 0` instead,
-// every such instruction is wrapped in a divergence "waterfall" loop (ELECT / PLOP3 / BRA.U.ANY, ~10 dependent
-// instructions per MMA).  Measured in round 2: the whole forward 4.04 -> 3.99 ms.
-__device__ __forceinline__ bool cv_elect_one()
-{
-    unsigned pred;
-    asm volatile("{ .reg .pred p; elect.sync _|p, 0xffffffff; selp.u32 %0, 1, 0, p; }" : "=r"(pred));
-    return pred != 0u;
-}
-
-// K-major operand descriptor (sm_100 version bit, LBO unused = 1, matrix base offset 0) for rows of ROW bytes:
-// 8-row groups ROW * 8 bytes apart (SBO); ROW = 128 / 64 / 32 <-> layout type SWIZZLE_128B (2) / 64B (4) / 32B (6).
-template <unsigned ROW>
-__device__ __forceinline__ uint64_t cv_desc(unsigned addr)
-{
-    constexpr uint64_t layout = ROW == 128 ? 2ull : ROW == 64 ? 4ull : 6ull;
-    return (uint64_t)((addr >> 4) & 0x3FFFu) | (1ull << 16) | ((uint64_t)(ROW * 8u >> 4) << 32) | (1ull << 46) | (layout << 61);
-}
-// D[tmem] (+)= A[smem] . B[smem]^T, issued by one thread; bit i of mask word w set = row 32w + i of D is not
-// written (disable-output-lane)
-__device__ __forceinline__ void cv_mma_masked(unsigned d_tmem, uint64_t a, uint64_t b, unsigned idesc, unsigned accumulate,
-                                              unsigned mask)
-{
-    asm volatile("{ .reg .pred p; setp.ne.b32 p, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, {%5, %5, %5, %5}, p; }"
-                 :: "r"(d_tmem), "l"(a), "l"(b), "r"(idesc), "r"(accumulate), "r"(mask) : "memory");
-}
-__device__ __forceinline__ void cv_commit(unsigned bar)
-{
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(bar) : "memory");
-}
-__device__ __forceinline__ void cv_ld16(unsigned taddr, uint32_t (&v)[16])
-{
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                   "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                 : "r"(taddr) : "memory");
-}
-
 __device__ __forceinline__ void cv_st256(void *p, const uint32_t (&v)[8])
 {
     asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
@@ -195,8 +128,8 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
                        OFF_PART = K::OFF_PART, OFF_CB = K::OFF_CB, OFF_AB = K::OFF_AB, W0_TAP = K::W0_TAP, W1_TAP = K::W1_TAP,
                        A0_BYTES = K::A0_BYTES, A_STAGE = K::A_STAGE;
     extern __shared__ unsigned char smem_dyn[];
-    const unsigned base = (cv_smem(smem_dyn) + 1023u) & ~1023u;
-    unsigned char *gen = smem_dyn + (base - cv_smem(smem_dyn));
+    const unsigned base = (smem_u32(smem_dyn) + 1023u) & ~1023u;
+    unsigned char *gen = smem_dyn + (base - smem_u32(smem_dyn));
     const unsigned bars = base + OFF_BAR;
     auto full = [&](int s) { return bars + 8u * s; };
     auto empty = [&](int s) { return bars + 8u * (2 + s); };
@@ -207,28 +140,24 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (tid == 0) {
-        for (int s = 0; s < STAGES; ++s) { cv_bar_init(full(s), 1); cv_bar_init(empty(s), 1); }
-        for (unsigned a = 0; a < ACC; ++a) { cv_bar_init(tfull(a), 1); cv_bar_init(tempty(a), 12); }
-        cv_bar_init(wfull, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (int s = 0; s < STAGES; ++s) { mbar_init(full(s), 1); mbar_init(empty(s), 1); }
+        for (unsigned a = 0; a < ACC; ++a) { mbar_init(tfull(a), 1); mbar_init(tempty(a), 12); }
+        mbar_init(wfull, 1);
+        mbar_fence_init();
     }
-    if (warp == 2) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     :: "r"(base + OFF_TMEM), "r"((unsigned)TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    if (warp == 2) tmem_alloc(base + OFF_TMEM, TMEM_COLS);
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const unsigned tmem = *s_tmem;
 
     if (warp == 0) {
-        if (cv_elect_one()) {
+        if (elect_one()) {
         // ---- TMA producer: the nine weight taps once, then one [10 rows x 16 px x 96 ch] block per tile
-        cv_bar_expect(wfull, K::W0_BYTES + K::W1_BYTES);
+        mbar_expect_tx(wfull, K::W0_BYTES + K::W1_BYTES);
         for (int t = 0; t < 9; ++t) {
-            cv_tma_2d(base + OFF_W0 + t * W0_TAP, &map_w0, 0, t * C, wfull);
-            if (K::KS1) cv_tma_2d(base + OFF_W1 + t * W1_TAP, &map_w1, K::BOX0, t * C, wfull);
+            tma_load_2d(base + OFF_W0 + t * W0_TAP, &map_w0, 0, t * C, wfull);
+            if (K::KS1) tma_load_2d(base + OFF_W1 + t * W1_TAP, &map_w1, K::BOX0, t * C, wfull);
         }
         // a CTA takes whole boards: tiles 2*board, 2*board + 1 back to back (the GN epilogue needs both)
         for (unsigned it = 0;; ++it) {
@@ -236,24 +165,24 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
             if (board >= boards) break;
             const unsigned s = it % STAGES, ph = (it / STAGES) & 1u;
             const int n = (int)board, y0 = (int)(it & 1u) * 8;
-            cv_bar_wait(empty(s), ph ^ 1u);
-            cv_bar_expect(full(s), A_STAGE);
-            cv_tma_4d(base + OFF_A + s * A_STAGE, &map_a0, 0, 0, y0 - 1, n, full(s));
-            if (K::KS1) cv_tma_4d(base + OFF_A + s * A_STAGE + A0_BYTES, &map_a1, K::BOX0, 0, y0 - 1, n, full(s));
+            mbar_wait(empty(s), ph ^ 1u);
+            mbar_expect_tx(full(s), A_STAGE);
+            tma_load_4d(base + OFF_A + s * A_STAGE, &map_a0, 0, 0, y0 - 1, n, full(s));
+            if (K::KS1) tma_load_4d(base + OFF_A + s * A_STAGE + A0_BYTES, &map_a1, K::BOX0, 0, y0 - 1, n, full(s));
         }
         }
     } else if (warp == 1) {
         // ---- MMA issuer.  idesc: D = F32, A = B = F16, K-major, M = 128, N = 96.
         constexpr unsigned idesc = (1u << 4) | ((unsigned)(C >> 3) << 17) | ((unsigned)(TILE_PX >> 4) << 24);
-        cv_bar_wait(wfull, 0);
+        mbar_wait(wfull, 0);
         for (unsigned it = 0;; ++it) {
             if (blockIdx.x + (long long)(it >> 1) * gridDim.x >= boards) break;
             const unsigned s = it % STAGES, ph = (it / STAGES) & 1u, acc = it % ACC, aph = (it / ACC) & 1u;
-            cv_bar_wait(tempty(acc), aph ^ 1u);                   // the epilogue has drained this accumulator
-            cv_bar_wait(full(s), ph);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            mbar_wait(tempty(acc), aph ^ 1u);                     // the epilogue has drained this accumulator
+            mbar_wait(full(s), ph);
+            tcgen05_fence_after();
             const unsigned a0 = base + OFF_A + s * A_STAGE, a1 = a0 + A0_BYTES, d = tmem + acc * C;
-            if (cv_elect_one()) {            // the whole warp runs the loop and the waits; one elected lane issues
+            if (elect_one()) {            // the whole warp runs the loop and the waits; one elected lane issues
             unsigned accumulate = 0u;
             if (!MSW_DBG(8))
 #pragma unroll
@@ -268,19 +197,19 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
                     const unsigned sa1 = a1 + (unsigned)((dy * HW_W + dxi - 1) * (int)K::ROW1);
 #pragma unroll
                     for (int k = 0; k < K::KS0; ++k) {                       // first channel block, 16 channels (32 bytes) per step
-                        cv_mma_masked(d, cv_desc<K::ROW0>(sa0) + 2u * k, cv_desc<K::ROW0>(base + OFF_W0 + tap * W0_TAP) + 2u * k, idesc,
-                                      accumulate, mask);
+                        umma_f16_masked(d, umma_desc<K::ROW0>(sa0) + 2u * k, umma_desc<K::ROW0>(base + OFF_W0 + tap * W0_TAP) + 2u * k,
+                                        idesc, accumulate, mask);
                         accumulate = 1u;
                     }
                     if constexpr (K::KS1 > 0) {
 #pragma unroll
                         for (int k = 0; k < K::KS1; ++k)                     // second channel block
-                            cv_mma_masked(d, cv_desc<K::ROW1>(sa1) + 2u * k, cv_desc<K::ROW1>(base + OFF_W1 + tap * W1_TAP) + 2u * k,
-                                          idesc, 1u, mask);
+                            umma_f16_masked(d, umma_desc<K::ROW1>(sa1) + 2u * k,
+                                            umma_desc<K::ROW1>(base + OFF_W1 + tap * W1_TAP) + 2u * k, idesc, 1u, mask);
                     }
                 }
-            cv_commit(empty(s));             // the smem stage is free once these MMAs have read it
-            cv_commit(tfull(acc));           // ... and the accumulator is complete
+            umma_commit(empty(s));           // the smem stage is free once these MMAs have read it
+            umma_commit(tfull(acc));         // ... and the accumulator is complete
             }
             __syncwarp();
         }
@@ -292,21 +221,21 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
             const long long board = blockIdx.x + (long long)(it >> 1) * gridDim.x;
             if (board >= boards) break;
             const unsigned acc = it % ACC, aph = (it / ACC) & 1u;
-            cv_bar_wait(tfull(acc), aph);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            mbar_wait(tfull(acc), aph);
+            tcgen05_fence_after();
             uint32_t v[32];
             {
                 uint32_t lo[16], hi[16];
                 const unsigned taddr = tmem + ((unsigned)(q * 32) << 16) + acc * C + third * 32;
-                cv_ld16(taddr, lo);
-                cv_ld16(taddr + 16, hi);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                tmem_ld16(taddr, lo);
+                tmem_ld16(taddr + 16, hi);
+                tmem_wait_ld();
 #pragma unroll
                 for (int j = 0; j < 16; ++j) { v[j] = lo[j]; v[16 + j] = hi[j]; }
             }
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            tcgen05_fence_before();
             __syncwarp();
-            if (lane == 0) cv_bar_arrive(tempty(acc));       // the accumulator is in registers: release it
+            if (lane == 0) mbar_arrive(tempty(acc));       // the accumulator is in registers: release it
             if (MSW_DBG(1)) continue;
             __half *dst = out + (board * 256 + (it & 1u) * 128 + q * 32 + lane) * (long long)C + third * 32;
 #pragma unroll
@@ -358,16 +287,16 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
                 const unsigned it = 2u * bi + half, acc = it % ACC, aph = (it / ACC) & 1u;
                 if (EPI != 0)     // the 16 KB of residual stream this warpgroup will read for this tile: one line per thread on its way to L2
                     asm volatile("prefetch.global.L2 [%0];" :: "l"(gp.res32 + cv_p8(board, half, third, 0, 0) + (q * 32 + lane) * 32));
-                cv_bar_wait(tfull(acc), aph);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                mbar_wait(tfull(acc), aph);
+                tcgen05_fence_after();
                 uint32_t lo[16], hi[16];
                 const unsigned taddr = tmem + ((unsigned)(q * 32) << 16) + acc * C + third * 32;
-                cv_ld16(taddr, lo);
-                cv_ld16(taddr + 16, hi);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                tmem_ld16(taddr, lo);
+                tmem_ld16(taddr + 16, hi);
+                tmem_wait_ld();
+                tcgen05_fence_before();
                 __syncwarp();
-                if (lane == 0) cv_bar_arrive(tempty(acc));
+                if (lane == 0) mbar_arrive(tempty(acc));
                 if (MSW_DBG(16)) continue;
 #pragma unroll
                 for (int jj = 0; jj < 16; ++jj) {
@@ -493,29 +422,12 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
         }
     }
 
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
     if (warp == 2) {
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"((unsigned)TMEM_COLS) : "memory");
+        tcgen05_fence_after();
+        tmem_dealloc(tmem, TMEM_COLS);
     }
-}
-
-typedef CUresult (*CvEncodeFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                               const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                               CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static CvEncodeFn cv_encode_fn()
-{
-    static const CvEncodeFn fn = [] {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-            q != cudaDriverEntryPointSuccess)
-            p = nullptr;
-        return reinterpret_cast<CvEncodeFn>(p);
-    }();
-    return fn;
 }
 
 }  // namespace msw
@@ -549,7 +461,7 @@ static int conv_launch(const char *who, const void *x16, const void *w_taps16, v
     if ((((uintptr_t)x16 | (uintptr_t)w_taps16 | (uintptr_t)y16) & 31u) != 0)
         return fail(MSW_ERR_ALIGN, "%s: tensors must be 32-byte aligned", who);
     if (n == 0) return MSW_OK;
-    if (!cv_encode_fn()) return fail(MSW_ERR_ARG, "%s: cuTensorMapEncodeTiled is not available", who);
+    if (!tensor_map_encoder_available()) return fail(MSW_ERR_ARG, "%s: cuTensorMapEncodeTiled is not available", who);
     // first channel block: 64 channels / 128-byte swizzle (Cin = 96) or all 16 channels / 32-byte swizzle (Cin = 16);
     // second block (Cin = 96 only): 32 channels / 64-byte swizzle
     const cuuint32_t b0 = Cin == 96 ? 64u : 16u;
@@ -559,14 +471,9 @@ static int conv_launch(const char *who, const void *x16, const void *w_taps16, v
         // activation [n][16][16][Cin] fp16: dims innermost first
         const cuuint64_t dims[4] = {(cuuint64_t)Cin, 16, 16, (cuuint64_t)n};
         const cuuint64_t strides[3] = {(cuuint64_t)Cin * 2, (cuuint64_t)Cin * 2 * 16, (cuuint64_t)Cin * 2 * 256};
-        const cuuint32_t estr[4] = {1, 1, 1, 1};
         const cuuint32_t box0[4] = {b0, 16, cv::ROWS_IN, 1}, box1[4] = {32, 16, cv::ROWS_IN, 1};
-        const CUresult r0 = cv_encode_fn()(&ma0, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void *>(x16), dims, strides,
-                                           box0, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw0,
-                                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        const CUresult r1 = cv_encode_fn()(&ma1, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void *>(x16), dims, strides,
-                                           box1, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
-                                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        const CUresult r0 = encode_tiled(&ma0, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, x16, dims, strides, box0, sw0);
+        const CUresult r1 = encode_tiled(&ma1, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, x16, dims, strides, box1, CU_TENSOR_MAP_SWIZZLE_64B);
         if (r0 != CUDA_SUCCESS || (Cin == 96 && r1 != CUDA_SUCCESS))
             return fail(MSW_ERR_ARG, "%s: activation tensor map failed (%d, %d)", who, (int)r0, (int)r1);
     }
@@ -574,14 +481,9 @@ static int conv_launch(const char *who, const void *x16, const void *w_taps16, v
         // weights [9 taps * 96 co][Cin] fp16
         const cuuint64_t dims[2] = {(cuuint64_t)Cin, (cuuint64_t)9 * C};
         const cuuint64_t strides[1] = {(cuuint64_t)Cin * 2};
-        const cuuint32_t estr[2] = {1, 1};
         const cuuint32_t box0[2] = {b0, (cuuint32_t)C}, box1[2] = {32, (cuuint32_t)C};
-        const CUresult r0 = cv_encode_fn()(&mw0, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void *>(w_taps16), dims, strides,
-                                           box0, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw0,
-                                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        const CUresult r1 = cv_encode_fn()(&mw1, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void *>(w_taps16), dims, strides,
-                                           box1, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
-                                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        const CUresult r0 = encode_tiled(&mw0, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, w_taps16, dims, strides, box0, sw0);
+        const CUresult r1 = encode_tiled(&mw1, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, w_taps16, dims, strides, box1, CU_TENSOR_MAP_SWIZZLE_64B);
         if (r0 != CUDA_SUCCESS || (Cin == 96 && r1 != CUDA_SUCCESS))
             return fail(MSW_ERR_ARG, "%s: weight tensor map failed (%d, %d)", who, (int)r0, (int)r1);
     }

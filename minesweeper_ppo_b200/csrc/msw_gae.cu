@@ -21,6 +21,7 @@
 // sizes, where the serial walk is the critical path.
 #include "../../include/msw_b200.h"
 #include "msw_error.h"
+#include "msw_sm100.cuh"
 
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -139,29 +140,6 @@ gae_kernel(const float *__restrict__ rewards, const float *__restrict__ values,
 }
 
 // ---------------------------------------------------------------------------
-// TMA helpers (cp.async.bulk.tensor.2d loads completing on an mbarrier, bulk-group stores, elect.sync)
-// ---------------------------------------------------------------------------
-__device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void tma_load_2d(void *dst, const CUtensorMap *map, int c0, int c1, unsigned long long *bar)
-{
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                 :: "r"(smem_u32(dst)), "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap *map, int c0, int c1, const void *src)
-{
-    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%1, %2}], [%3];"
-                 :: "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(src)) : "memory");
-}
-
-__device__ __forceinline__ bool elect_one()      // one lane of a converged warp (elect.sync)
-{
-    unsigned pred;
-    asm volatile("{ .reg .pred p; elect.sync _|p, 0xffffffff; selp.u32 %0, 1, 0, p; }" : "=r"(pred));
-    return pred != 0u;
-}
-
-// ---------------------------------------------------------------------------
 // TMA kernel (the default when N % 16 == 0 and the arrays are 16-byte aligned): the same arithmetic in [32 x 32]
 // time slices through a 4-stage shared-memory ring, with the three kinds of work on different warps so that only
 // the serial walk is on a CTA's critical path:
@@ -177,7 +155,7 @@ __device__ __forceinline__ bool elect_one()      // one lane of a converged warp
 // Measured on one B200 (profiles/r02x_gae_ab.txt) against round 2's first TMA kernel, which moved whole [128 x 32]
 // tiles load -> delta -> walk -> store with nothing overlapping inside a CTA (commit 9cc9c01): T=128, N=8,192
 // 5.2 vs 7.0 us back to back, 12.3 vs 14.3 us cold; N=524,288 (HBM-bound) 186 vs 222 us = 6.13 vs 5.15 TB/s
-// (0.94 vs 0.79 of the measured copy peak).
+// (0.94 vs 0.79 of the measured copy peak).  The mbarrier / TMA wrappers are in msw_sm100.cuh.
 // ---------------------------------------------------------------------------
 constexpr int PG_ROWS = 32, PG_COLS = 32, PG_STAGES = 4, PG_DWARPS = 3, PG_THREADS = (1 + PG_DWARPS + 1) * 32;
 
@@ -190,18 +168,6 @@ struct PipeSmem {
     PipeStage st[PG_STAGES];
     alignas(8) unsigned long long full[PG_STAGES], dd[PG_STAGES], done[PG_STAGES];
 };
-
-__device__ __forceinline__ void mbar_wait(unsigned long long *bar, unsigned parity)
-{
-    unsigned ok = 0;
-    while (!ok)
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                     : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(unsigned long long *bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(smem_u32(bar)) : "memory");
-}
 
 template <int BATCH>
 __global__ void __launch_bounds__(PG_THREADS, BATCH == PG_ROWS ? 1 : 5)
@@ -219,11 +185,11 @@ gae_pipe_kernel(const __grid_constant__ CUtensorMap m_rewards, const __grid_cons
 
     if (tid == 0) {
         for (int s = 0; s < PG_STAGES; ++s) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(smem_u32(&S.full[s])));
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(&S.dd[s])), "r"(PG_DWARPS * 32));
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 32;" :: "r"(smem_u32(&S.done[s])));
+            mbar_init(smem_u32(&S.full[s]), 1);
+            mbar_init(smem_u32(&S.dd[s]), PG_DWARPS * 32);
+            mbar_init(smem_u32(&S.done[s]), 32);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_fence_init();
     }
     __syncthreads();
 
@@ -231,31 +197,32 @@ gae_pipe_kernel(const __grid_constant__ CUtensorMap m_rewards, const __grid_cons
         // ---- producer
         if (elect_one()) {
             // the store descriptors are first needed a few us into the kernel: fetch them now, off the critical path
-            asm volatile("prefetch.tensormap [%0];" :: "l"(&m_adv) : "memory");
-            asm volatile("prefetch.tensormap [%0];" :: "l"(&m_ret) : "memory");
+            tma_prefetch(&m_adv);
+            tma_prefetch(&m_ret);
             auto load = [&](int j) {
                 PipeStage &st = S.st[j % PG_STAGES];
-                unsigned long long *bar = &S.full[j % PG_STAGES];
+                const unsigned bar = smem_u32(&S.full[j % PG_STAGES]);
                 const int row0 = (slices - 1 - j) * PG_ROWS;
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(bar)), "r"(SLICE_BYTES) : "memory");
-                tma_load_2d(&st.r[0][0], &m_rewards, col0, row0, bar);
-                tma_load_2d(&st.v[0][0], &m_values, col0, row0, bar);
-                tma_load_2d(&st.d[0][0], &m_dones, col0, row0, bar);
+                mbar_expect_tx(bar, SLICE_BYTES);
+                tma_load_2d(smem_u32(&st.r[0][0]), &m_rewards, col0, row0, bar);
+                tma_load_2d(smem_u32(&st.v[0][0]), &m_values, col0, row0, bar);
+                tma_load_2d(smem_u32(&st.d[0][0]), &m_dones, col0, row0, bar);
             };
             for (int j = 0; j < slices && j < PG_STAGES; ++j) load(j);
             for (int j = 0; j < slices; ++j) {
                 const int s = j % PG_STAGES;
-                mbar_wait(&S.done[s], (unsigned)(j / PG_STAGES) & 1u);
+                const unsigned ph = (unsigned)(j / PG_STAGES) & 1u;
+                mbar_wait(smem_u32(&S.done[s]), ph);
                 const int row0 = (slices - 1 - j) * PG_ROWS;
-                tma_store_2d(&m_adv, col0, row0, &S.st[s].r[0][0]);
-                tma_store_2d(&m_ret, col0, row0, &S.st[s].v[0][0]);
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                tma_store_2d(&m_adv, col0, row0, smem_u32(&S.st[s].r[0][0]));
+                tma_store_2d(&m_ret, col0, row0, smem_u32(&S.st[s].v[0][0]));
+                bulk_commit();
                 if (j + PG_STAGES < slices) {
-                    asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // the stage's stores have read it
+                    bulk_wait_read<0>();                  // the stage's stores have read it
                     load(j + PG_STAGES);
                 }
             }
-            asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+            bulk_wait<0>();
         }
         return;
     }
@@ -268,7 +235,8 @@ gae_pipe_kernel(const __grid_constant__ CUtensorMap m_rewards, const __grid_cons
             PipeStage &st = S.st[j % PG_STAGES];
             const int row0 = (slices - 1 - j) * PG_ROWS;
             const int rows = (int)(T - row0 < PG_ROWS ? T - row0 : PG_ROWS);
-            mbar_wait(&S.full[j % PG_STAGES], (unsigned)(j / PG_STAGES) & 1u);
+            const unsigned ph = (unsigned)(j / PG_STAGES) & 1u;
+            mbar_wait(smem_u32(&S.full[j % PG_STAGES]), ph);
             const float gvn_next = __fmul_rn(gamma, st.v[0][lane]);         // for the slice before this one in time
             // delta[t] = (r[t] + (gamma * v[t+1]) * nnt[t]) - v[t] (buffers.py:88-90)
 #pragma unroll
@@ -280,7 +248,7 @@ gae_pipe_kernel(const __grid_constant__ CUtensorMap m_rewards, const __grid_cons
                 }
             }
             gvn = gvn_next;
-            mbar_arrive(&S.dd[j % PG_STAGES]);
+            mbar_arrive(smem_u32(&S.dd[j % PG_STAGES]));
         }
         return;
     }
@@ -292,7 +260,8 @@ gae_pipe_kernel(const __grid_constant__ CUtensorMap m_rewards, const __grid_cons
         PipeStage &st = S.st[j % PG_STAGES];
         const int row0 = (slices - 1 - j) * PG_ROWS;
         const int rows = (int)(T - row0 < PG_ROWS ? T - row0 : PG_ROWS);
-        mbar_wait(&S.dd[j % PG_STAGES], (unsigned)(j / PG_STAGES) & 1u);
+        const unsigned ph = (unsigned)(j / PG_STAGES) & 1u;
+        mbar_wait(smem_u32(&S.dd[j % PG_STAGES]), ph);
         // BATCH rows of the column go to registers ahead of the dependent FMUL -> FADD chain.  BATCH = 32 (the whole
         // slice, 96 loads in flight, 127 registers): the chain never waits for shared memory -- 5.2 instead of 6.2-7.1 us
         // at T=128, N=8,192, where the walk is the critical path -- but only 3 CTAs fit an SM, which costs 9 % when
@@ -334,27 +303,9 @@ gae_pipe_kernel(const __grid_constant__ CUtensorMap m_rewards, const __grid_cons
                 }
             }
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");        // generic-proxy writes -> visible to the TMA store
-        mbar_arrive(&S.done[j % PG_STAGES]);
+        fence_proxy_async();                    // generic-proxy writes -> visible to the TMA store
+        mbar_arrive(smem_u32(&S.done[j % PG_STAGES]));
     }
-}
-
-// cuTensorMapEncodeTiled through the runtime's driver entry point (no -lcuda at link time)
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn encode_tiled_fn()
-{
-    static const EncodeTiledFn fn = [] {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-            q != cudaDriverEntryPointSuccess)
-            p = nullptr;
-        return reinterpret_cast<EncodeTiledFn>(p);
-    }();
-    return fn;
 }
 
 // [T][N] row-major array of `es`-byte elements, box = [PG_ROWS][PG_COLS]
@@ -362,10 +313,8 @@ static bool make_map(CUtensorMap *m, const void *base, CUtensorMapDataType dt, s
 {
     const cuuint64_t dims[2] = {(cuuint64_t)N, (cuuint64_t)T};
     const cuuint64_t strides[1] = {(cuuint64_t)N * es};
-    const cuuint32_t box[2] = {PG_COLS, PG_ROWS}, estr[2] = {1, 1};
-    return encode_tiled_fn()(m, dt, 2, const_cast<void *>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    const cuuint32_t box[2] = {PG_COLS, PG_ROWS};
+    return encode_tiled(m, dt, 2, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE) == CUDA_SUCCESS;
 }
 
 }  // namespace msw
@@ -397,7 +346,7 @@ extern "C" int msw_gae(const float *rewards, const float *values, const uint8_t 
     constexpr bool tma_on = true;
 #endif
     const uintptr_t bases = (uintptr_t)rewards | (uintptr_t)values | (uintptr_t)dones | (uintptr_t)advantages | (uintptr_t)returns;
-    if (tma_on && N % 16 == 0 && (bases & 15u) == 0 && T <= 0x7fffffffLL && encode_tiled_fn()) {
+    if (tma_on && N % 16 == 0 && (bases & 15u) == 0 && T <= 0x7fffffffLL && tensor_map_encoder_available()) {
         CUtensorMap mr, mv, md, ma, mt;
         if (!make_map(&mr, rewards, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, T, N) ||
             !make_map(&mv, values, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, T, N) ||

@@ -20,6 +20,7 @@
 #include "../../include/msw_b200.h"
 #include "msw_common.cuh"
 #include "msw_error.h"
+#include "msw_sm100.cuh"
 
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
@@ -27,19 +28,6 @@
 #include <stdlib.h>
 
 namespace msw {
-
-// 16-byte asynchronous global->shared copy (LDGSTS): staging a whole [HW][C] sample this way puts
-// every thread's ~12 loads in flight at once instead of one at a time (ncu: the synchronous loop
-// left the kernel at half the HBM rate).
-__device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src)
-{
-    const unsigned s = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" :: "r"(s), "l"(gmem_src) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all()
-{
-    asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory");
-}
 
 // Chan et al. update of (count, mean, M2) a <- a (+) b; empty sides pass the other through.
 __device__ __forceinline__ void chan_merge(float &na, float &ma, float &qa, float nb, float mb, float qb)
@@ -61,7 +49,6 @@ struct GnParams {
     float *y32;             // nullable [n][HW][C]
     int HW, C, G, cpg, CB, PPB;
     unsigned tile_bytes;
-    int bulk;                       // 1: the fp16 sample moves with ONE cp.async.bulk each way (load, y16 store)
     float eps, inv_count, drop_p, drop_scale;
     int relu;
     uint32_t k0, k1, call_lo, call_hi;
@@ -92,42 +79,22 @@ __global__ void __launch_bounds__(256, 4) gn_act_kernel(const GnParams p, long l
     float cb0[8];
 #pragma unroll
     for (int k = 0; k < 8; ++k) cb0[k] = (p.cbias && active) ? p.cbias[j * 8 + k] : 0.0f;
-    auto stage = [&](long long s, int buf) {            // each thread copies (and later reads) only its own chunks
-        if (active) {
-            uint4 *tile = reinterpret_cast<uint4 *>(smem_raw + buf * tile_bytes);
-            const uint4 *src = reinterpret_cast<const uint4 *>(p.x) + s * (long long)p.HW * p.CB;
-            for (int r = r0; r < p.HW; r += p.PPB) cp_async16(tile + r * p.CB + j, src + r * p.CB + j);
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-    };
 
     const long long n = blockIdx.x;
-    const int buf = 0;
     __shared__ __align__(8) unsigned long long s_bar;
     const unsigned sample_bytes = (unsigned)p.HW * (unsigned)p.C * 2u;
     if (n < n_samples) {
-        if (p.bulk) {
-            // the sample is one contiguous block of global memory: one bulk copy, completion on an mbarrier
-            const unsigned bar = (unsigned)__cvta_generic_to_shared(&s_bar);
-            if (tid == 0) {
-                asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(bar));
-                asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar), "r"(sample_bytes) : "memory");
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                             :: "r"((unsigned)__cvta_generic_to_shared(smem_raw)),
-                                "l"(reinterpret_cast<const uint4 *>(p.x) + n * (long long)p.HW * p.CB), "r"(sample_bytes), "r"(bar)
-                             : "memory");
-            }
-            __syncthreads();                          // the barrier is initialised before anyone polls it
-            unsigned done = 0;
-            while (!done)
-                asm volatile("{ .reg .pred q; mbarrier.try_wait.parity.shared::cta.b64 q, [%1], 0; selp.u32 %0, 1, 0, q; }"
-                             : "=r"(done) : "r"(bar) : "memory");
-        } else {
-            stage(n, 0);
-            asm volatile("cp.async.wait_group 0;" ::: "memory");
+        // the sample is one contiguous block of global memory: one bulk copy, completion on an mbarrier
+        const unsigned bar = smem_u32(&s_bar);
+        if (tid == 0) {
+            mbar_init(bar, 1);
+            mbar_fence_init();
+            mbar_expect_tx(bar, sample_bytes);
+            bulk_load(smem_u32(smem_raw), reinterpret_cast<const uint4 *>(p.x) + n * (long long)p.HW * p.CB, sample_bytes, bar);
         }
-        uint4 *tile = reinterpret_cast<uint4 *>(smem_raw + buf * tile_bytes);
+        __syncthreads();                              // the barrier is initialised before anyone polls it
+        mbar_wait(bar, 0);
+        uint4 *tile = reinterpret_cast<uint4 *>(smem_raw);
         const long long base = n * (long long)p.HW * p.CB;                       // in uint4 chunks
 
         // ONE pass for the statistics: per thread, shifted sums S1 = sum (v - c), S2 = sum (v - c)^2 of
@@ -220,7 +187,6 @@ __global__ void __launch_bounds__(256, 4) gn_act_kernel(const GnParams p, long l
                 }
             }
             const float4 *__restrict__ res = p.res ? reinterpret_cast<const float4 *>(p.res) + 2 * base : nullptr;
-            uint4 *__restrict__ y16 = p.y16 ? reinterpret_cast<uint4 *>(p.y16) + base : nullptr;
             float4 *__restrict__ y32 = p.y32 ? reinterpret_cast<float4 *>(p.y32) + 2 * base : nullptr;
 #pragma unroll
             for (int k = 0; k < 8; ++k) psum[k] = 0.0f;
@@ -259,24 +225,22 @@ __global__ void __launch_bounds__(256, 4) gn_act_kernel(const GnParams p, long l
                     y32[2 * idx] = make_float4(o[0], o[1], o[2], o[3]);
                     y32[2 * idx + 1] = make_float4(o[4], o[5], o[6], o[7]);
                 }
-                if (y16) {
+                if (p.y16) {
                     uint4 out;
                     __half2 *oh = reinterpret_cast<__half2 *>(&out);
 #pragma unroll
                     for (int k = 0; k < 4; ++k) oh[k] = __floats2half2_rn(o[2 * k], o[2 * k + 1]);
-                    if (p.bulk) tile[idx] = out;      // in place over the thread's own input chunk
-                    else y16[idx] = out;
+                    tile[idx] = out;                  // in place over the thread's own input chunk
                 }
             }
         }
-        if (p.bulk && p.y16) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");    // generic-proxy writes -> visible to the bulk store
+        if (p.y16) {
+            fence_proxy_async();                      // generic-proxy writes -> visible to the bulk store
             __syncthreads();
             if (tid == 0) {
-                asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
-                             :: "l"(reinterpret_cast<uint4 *>(p.y16) + n * (long long)p.HW * p.CB),
-                                "r"((unsigned)__cvta_generic_to_shared(smem_raw)), "r"(sample_bytes) : "memory");
-                asm volatile("cp.async.bulk.commit_group;\ncp.async.bulk.wait_group.read 0;" ::: "memory");
+                bulk_store(reinterpret_cast<uint4 *>(p.y16) + n * (long long)p.HW * p.CB, smem_u32(smem_raw), sample_bytes);
+                bulk_commit();
+                bulk_wait_read<0>();
             }
         }
         if (p.pool) {
@@ -387,8 +351,14 @@ __global__ void __launch_bounds__(256) gn_act_bwd_kernel(const GnBwdParams p)
     // pass A: group sums of dy*gamma and dy*gamma*z; per-channel dgamma / dbeta
     float s1 = 0.0f, s2 = 0.0f;
     if (active) {
-        for (int r = r0; r < p.HW; r += p.PPB) cp_async16(tile + r * p.CB + j, xs + r * p.CB + j);
-        cp_async_wait_all();
+        // cp.async puts every thread's loads in flight at once (a synchronous copy loop left the forward kernel
+        // at half the HBM rate)
+        for (int r = r0; r < p.HW; r += p.PPB) {
+            const uint4 *src = xs + r * p.CB + j;
+            cp_async16(smem_u32(tile + r * p.CB + j), src);
+        }
+        cp_async_commit();
+        cp_async_wait<0>();
 #pragma unroll 2
         for (int r = r0; r < p.HW; r += p.PPB) {
             const int idx = r * p.CB + j;
@@ -538,7 +508,6 @@ extern "C" int msw_gn_act(const void *x16, const float *conv_bias, const float *
     p.pool = pool32;
     p.sample_base = (long long)sample_id_base;
     p.tile_bytes = (unsigned)tile_bytes;
-    p.bulk = 1;      // one cp.async.bulk per sample (the per-thread cp.async / STG path measured 6 % slower in round 1, DESIGN.md section 4.5)
     if ((save_mean != nullptr) != (save_rstd != nullptr) || (save_mean != nullptr) != (save_mask != nullptr))
         return fail(MSW_ERR_ARG, "msw_gn_act: save_mean / save_rstd / save_mask must be given together");
     p.save_mean = save_mean; p.save_rstd = save_rstd; p.save_mask = save_mask;

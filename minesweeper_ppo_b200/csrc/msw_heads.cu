@@ -16,6 +16,7 @@
 // plus 4 bytes of output per row.
 #include "../../include/msw_b200.h"
 #include "msw_error.h"
+#include "msw_sm100.cuh"
 
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
@@ -27,16 +28,10 @@ namespace msw {
 constexpr int HEADS_ROWS = 128;     // rows of A per CTA tile
 constexpr int HEADS_THREADS = 256;  // 8 warps: 4 along the rows x 2 heads
 
-__device__ __forceinline__ void heads_cp16(void *smem_dst, const void *gmem_src)
-{
-    const unsigned s = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" :: "r"(s), "l"(gmem_src) : "memory");
-}
 __device__ __forceinline__ void ldmatrix_x4(uint32_t (&r)[4], const void *smem)
 {
-    const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
     asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(s));
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(smem_u32(smem)));
 }
 __device__ __forceinline__ void mma_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1)
 {
@@ -74,16 +69,19 @@ heads_kernel(const __half *__restrict__ A, const __half *__restrict__ W1, const 
             const int r = q / CH, c = q % CH;
             long long row = row0 + r;
             if (row >= R) row = R - 1;               // tail rows repeat the last row; their results are not stored
-            heads_cp16(&S.a[buf][r][c * 8], A + row * C + c * 8);
+            const __half *src = A + row * C + c * 8;
+            cp_async16(smem_u32(&S.a[buf][r][c * 8]), src);
         }
     };
 
     long long tile = blockIdx.x;
     if (tile >= tiles) return;
-    for (int q = tid; q < 2 * C * CH; q += HEADS_THREADS)
-        heads_cp16(&S.w[q / CH][(q % CH) * 8], W1 + (long long)(q / CH) * C + (q % CH) * 8);
+    for (int q = tid; q < 2 * C * CH; q += HEADS_THREADS) {
+        const __half *src = W1 + (long long)(q / CH) * C + (q % CH) * 8;
+        cp_async16(smem_u32(&S.w[q / CH][(q % CH) * 8]), src);
+    }
     stage_a(tile, 0);
-    asm volatile("cp.async.commit_group;" ::: "memory");
+    cp_async_commit();
     for (int q = tid; q < 2 * C; q += HEADS_THREADS) {
         S.b1[q] = __half2float(B1[q]);
         S.w2[q] = __half2float(W2[q]);
@@ -95,7 +93,8 @@ heads_kernel(const __half *__restrict__ A, const __half *__restrict__ W1, const 
     for (; tile < tiles; tile += gridDim.x, buf ^= 1) {
         const long long next = tile + gridDim.x;
         if (next < tiles) stage_a(next, buf ^ 1);
-        asm volatile("cp.async.commit_group;\ncp.async.wait_group 1;" ::: "memory");
+        cp_async_commit();
+        cp_async_wait<1>();
         __syncthreads();                             // tile `buf` (and, the first time, W1 / b1 / w2) is visible
 
         float acc[2][C / 8][4];
@@ -153,7 +152,7 @@ heads_kernel(const __half *__restrict__ A, const __half *__restrict__ W1, const 
             }
         __syncthreads();                             // everyone is done with `buf` before it is refilled
     }
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
+    cp_async_wait<0>();
 }
 
 template <int C>

@@ -15,6 +15,7 @@
 // tensor's edge, TMA zero-fills it, and the issuer simply skips the k-steps that would multiply zeros.
 #include "../../include/msw_b200.h"
 #include "msw_error.h"
+#include "msw_sm100.cuh"
 
 #include <cuda.h>
 #include <cuda_fp16.h>
@@ -38,66 +39,6 @@ struct TcCfg {
     static constexpr unsigned BYTES = OFF_TMEM + 16u + 1024u;   // + slack to align the base to 1024 B
 };
 
-__device__ __forceinline__ unsigned tc_smem(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void tc_bar_init(unsigned bar, unsigned count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(bar), "r"(count));
-}
-__device__ __forceinline__ void tc_bar_expect(unsigned bar, unsigned bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void tc_bar_arrive(unsigned bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_bar_wait(unsigned bar, unsigned parity)
-{
-    unsigned done = 0;
-    while (!done)
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tc_tma_load(unsigned dst, const CUtensorMap *map, int c0, int c1, unsigned bar)
-{
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                 :: "r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar) : "memory");
-}
-// K-major operand tile, 128-byte swizzle: rows 128 B apart, 8-row groups 1024 B apart (SBO), LBO unused (= 1),
-// descriptor version 1 (sm_100), layout type 2 (SWIZZLE_128B).  `addr` is the shared-memory byte address.
-__device__ __forceinline__ uint64_t tc_desc(unsigned addr)
-{
-    return (uint64_t)((addr >> 4) & 0x3FFFu) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
-}
-__device__ __forceinline__ void tc_mma(unsigned d_tmem, uint64_t a, uint64_t b, unsigned idesc, unsigned accumulate)
-{
-    asm volatile("{ .reg .pred p; setp.ne.b32 p, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p; }"
-                 :: "r"(d_tmem), "l"(a), "l"(b), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void tc_commit(unsigned bar)
-{
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(bar) : "memory");
-}
-// One lane of a converged warp: inside an elect.sync region ptxas issues tcgen05 / TMA instructions without the
-// divergence waterfall it wraps around them under `lane == 0` (see msw_conv_tc.cu).
-__device__ __forceinline__ bool tc_elect_one()
-{
-    unsigned pred;
-    asm volatile("{ .reg .pred p; elect.sync _|p, 0xffffffff; selp.u32 %0, 1, 0, p; }" : "=r"(pred));
-    return pred != 0u;
-}
-__device__ __forceinline__ void tc_ld32(unsigned taddr, uint32_t (&v)[32])
-{
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-                 "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-                 "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                   "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-                   "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-                   "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-                 : "r"(taddr) : "memory");
-}
-
 template <int C>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 heads_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_w,
@@ -106,8 +47,8 @@ heads_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
 {
     using Cfg = TcCfg<C>;
     extern __shared__ unsigned char smem_dyn[];
-    const unsigned base = (tc_smem(smem_dyn) + 1023u) & ~1023u;          // swizzled TMA tiles need 1024-byte alignment
-    unsigned char *gen = smem_dyn + (base - tc_smem(smem_dyn));           // generic pointer to the same place
+    const unsigned base = (smem_u32(smem_dyn) + 1023u) & ~1023u;         // swizzled TMA tiles need 1024-byte alignment
+    unsigned char *gen = smem_dyn + (base - smem_u32(smem_dyn));          // generic pointer to the same place
     const unsigned sB = base, sA = base + Cfg::OFF_A;
     float *s_b1 = reinterpret_cast<float *>(gen + Cfg::OFF_B1), *s_w2 = reinterpret_cast<float *>(gen + Cfg::OFF_W2);
     const unsigned bars = base + Cfg::OFF_BAR;
@@ -120,62 +61,59 @@ heads_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (tid == 0) {
-        for (int s = 0; s < TC_STAGES; ++s) { tc_bar_init(full(s), 1); tc_bar_init(empty(s), 1); }
-        for (int a = 0; a < 2; ++a) { tc_bar_init(tfull(a), 1); tc_bar_init(tempty(a), 8); }
-        tc_bar_init(bfull, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (int s = 0; s < TC_STAGES; ++s) { mbar_init(full(s), 1); mbar_init(empty(s), 1); }
+        for (int a = 0; a < 2; ++a) { mbar_init(tfull(a), 1); mbar_init(tempty(a), 8); }
+        mbar_init(bfull, 1);
+        mbar_fence_init();
     }
-    if (warp == 2) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     :: "r"(base + Cfg::OFF_TMEM), "r"((unsigned)TC_TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 2) tmem_alloc(base + Cfg::OFF_TMEM, TC_TMEM_COLS);
     if (warp >= 4)
         for (int q = tid - 128; q < Cfg::N; q += TC_THREADS - 128) {
             s_b1[q] = __half2float(B1[q]);
             s_w2[q] = __half2float(W2[q]);
         }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const unsigned tmem = *s_tmem;
 
+    // warps 0 and 1 issue TMA / tcgen05 from one lane chosen by elect_one (msw_sm100.cuh says why not lane == 0)
     if (warp == 0) {
-        if (tc_elect_one()) {
+        if (elect_one()) {
         // ---- TMA producer
-        tc_bar_expect(bfull, Cfg::B_BYTES);
-        for (int kb = 0; kb < Cfg::KB; ++kb) tc_tma_load(sB + kb * Cfg::B_BLOCK, &map_w, kb * 64, 0, bfull);
+        mbar_expect_tx(bfull, Cfg::B_BYTES);
+        for (int kb = 0; kb < Cfg::KB; ++kb) tma_load_2d(sB + kb * Cfg::B_BLOCK, &map_w, kb * 64, 0, bfull);
         unsigned it = 0;
         for (long long tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++it) {
             const unsigned s = it % TC_STAGES, ph = (it / TC_STAGES) & 1u;
-            tc_bar_wait(empty(s), ph ^ 1u);
-            tc_bar_expect(full(s), Cfg::A_STAGE);
+            mbar_wait(empty(s), ph ^ 1u);
+            mbar_expect_tx(full(s), Cfg::A_STAGE);
             for (int kb = 0; kb < Cfg::KB; ++kb)
-                tc_tma_load(sA + s * Cfg::A_STAGE + kb * Cfg::A_BLOCK, &map_a, kb * 64, (int)(tile * TC_ROWS), full(s));
+                tma_load_2d(sA + s * Cfg::A_STAGE + kb * Cfg::A_BLOCK, &map_a, kb * 64, (int)(tile * TC_ROWS), full(s));
         }
         }
     } else if (warp == 1) {
         // ---- MMA issuer.  Instruction descriptor: D = F32 (bits 4-5 = 1), A = B = F16 (0), both K-major (0),
         // N >> 3 at bits 17-22, M >> 4 at bits 24-28.
         constexpr unsigned idesc = (1u << 4) | ((unsigned)(Cfg::N >> 3) << 17) | ((unsigned)(TC_ROWS >> 4) << 24);
-        tc_bar_wait(bfull, 0);
+        mbar_wait(bfull, 0);
         unsigned it = 0;
         for (long long tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++it) {
             const unsigned s = it % TC_STAGES, ph = (it / TC_STAGES) & 1u, as = it & 1u, aph = (it >> 1) & 1u;
-            tc_bar_wait(tempty(as), aph ^ 1u);
-            tc_bar_wait(full(s), ph);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            mbar_wait(tempty(as), aph ^ 1u);
+            mbar_wait(full(s), ph);
+            tcgen05_fence_after();
             const unsigned d = tmem + as * TC_ACC_STRIDE;
-            if (tc_elect_one()) {
+            if (elect_one()) {
 #pragma unroll
             for (int ks = 0; ks < Cfg::KSTEPS; ++ks) {
                 const int kb = ks / 4, k = ks % 4;                          // 4 k-steps of 32 bytes per swizzle atom
-                const uint64_t da = tc_desc(sA + s * Cfg::A_STAGE + kb * Cfg::A_BLOCK) + (uint64_t)(2 * k);
-                const uint64_t db = tc_desc(sB + kb * Cfg::B_BLOCK) + (uint64_t)(2 * k);
-                tc_mma(d, da, db, idesc, ks > 0 ? 1u : 0u);
+                const uint64_t da = umma_desc<128>(sA + s * Cfg::A_STAGE + kb * Cfg::A_BLOCK) + (uint64_t)(2 * k);
+                const uint64_t db = umma_desc<128>(sB + kb * Cfg::B_BLOCK) + (uint64_t)(2 * k);
+                umma_f16(d, da, db, idesc, ks > 0 ? 1u : 0u);
             }
-            tc_commit(empty(s));             // the smem stage is free once these MMAs have read it
-            tc_commit(tfull(as));            // ... and the accumulator is complete
+            umma_commit(empty(s));           // the smem stage is free once these MMAs have read it
+            umma_commit(tfull(as));          // ... and the accumulator is complete
             }
             __syncwarp();
         }
@@ -188,15 +126,15 @@ heads_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
         unsigned it = 0;
         for (long long tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++it) {
             const unsigned as = it & 1u, aph = (it >> 1) & 1u;
-            tc_bar_wait(tfull(as), aph);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            mbar_wait(tfull(as), aph);
+            tcgen05_fence_after();
             const unsigned taddr = tmem + as * TC_ACC_STRIDE + head * C + ((unsigned)(q * 32) << 16);
             float sum = 0.0f;
 #pragma unroll
             for (int c0 = 0; c0 < C; c0 += 32) {
                 uint32_t v[32];
-                tc_ld32(taddr + c0, v);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                tmem_ld32(taddr + c0, v);
+                tmem_wait_ld();
 #pragma unroll
                 for (int j = 0; j < 32; j += 2) {
                     // hid = relu(fp16(acc + b1)) for two columns at once, then fp32 dot with w2
@@ -207,36 +145,19 @@ heads_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
                     sum = fmaf(f.y, w2[c0 + j + 1], fmaf(f.x, w2[c0 + j], sum));
                 }
             }
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            tcgen05_fence_before();
             __syncwarp();
-            if (lane == 0) tc_bar_arrive(tempty(as));
+            if (lane == 0) mbar_arrive(tempty(as));
             const long long row = tile * TC_ROWS + q * 32 + lane;
             if (row < R) out[row] = __float2half_rn(sum + b2);
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
     if (warp == 2) {
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"((unsigned)TC_TMEM_COLS) : "memory");
+        tcgen05_fence_after();
+        tmem_dealloc(tmem, TC_TMEM_COLS);
     }
-}
-
-typedef CUresult (*TcEncodeFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                               const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                               CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static TcEncodeFn tc_encode_fn()
-{
-    static const TcEncodeFn fn = [] {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-            q != cudaDriverEntryPointSuccess)
-            p = nullptr;
-        return reinterpret_cast<TcEncodeFn>(p);
-    }();
-    return fn;
 }
 
 // fp16 [rows][C] row-major, box = [box_rows][64 elements = 128 bytes], 128-byte swizzle, zero fill past the edges
@@ -244,10 +165,8 @@ static bool tc_make_map(CUtensorMap *m, const void *basep, int64_t rows, int C, 
 {
     const cuuint64_t dims[2] = {(cuuint64_t)C, (cuuint64_t)rows};
     const cuuint64_t strides[1] = {(cuuint64_t)C * 2};
-    const cuuint32_t box[2] = {64u, (cuuint32_t)box_rows}, estr[2] = {1, 1};
-    return tc_encode_fn()(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void *>(basep), dims, strides, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    const cuuint32_t box[2] = {64u, (cuuint32_t)box_rows};
+    return encode_tiled(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, basep, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B) == CUDA_SUCCESS;
 }
 
 template <int C>
@@ -273,7 +192,7 @@ static int launch_heads_tc(const void *a16, const void *w1, const void *b1, cons
 int heads_tc_launch(int C, const void *a16, const void *w1, const void *b1, const void *w2, const void *b2,
                     void *out_policy, void *out_mine, int64_t R, cudaStream_t stream)
 {
-    if (!tc_encode_fn() || R > 0x7fffffffLL) return -1;
+    if (!tensor_map_encoder_available() || R > 0x7fffffffLL) return -1;
     switch (C) {
     case 64: return launch_heads_tc<64>(a16, w1, b1, w2, b2, out_policy, out_mine, R, stream);
     case 96: return launch_heads_tc<96>(a16, w1, b1, w2, b2, out_policy, out_mine, R, stream);
