@@ -325,7 +325,8 @@ int msw_cell_heads(const void *a16, const void *w1, const void *b1, const void *
 
 /* 3x3 "same" convolution of the policy trunk (cnn_residual.py:10-13: Conv2d(C, C, 3, padding=1); :50: the
  * stem Conv2d(10, C, 3, padding=1) on the 16-channel input of msw_pack_obs16) on the tcgen05 tensor cores, for
- * the shape the medium config uses: 16x16 boards, C = 96, Cin = 96 or 16.  x16: fp16 NHWC [n][16][16][Cin];
+ * the shapes the medium config and the default residual model use: 16x16 boards, C = 96 (Cin = 96 or 16) or
+ * C = 128 (Cin = 128 or 16; each board on a 2-CTA cluster).  x16: fp16 NHWC [n][16][16][Cin];
  * w_taps16: fp16 [9][C][Cin], tap = ky*3 + kx of the module's [C][Cin][3][3] weight (zero for padded input
  * channels); y16: fp16 NHWC conv output WITHOUT bias (msw_gn_act adds it), fp32 accumulation. */
 int msw_conv3x3(const void *x16, const void *w_taps16, void *y16, int64_t n, int32_t H, int32_t W,
@@ -335,13 +336,16 @@ int msw_conv3x3(const void *x16, const void *w_taps16, void *y16, int64_t n, int
  * residual), ReLU, Dropout2d" of a residual block half (cnn_residual.py:17-27):
  *   y16 = fp16(relu(GN(fp16(conv(x16)) + conv_bias) [+ res32]) [* Dropout2d]),  y32 (nullable) the same in fp32;
  * the conv output is rounded to fp16 before the norm exactly as the autocast reference does; Dropout2d draws
- * msw_gn_act's stream, keyed by sample_id_base + board.  16x16 boards, C = 96, G = 6, Cin = 96 or 16 (the stem).
- * res32 (nullable; Cin = 96 only) and y32 are in the kernels' PRIVATE "P8" order -- [n][tile 2][channel third 3]
- * [8-channel chunk 4][pixel-in-tile 128][8] floats -- in which every 256-bit access of a warp is one contiguous
+ * msw_gn_act's stream, keyed by sample_id_base + board.  16x16 boards, groups of 16 channels: C = 96 with G = 6
+ * or C = 128 with G = 8; Cin = C or 16 (the stem).
+ * res32 (nullable; Cin = C only) and y32 are in the kernels' PRIVATE "P8" order -- [n][tile 2][32-channel slice
+ * C/32][8-channel chunk 4][pixel-in-tile 128][8] floats -- in which every 256-bit access of a warp is one contiguous
  * KB (the pixel-major NHWC order costs one line per lane); only this function reads or writes that stream.
- * pool4 (nullable, with res32, instead of y32): fp32 [n][4][C] per-row-quarter sums of the fp32 output, whose sum
- * over the 4 quarters / 256 is the AdaptiveAvgPool2d(1) of the value head (cnn_residual.py:65).
- * max_ctas: 0 = one persistent CTA per SM; k > 0 caps the grid so that two launches on different streams can
+ * pool4 (nullable, with res32, instead of y32): fp32 [n][Q][C] partial sums of the fp32 output -- Q = 4 row
+ * quarters (C = 96) or 8 = 2 tiles x 4 row quarters (C = 128) -- whose sum over Q / 256 is the
+ * AdaptiveAvgPool2d(1) of the value head (cnn_residual.py:65).
+ * max_ctas: 0 = one persistent CTA per SM; k > 0 caps the grid (C = 128: rounded down to an even count, one
+ * 2-CTA cluster per board at a time) so that two launches on different streams can
  * share the GPU (FusedRolloutForward overlaps an HBM-bound residual layer with an MMA-bound one that way). */
 int msw_conv3x3_gn(const void *x16, const void *w_taps16, const float *conv_bias, const float *res32,
                    const float *gamma, const float *beta, void *y16, float *y32, float *pool4, int64_t n,

@@ -2,6 +2,7 @@
 // 16 -> 96; fp16 NHWC in, fp32 accumulate, fp16 NHWC out) on the 5th-generation tensor cores, plain
 // (conv3x3_tc_kernel<false>: no bias, it is folded into msw_gn_act) or with GroupNorm / ReLU / Dropout2d /
 // residual add (and the value head's average pool) fused into the epilogue (conv3x3_tc_kernel<true>).
+// 128 -> 128 channels (and the stem's 16 -> 128) run on conv3x3_pair_kernel below: one board per CTA pair.
 //
 // out[y][x][co] = sum_{dy,dx,ci} in[y+dy][x+dx][ci] * w[co][ci][dy][dx] is computed as nine shifted GEMMs
 // per 128-pixel tile (8 image rows of one board) that all accumulate into ONE TMEM accumulator.  The tile's
@@ -30,6 +31,7 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdio.h>
 #include <stdlib.h>
 
 // Ablation switches for tools/convgn_ablation.py: compiled in only with -DMSW_DEV_KNOBS (the product library has none).
@@ -430,6 +432,359 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// 128 output channels: one board per CTA pair (2-CTA cluster, tcgen05 cta_group::2, M = 256, N = 128).
+//
+// At C = 128 the nine [128 x 128] weight taps take 288 KB, more than a CTA's shared memory, so each CTA of the pair
+// holds the nine taps of HALF the output channels (rank r: [64r, 64r + 64), 147,456 B) and stages tile r of the
+// board (image rows 8r .. 8r + 7, i.e. input rows 8r - 1 .. 8r + 8: the same 4-D TMA box as above).  The leader
+// (rank 0) issues one cta_group::2 MMA per tap and k-step for both tiles (9 taps x 8 k-steps = 72 per board); A
+// rows 128 .. 255 are the peer's tile, B's 64 + 64 rows the two weight halves, and each CTA's TMEM receives its own
+// 128 pixels x all 128 output channels.  Taps, shifted descriptors and the disable-output-lane masks are those of
+// conv3x3_tc_kernel, the mask covering the 256 rows of the pair.  K = 128 = two 64-channel blocks (128-byte rows,
+// 128-byte swizzle; both through the same tensor map); the stem (CIN = 16) is as above.
+//
+// GroupNorm statistics of a board span both tiles.  Every epilogue warp writes its (mean, M2) of its two groups
+// into its own CTA's exchange area AND the partner's (st.shared::cluster), then arrives on the partner's xfull
+// barrier; both CTAs then merge the same 2 x 16 partials in the same order, so they fold bit-identical a and b.  No
+// cluster barrier inside the loop: the producer and MMA warps never wait on an epilogue's statistics.
+//
+// Shared memory per CTA (CIN = 128; 232,064 of 232,448 B), from a 1024-byte aligned base:
+//        0  W0  [9 taps][64 co][64 ch]  128-byte swizzle     73,728
+//   73,728  W1  [9 taps][64 co][64 ch]  (channels 64..127)   73,728
+//  147,456  A   [2 stages][2 blocks][160 px][64 ch]          81,920
+//  229,376  barriers full[2] empty[2] wfull tfull[4] tempty[4] xfull[2], TMEM address   128
+//  229,504  X   [2 parity][2 tile][16 warps][mean0, M2_0, mean1, M2_1] f32               1,024
+//  230,528  conv bias [128] f32                                                          512
+//  231,040  a | b [2][128] f32                                                           1,024
+// Roles: warp 0 TMA producer (both CTAs), warp 1 MMA issuer (leader), warp 2 TMEM allocation (both), warps 4-19
+// epilogue (thread = pixel of the CTA's tile, warpgroup g = channels [32g, 32g + 32): groups 2g and 2g + 1).
+namespace cvp {
+constexpr int C = 128, HALF = 64, HW_W = 16, TILE_PX = 128, PX_IN = 160;
+constexpr int THREADS = 640, EPI_WARPS = 16, STAGES = 2, ACC = 4, TMEM_COLS = 512;    // 4 x 128 accumulator columns
+
+template <int CIN>
+struct Cfg {
+    static_assert(CIN == 128 || CIN == 16, "supported input widths");
+    static constexpr unsigned ROW0 = CIN == 128 ? 128u : 32u, ROW1 = CIN == 128 ? 128u : 0u;   // bytes per pixel row
+    static constexpr int KS0 = CIN == 128 ? 4 : 1, KS1 = CIN == 128 ? 4 : 0;                   // 16-channel k-steps
+    static constexpr int BOX0 = CIN == 128 ? 64 : 16;                                          // channels per block
+    static constexpr unsigned W0_TAP = HALF * ROW0, W1_TAP = HALF * ROW1;                      // this CTA's rows of a tap
+    static constexpr unsigned W0_BYTES = 9 * W0_TAP, W1_BYTES = 9 * W1_TAP;
+    static constexpr unsigned A0_BYTES = PX_IN * ROW0, A_STAGE = A0_BYTES + PX_IN * ROW1;
+    // the stem keeps conv3x3_tc_kernel's 1 KB in front of its activation ring; at CIN = 128 the first tap's read
+    // of one row before a stage lands in the weights, in rows the mask switches off
+    static constexpr unsigned OFF_W0 = 0, OFF_W1 = W0_BYTES, OFF_A = W0_BYTES + W1_BYTES + (CIN == 128 ? 0u : 1024u);
+    static constexpr unsigned OFF_BAR = OFF_A + STAGES * A_STAGE;
+    static constexpr unsigned OFF_TMEM = OFF_BAR + 15 * 8u;
+    static constexpr unsigned OFF_X = OFF_BAR + 128u;
+    static constexpr unsigned OFF_CB = OFF_X + 2 * 2 * EPI_WARPS * 4 * 4u;
+    static constexpr unsigned OFF_AB = OFF_CB + C * 4u;
+    static constexpr unsigned SMEM_BYTES = OFF_AB + 2 * C * 4u;
+    static_assert(OFF_A % 1024 == 0 && A0_BYTES % 1024 == 0 && A_STAGE % 1024 == 0 && W0_TAP % 1024 == 0, "swizzle atoms");
+    static_assert(SMEM_BYTES <= 232448, "shared memory of one CTA");
+};
+}  // namespace cvp
+
+// float offset of (board, tile, quarter, chunk, pixel-in-tile) in the C = 128 P8 order
+__device__ __forceinline__ long long cvp_p8(long long board, int tile, int quarter, int c4, int pp)
+{
+    return ((((board * 2 + tile) * 4 + quarter) * 4 + c4) * 128 + pp) * 8;
+}
+
+// GN / CIN / EPI as conv3x3_tc_kernel; pool4 is [n][tile 2 x row quarter 4][128].
+template <bool GN, int CIN, int EPI>
+__global__ void __launch_bounds__(cvp::THREADS, 1)
+conv3x3_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_constant__ CUtensorMap map_a1,
+                    const __grid_constant__ CUtensorMap map_w0, const __grid_constant__ CUtensorMap map_w1,
+                    __half *__restrict__ out, long long boards, const __grid_constant__ ConvGnParams gp)
+{
+    using namespace cvp;
+    using K = Cfg<CIN>;
+    constexpr unsigned OFF_A = K::OFF_A, W0_TAP = K::W0_TAP, W1_TAP = K::W1_TAP, A0_BYTES = K::A0_BYTES, A_STAGE = K::A_STAGE;
+    extern __shared__ __align__(1024) unsigned char smem_pair[];
+    const unsigned base = smem_u32(smem_pair);
+    if (base & 1023u) {                  // the layout has no room to realign; uniform over the grid
+        if (threadIdx.x == 0 && blockIdx.x == 0) printf("conv3x3_pair_kernel: dynamic shared memory is not 1024-byte aligned\n");
+        return;
+    }
+    const unsigned bars = base + K::OFF_BAR;
+    auto full = [&](unsigned s) { return bars + 8u * s; };
+    auto empty = [&](unsigned s) { return bars + 8u * (2 + s); };
+    const unsigned wfull = bars + 8u * 4;
+    auto tfull = [&](unsigned a) { return bars + 8u * (5 + a); };
+    auto tempty = [&](unsigned a) { return bars + 8u * (9 + a); };
+    auto xfull = [&](unsigned p) { return bars + 8u * (13 + p); };
+    volatile uint32_t *s_tmem = reinterpret_cast<volatile uint32_t *>(smem_pair + K::OFF_TMEM);
+
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const unsigned rank = cluster_ctarank(), peer = rank ^ 1u;
+    const long long board0 = blockIdx.x >> 1, bstride = gridDim.x >> 1;     // the pair's boards: board0 + i * bstride
+    if (tid == 0) {
+        for (unsigned s = 0; s < STAGES; ++s) { mbar_init(full(s), 2); mbar_init(empty(s), 1); }   // full: both producers
+        for (unsigned a = 0; a < ACC; ++a) { mbar_init(tfull(a), 1); mbar_init(tempty(a), 2 * EPI_WARPS); }
+        mbar_init(wfull, 2);
+        for (unsigned p = 0; p < 2; ++p) mbar_init(xfull(p), EPI_WARPS);    // the partner's epilogue warps
+        mbar_fence_init();
+    }
+    if (warp == 2) tmem_alloc_pair(base + K::OFF_TMEM, TMEM_COLS);
+    tcgen05_fence_before();
+    cluster_sync();                      // both CTAs' barriers are initialised before anyone arrives on them
+    tcgen05_fence_after();
+    const unsigned tmem = *s_tmem;
+
+    if (warp == 0) {
+        if (elect_one()) {
+        // ---- TMA producer: this CTA's 64 output channels of the nine taps once, then tile `rank` of every board;
+        // completion is counted on the leader's barriers (the MMA issuer's)
+        const unsigned wbar = mapa_shared(wfull, 0u);
+        const int wrow = (int)rank * HALF;
+        mbar_expect_tx_cluster(wbar, K::W0_BYTES + K::W1_BYTES);
+        for (int t = 0; t < 9; ++t) {
+            tma_load_2d_pair(base + K::OFF_W0 + t * W0_TAP, &map_w0, 0, t * C + wrow, wbar);
+            if (K::KS1) tma_load_2d_pair(base + K::OFF_W1 + t * W1_TAP, &map_w1, K::BOX0, t * C + wrow, wbar);
+        }
+        for (unsigned it = 0;; ++it) {
+            const long long board = board0 + (long long)it * bstride;
+            if (board >= boards) break;
+            const unsigned s = it % STAGES, ph = (it / STAGES) & 1u;
+            mbar_wait(empty(s), ph ^ 1u);
+            const unsigned fbar = mapa_shared(full(s), 0u);
+            mbar_expect_tx_cluster(fbar, A_STAGE);
+            tma_load_4d_pair(base + OFF_A + s * A_STAGE, &map_a0, 0, 0, 8 * (int)rank - 1, (int)board, fbar);
+            if (K::KS1) tma_load_4d_pair(base + OFF_A + s * A_STAGE + A0_BYTES, &map_a1, K::BOX0, 0, 8 * (int)rank - 1, (int)board, fbar);
+        }
+        }
+    } else if (warp == 1 && rank == 0) {
+        // ---- MMA issuer.  idesc: D = F32, A = B = F16, K-major, M = 256 (the pair), N = 128.
+        constexpr unsigned idesc = (1u << 4) | ((unsigned)(C >> 3) << 17) | ((unsigned)((2 * TILE_PX) >> 4) << 24);
+        mbar_wait(wfull, 0);
+        for (unsigned it = 0;; ++it) {
+            if (board0 + (long long)it * bstride >= boards) break;
+            const unsigned s = it % STAGES, ph = (it / STAGES) & 1u, acc = it % ACC, aph = (it / ACC) & 1u;
+            mbar_wait_cluster(tempty(acc), aph ^ 1u);            // both CTAs' epilogues have drained this accumulator
+            mbar_wait_cluster(full(s), ph);                      // both tiles have landed
+            tcgen05_fence_after();
+            const unsigned a0 = base + OFF_A + s * A_STAGE, a1 = a0 + A0_BYTES, d = tmem + acc * C;
+            if (elect_one()) {
+            unsigned accumulate = 0u;
+#pragma unroll
+            for (int dy = 0; dy < 3; ++dy)
+#pragma unroll
+                for (int o = 0; o < 3; ++o) {
+                    const int dxi = o == 0 ? 1 : o == 1 ? 0 : 2;           // the unmasked centre tap first
+                    const int tap = dy * 3 + dxi;
+                    const unsigned mask = dxi == 0 ? 0x00010001u : dxi == 2 ? 0x80008000u : 0u;
+                    const unsigned sa0 = a0 + (unsigned)((dy * HW_W + dxi - 1) * (int)K::ROW0);
+                    const unsigned sa1 = a1 + (unsigned)((dy * HW_W + dxi - 1) * (int)K::ROW1);
+#pragma unroll
+                    for (int k = 0; k < K::KS0; ++k) {
+                        umma_f16_masked_pair(d, umma_desc<K::ROW0>(sa0) + 2u * k,
+                                             umma_desc<K::ROW0>(base + K::OFF_W0 + tap * W0_TAP) + 2u * k, idesc, accumulate, mask);
+                        accumulate = 1u;
+                    }
+                    if constexpr (K::KS1 > 0) {
+#pragma unroll
+                        for (int k = 0; k < K::KS1; ++k)
+                            umma_f16_masked_pair(d, umma_desc<K::ROW1>(sa1) + 2u * k,
+                                                 umma_desc<K::ROW1>(base + K::OFF_W1 + tap * W1_TAP) + 2u * k, idesc, 1u, mask);
+                    }
+                }
+            umma_commit_pair(empty(s));          // both CTAs' stage s is free once these MMAs have read it
+            umma_commit_pair(tfull(acc));        // ... and both halves of the accumulator are complete
+            }
+            __syncwarp();
+        }
+    } else if (warp >= 4) {
+        const int we = warp - 4, q = warp & 3, wg = we >> 2, cbase = wg * 32, te = tid - 128, pp = q * 32 + lane;
+        if constexpr (!GN) {
+        for (unsigned it = 0;; ++it) {
+            const long long board = board0 + (long long)it * bstride;
+            if (board >= boards) break;
+            const unsigned acc = it % ACC, aph = (it / ACC) & 1u;
+            mbar_wait(tfull(acc), aph);
+            tcgen05_fence_after();
+            uint32_t lo[16], hi[16];
+            const unsigned taddr = tmem + ((unsigned)(q * 32) << 16) + acc * C + cbase;
+            tmem_ld16(taddr, lo);
+            tmem_ld16(taddr + 16, hi);
+            tmem_wait_ld();
+            tcgen05_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive_cluster(mapa_shared(tempty(acc), 0u));
+            __half *dst = out + (board * 256 + rank * 128 + pp) * (long long)C + cbase;
+#pragma unroll
+            for (int c0 = 0; c0 < 32; c0 += 16) {
+                const uint32_t *src = c0 == 0 ? lo : hi;
+                uint32_t packed[8];
+#pragma unroll
+                for (int k = 0; k < 8; ++k) {
+                    const __half2 hh = __floats2half2_rn(__uint_as_float(src[2 * k]), __uint_as_float(src[2 * k + 1]));
+                    packed[k] = *reinterpret_cast<const uint32_t *>(&hh);
+                }
+                cv_st256(dst + c0, packed);
+            }
+        }
+        } else {
+        float *s_x = reinterpret_cast<float *>(smem_pair + K::OFF_X);    // [parity][tile][warp][mean0, M2_0, mean1, M2_1]
+        float *s_cb = reinterpret_cast<float *>(smem_pair + K::OFF_CB);
+        float *s_ab = reinterpret_cast<float *>(smem_pair + K::OFF_AB);  // [a | b][channel]
+        const uint32_t thresh = (uint32_t)(gp.drop_p * 65536.0f);
+        if (te < C) s_cb[te] = gp.cbias[te];
+        asm volatile("bar.sync 1, 512;" ::: "memory");
+        const float2 *cb2 = reinterpret_cast<const float2 *>(s_cb + cbase);
+        const unsigned x_peer = mapa_shared(base + K::OFF_X, peer);
+        for (unsigned bi = 0;; ++bi) {
+            const long long board = board0 + (long long)bi * bstride;
+            if (board >= boards) break;
+            const unsigned par = bi & 1u, acc = bi % ACC, aph = (bi / ACC) & 1u;
+            float sc = gp.drop_scale;            // Dropout2d: msw_gn_act's stream, keyed by global board and 8-channel chunk
+            if (EPI == 0 && te < C && gp.drop_p > 0.0f) {
+                uint32_t w[4];
+                const long long gb = gp.sample_base + board;
+                philox4x32_10(gp.k0, gp.k1 ^ 0x44524f50u, (uint32_t)gb, (uint32_t)(gb >> 32) ^ (uint32_t)(te >> 3), gp.call_lo,
+                              gp.call_hi + (gp.epoch ? *gp.epoch : 0u), w);
+                const int k = te & 7;
+                const uint32_t u16 = (w[k >> 1] >> (16 * (k & 1))) & 0xFFFFu;
+                if (u16 < thresh) sc = 0.0f;
+            }
+            if (EPI != 0)     // the 16 KB of residual stream this warpgroup reads for this tile: one line per thread
+                asm volatile("prefetch.global.L2 [%0];" :: "l"(gp.res32 + cvp_p8(board, (int)rank, wg, 0, 0) + pp * 32));
+            mbar_wait(tfull(acc), aph);
+            tcgen05_fence_after();
+            uint32_t lo[16], hi[16];
+            const unsigned taddr = tmem + ((unsigned)(q * 32) << 16) + acc * C + cbase;
+            tmem_ld16(taddr, lo);
+            tmem_ld16(taddr + 16, hi);
+            tmem_wait_ld();
+            tcgen05_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive_cluster(mapa_shared(tempty(acc), 0u));
+            uint32_t h[16];                      // fp16-rounded conv output (the reference's rounding point)
+            float shift0 = 0.0f, shift1 = 0.0f, s1a = 0.0f, s2a = 0.0f, s1b = 0.0f, s2b = 0.0f;
+#pragma unroll
+            for (int jj = 0; jj < 16; ++jj) {
+                const uint32_t *src = jj < 8 ? lo : hi;
+                const __half2 hh = __floats2half2_rn(__uint_as_float(src[(2 * jj) & 15]), __uint_as_float(src[(2 * jj + 1) & 15]));
+                h[jj] = *reinterpret_cast<const uint32_t *>(&hh);
+                const float2 f = __half22float2(hh), cb = cb2[jj];
+                const float v0 = f.x + cb.x, v1 = f.y + cb.y;
+                if (jj == 0) shift0 = __shfl_sync(0xffffffffu, v0, 0);
+                if (jj == 8) shift1 = __shfl_sync(0xffffffffu, v0, 0);
+                if (jj < 8) {
+                    const float d0 = v0 - shift0, d1 = v1 - shift0;
+                    s1a += d0 + d1;
+                    s2a = fmaf(d0, d0, fmaf(d1, d1, s2a));
+                } else {
+                    const float d0 = v0 - shift1, d1 = v1 - shift1;
+                    s1b += d0 + d1;
+                    s2b = fmaf(d0, d0, fmaf(d1, d1, s2b));
+                }
+            }
+            // the warp's (mean, M2) of its 512 values per group, into both CTAs' exchange areas
+            s1a = cv_warp_sum(s1a); s2a = cv_warp_sum(s2a);
+            s1b = cv_warp_sum(s1b); s2b = cv_warp_sum(s2b);
+            if (lane == 0) {
+                const float4 st = make_float4(shift0 + s1a * (1.0f / 512.0f), s2a - s1a * s1a * (1.0f / 512.0f),
+                                              shift1 + s1b * (1.0f / 512.0f), s2b - s1b * s1b * (1.0f / 512.0f));
+                const unsigned slot = ((par * 2 + rank) * EPI_WARPS + we) * 16u;
+                *reinterpret_cast<float4 *>(smem_pair + K::OFF_X + slot) = st;
+                st_shared_cluster_v4(x_peer + slot, st);
+                mbar_arrive_cluster(mapa_shared(xfull(par), peer));
+            }
+            asm volatile("bar.sync 1, 512;" ::: "memory");
+            if (te < C) {
+                // one thread per channel: the board's statistics from tile 0's then tile 1's four warps (Chan et al.,
+                // the same order in both CTAs), folded with the affine, the conv bias and the Dropout2d scale
+                mbar_wait_cluster(xfull(par), (bi >> 1) & 1u);
+                const int c = te, gsel = (c >> 4) & 1, w4 = (c >> 5) * 4;
+                float na = 0.0f, mg = 0.0f, m2 = 0.0f;
+#pragma unroll
+                for (int t = 0; t < 2; ++t)
+#pragma unroll
+                    for (int qq = 0; qq < 4; ++qq) {
+                        const float *src = s_x + ((par * 2 + t) * EPI_WARPS + w4 + qq) * 4 + 2 * gsel;
+                        const float nn = na + 512.0f, delta = src[0] - mg, w = 512.0f / nn;
+                        mg = fmaf(delta, w, mg);
+                        m2 += src[1] + delta * delta * (na * w);
+                        na = nn;
+                    }
+                const float rg = rsqrtf(m2 * (1.0f / 4096.0f) + gp.eps);
+                const float a = gp.gamma[c] * rg;
+                s_ab[c] = a * sc;
+                s_ab[C + c] = fmaf(s_cb[c] - mg, a, gp.beta[c]) * sc;
+            }
+            asm volatile("bar.sync 1, 512;" ::: "memory");
+            // ---- normalise, (+ residual), ReLU, store: 8 channels at a time
+            const float4 *a4 = reinterpret_cast<const float4 *>(s_ab + cbase);
+            const float4 *b4 = reinterpret_cast<const float4 *>(s_ab + C + cbase);
+            uint32_t rnext[8];
+            if (EPI != 0) cv_ld256(gp.res32 + cvp_p8(board, (int)rank, wg, 0, pp), rnext);
+#pragma unroll
+            for (int c0 = 0; c0 < 32; c0 += 8) {
+                const float4 aa0 = a4[c0 >> 2], aa1 = a4[(c0 >> 2) + 1], bb0 = b4[c0 >> 2], bb1 = b4[(c0 >> 2) + 1];
+                const float av[8] = {aa0.x, aa0.y, aa0.z, aa0.w, aa1.x, aa1.y, aa1.z, aa1.w};
+                const float bv[8] = {bb0.x, bb0.y, bb0.z, bb0.w, bb1.x, bb1.y, bb1.z, bb1.w};
+                uint32_t rr[8];
+                if (EPI != 0) {
+#pragma unroll
+                    for (int k = 0; k < 8; ++k) rr[k] = rnext[k];
+                    if (c0 < 24) cv_ld256(gp.res32 + cvp_p8(board, (int)rank, wg, (c0 >> 3) + 1, pp), rnext);
+                }
+                uint32_t o[8];
+#pragma unroll
+                for (int j = 0; j < 8; j += 2) {
+                    const float2 f = __half22float2(*reinterpret_cast<const __half2 *>(&h[(c0 + j) >> 1]));
+                    float v0 = fmaf(f.x, av[j], bv[j]), v1 = fmaf(f.y, av[j + 1], bv[j + 1]);
+                    if (EPI != 0) { v0 += __uint_as_float(rr[j]); v1 += __uint_as_float(rr[j + 1]); }
+                    o[j] = __float_as_uint(fmaxf(v0, 0.0f));
+                    o[j + 1] = __float_as_uint(fmaxf(v1, 0.0f));
+                }
+                if (EPI != 2 && gp.y32) cv_st256(gp.y32 + cvp_p8(board, (int)rank, wg, c0 >> 3, pp), o);
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    const __half2 hh = __floats2half2_rn(__uint_as_float(o[2 * k]), __uint_as_float(o[2 * k + 1]));
+                    h[(c0 >> 1) + k] = *reinterpret_cast<const uint32_t *>(&hh);
+                }
+                if (EPI == 2) {
+                    // warp sum of 8 channels over the 32 lanes (pixels), the fixed butterfly of conv3x3_tc_kernel
+                    const bool b4s = lane & 16, b3s = lane & 8, b2s = lane & 4;
+                    float a1[4], a2[2], a3;
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) {
+                        const float lo4 = __uint_as_float(o[i]), hi4 = __uint_as_float(o[4 + i]);
+                        a1[i] = (b4s ? hi4 : lo4) + __shfl_xor_sync(0xffffffffu, b4s ? lo4 : hi4, 16);
+                    }
+#pragma unroll
+                    for (int i = 0; i < 2; ++i)
+                        a2[i] = (b3s ? a1[2 + i] : a1[i]) + __shfl_xor_sync(0xffffffffu, b3s ? a1[i] : a1[2 + i], 8);
+                    a3 = (b2s ? a2[1] : a2[0]) + __shfl_xor_sync(0xffffffffu, b2s ? a2[0] : a2[1], 4);
+                    a3 += __shfl_xor_sync(0xffffffffu, a3, 2);
+                    a3 += __shfl_xor_sync(0xffffffffu, a3, 1);
+                    if ((lane & 3) == 0)
+                        gp.pool4[(board * 8 + rank * 4 + q) * C + cbase + c0 + (b4s ? 4 : 0) + (b3s ? 2 : 0) + (b2s ? 1 : 0)] = a3;
+                }
+            }
+            __half *dst = out + (board * 256 + rank * 128 + pp) * (long long)C + cbase;
+#pragma unroll
+            for (int c0 = 0; c0 < 32; c0 += 16) {
+                uint32_t packed[8];
+#pragma unroll
+                for (int k = 0; k < 8; ++k) packed[k] = h[(c0 >> 1) + k];
+                cv_st256(dst + c0, packed);
+            }
+        }
+        }
+    }
+
+    tcgen05_fence_before();
+    cluster_sync();                      // neither CTA leaves (or frees TMEM) while its partner may still signal it
+    if (warp == 2) {
+        tcgen05_fence_after();
+        tmem_dealloc_pair(tmem, TMEM_COLS);
+    }
+}
+
 }  // namespace msw
 
 template <bool GN, int CIN, int EPI>
@@ -448,24 +803,58 @@ static int conv_launch_t(const CUtensorMap &ma0, const CUtensorMap &ma1, const C
     return MSW_OK;
 }
 
+// The CTA-pair kernel: clusters of 2, one board per cluster at a time, at most one cluster per two SMs (the
+// launch's grid cap is rounded down to an even count).
+template <bool GN, int CIN, int EPI>
+static int conv_pair_launch_t(const CUtensorMap &ma0, const CUtensorMap &ma1, const CUtensorMap &mw0, const CUtensorMap &mw1,
+                              void *y16, int64_t n, const msw::ConvGnParams &gp, int max_ctas, cudaStream_t stream)
+{
+    using namespace msw;
+    using K = cvp::Cfg<CIN>;
+    MSW_SET_MAX_SMEM((conv3x3_pair_kernel<GN, CIN, EPI>), K::SMEM_BYTES);
+    int sms = sm_count();
+    if (max_ctas > 0 && max_ctas < sms) sms = max_ctas;
+    const long long pairs_max = sms / 2 > 0 ? sms / 2 : 1;
+    const long long pairs = n < pairs_max ? n : pairs_max;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(2 * pairs), 1, 1);
+    cfg.blockDim = dim3(cvp::THREADS, 1, 1);
+    cfg.dynamicSmemBytes = K::SMEM_BYTES;
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 2;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    MSW_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv3x3_pair_kernel<GN, CIN, EPI>, ma0, ma1, mw0, mw1, (__half *)y16, (long long)n, gp));
+    MSW_CUDA_TRY(cudaGetLastError());
+    return MSW_OK;
+}
+
 // Shared host side of msw_conv3x3 / msw_conv3x3_gn: argument checks, the four tensor maps, the launch.
+// C = 96 (Cin 96 or 16): conv3x3_tc_kernel, one CTA per board; C = 128 (Cin 128 or 16): conv3x3_pair_kernel.
 static int conv_launch(const char *who, const void *x16, const void *w_taps16, void *y16, int64_t n, int32_t H, int32_t W,
                        int32_t Cin, int32_t C, const msw::ConvGnParams *gn, int max_ctas, void *stream)
 {
     using namespace msw;
     if (!x16 || !w_taps16 || !y16) return fail(MSW_ERR_NULL, "%s: NULL pointer", who);
-    if (H != 16 || W != 16 || C != cv::C || (Cin != 96 && Cin != 16))
-        return fail(MSW_ERR_BAD_SHAPE, "%s: only 16x16 boards, 96 output and 96 or 16 input channels (got %dx%d, %d -> %d)", who, H,
-                    W, Cin, C);
+    if (H != 16 || W != 16 || (C != cv::C && C != cvp::C) || (Cin != C && Cin != 16))
+        return fail(MSW_ERR_BAD_SHAPE, "%s: only 16x16 boards, 96 or 128 output channels and as many or 16 input channels (got %dx%d, %d -> %d)",
+                    who, H, W, Cin, C);
     if (n < 0 || n > 0x3fffffffLL) return fail(MSW_ERR_BAD_SHAPE, "%s: n=%lld", who, (long long)n);
     if ((((uintptr_t)x16 | (uintptr_t)w_taps16 | (uintptr_t)y16) & 31u) != 0)
         return fail(MSW_ERR_ALIGN, "%s: tensors must be 32-byte aligned", who);
     if (n == 0) return MSW_OK;
     if (!tensor_map_encoder_available()) return fail(MSW_ERR_ARG, "%s: cuTensorMapEncodeTiled is not available", who);
-    // first channel block: 64 channels / 128-byte swizzle (Cin = 96) or all 16 channels / 32-byte swizzle (Cin = 16);
-    // second block (Cin = 96 only): 32 channels / 64-byte swizzle
-    const cuuint32_t b0 = Cin == 96 ? 64u : 16u;
-    const CUtensorMapSwizzle sw0 = Cin == 96 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_32B;
+    const bool pair = C == cvp::C;
+    // first channel block: 64 channels / 128-byte swizzle (Cin = 96, 128) or all 16 channels / 32-byte swizzle (Cin = 16);
+    // second block: 32 channels / 64-byte swizzle (Cin = 96), channels 64..127 through the first block's maps (Cin = 128)
+    const cuuint32_t b0 = Cin == 16 ? 16u : 64u;
+    const CUtensorMapSwizzle sw0 = Cin == 16 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_128B;
+    // weight rows per tap and CTA: all C output channels, or half of them on a CTA pair
+    const cuuint32_t wrows = pair ? (cuuint32_t)cvp::HALF : (cuuint32_t)C;
     CUtensorMap ma0, ma1, mw0, mw1;
     {
         // activation [n][16][16][Cin] fp16: dims innermost first
@@ -473,19 +862,23 @@ static int conv_launch(const char *who, const void *x16, const void *w_taps16, v
         const cuuint64_t strides[3] = {(cuuint64_t)Cin * 2, (cuuint64_t)Cin * 2 * 16, (cuuint64_t)Cin * 2 * 256};
         const cuuint32_t box0[4] = {b0, 16, cv::ROWS_IN, 1}, box1[4] = {32, 16, cv::ROWS_IN, 1};
         const CUresult r0 = encode_tiled(&ma0, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, x16, dims, strides, box0, sw0);
-        const CUresult r1 = encode_tiled(&ma1, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, x16, dims, strides, box1, CU_TENSOR_MAP_SWIZZLE_64B);
-        if (r0 != CUDA_SUCCESS || (Cin == 96 && r1 != CUDA_SUCCESS))
+        const CUresult r1 = Cin == 96 ? encode_tiled(&ma1, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, x16, dims, strides, box1, CU_TENSOR_MAP_SWIZZLE_64B)
+                                      : CUDA_SUCCESS;
+        if (r0 != CUDA_SUCCESS || r1 != CUDA_SUCCESS)
             return fail(MSW_ERR_ARG, "%s: activation tensor map failed (%d, %d)", who, (int)r0, (int)r1);
+        if (Cin != 96) ma1 = ma0;
     }
     {
-        // weights [9 taps * 96 co][Cin] fp16
+        // weights [9 taps * C co][Cin] fp16
         const cuuint64_t dims[2] = {(cuuint64_t)Cin, (cuuint64_t)9 * C};
         const cuuint64_t strides[1] = {(cuuint64_t)Cin * 2};
-        const cuuint32_t box0[2] = {b0, (cuuint32_t)C}, box1[2] = {32, (cuuint32_t)C};
+        const cuuint32_t box0[2] = {b0, wrows}, box1[2] = {32, wrows};
         const CUresult r0 = encode_tiled(&mw0, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, w_taps16, dims, strides, box0, sw0);
-        const CUresult r1 = encode_tiled(&mw1, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, w_taps16, dims, strides, box1, CU_TENSOR_MAP_SWIZZLE_64B);
-        if (r0 != CUDA_SUCCESS || (Cin == 96 && r1 != CUDA_SUCCESS))
+        const CUresult r1 = Cin == 96 ? encode_tiled(&mw1, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, w_taps16, dims, strides, box1, CU_TENSOR_MAP_SWIZZLE_64B)
+                                      : CUDA_SUCCESS;
+        if (r0 != CUDA_SUCCESS || r1 != CUDA_SUCCESS)
             return fail(MSW_ERR_ARG, "%s: weight tensor map failed (%d, %d)", who, (int)r0, (int)r1);
+        if (Cin != 96) mw1 = mw0;
     }
 #ifdef MSW_DEV_KNOBS
     const char *dbg_env = getenv("MSW_CONV_DBG");          // tools/convgn_ablation.py only
@@ -496,6 +889,14 @@ static int conv_launch(const char *who, const void *x16, const void *w_taps16, v
     const ConvGnParams none = {};
     const ConvGnParams &gp = gn ? *gn : none;
     cudaStream_t st = (cudaStream_t)stream;
+    if (pair) {
+        if (!gn) return Cin == 128 ? conv_pair_launch_t<false, 128, 0>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st)
+                                   : conv_pair_launch_t<false, 16, 0>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
+        if (Cin == 16) return conv_pair_launch_t<true, 16, 0>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
+        if (!gp.res32) return conv_pair_launch_t<true, 128, 0>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
+        return gp.pool4 ? conv_pair_launch_t<true, 128, 2>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st)
+                        : conv_pair_launch_t<true, 128, 1>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
+    }
     if (!gn) return Cin == 96 ? conv_launch_t<false, 96, 0>(ma0, ma1, mw0, mw1, y16, n, dbg, gp, max_ctas, st)
                               : conv_launch_t<false, 16, 0>(ma0, ma1, mw0, mw1, y16, n, dbg, gp, max_ctas, st);
     if (Cin == 16) return conv_launch_t<true, 16, 0>(ma0, ma1, mw0, mw1, y16, n, dbg, gp, max_ctas, st);          // the stem has no residual
@@ -518,10 +919,10 @@ extern "C" int msw_conv3x3_gn(const void *x16, const void *w_taps16, const float
 {
     using namespace msw;
     if (!conv_bias || !gamma || !beta) return fail(MSW_ERR_NULL, "msw_conv3x3_gn: NULL pointer");
-    if (G != 6) return fail(MSW_ERR_BAD_SHAPE, "msw_conv3x3_gn: needs 6 groups of 16 channels (G=%d)", G);
+    if (G != (C == 128 ? 8 : 6)) return fail(MSW_ERR_BAD_SHAPE, "msw_conv3x3_gn: needs groups of 16 channels (C=%d, G=%d)", C, G);
     if (drop_p < 0.0f || drop_p >= 1.0f) return fail(MSW_ERR_ARG, "msw_conv3x3_gn: drop_p=%f", drop_p);
     if (drop_p > 0.0f && res32) return fail(MSW_ERR_ARG, "msw_conv3x3_gn: dropout is only defined on the no-residual path");
-    if (Cin != 96 && res32) return fail(MSW_ERR_ARG, "msw_conv3x3_gn: the residual path needs Cin = 96");
+    if (Cin != C && res32) return fail(MSW_ERR_ARG, "msw_conv3x3_gn: the residual path needs Cin = C");
     if (pool4 && (!res32 || y32)) return fail(MSW_ERR_ARG, "msw_conv3x3_gn: pool4 replaces y32 on the residual path");
     if (res32 && !pool4 && !y32) return fail(MSW_ERR_ARG, "msw_conv3x3_gn: the residual path writes y32 or pool4");
     if ((((uintptr_t)res32 | (uintptr_t)y32) & 31u) != 0)

@@ -193,4 +193,88 @@ __device__ __forceinline__ void tmem_ld32(unsigned taddr, uint32_t (&v)[32])
 }
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
+// ---------------------------------------------------------------------------
+// Clusters and CTA pairs (tcgen05 cta_group::2): two CTAs of a 2-CTA cluster share each MMA.  The leader
+// (rank 0) issues it; A rows 0..127 come from the leader's shared memory and rows 128..255 from the peer's at the
+// same address, B's N rows are split in halves the same way, and D rows 0..127 / 128..255 land in the leader's /
+// the peer's TMEM.  Barrier and shared-memory operands named `*_cluster` are shared::cluster addresses (mapa).
+// ---------------------------------------------------------------------------
+__device__ __forceinline__ unsigned cluster_ctarank()
+{
+    unsigned r;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+    return r;
+}
+// the shared::cluster address of this CTA's shared address `addr` in CTA `rank` of the cluster
+__device__ __forceinline__ unsigned mapa_shared(unsigned addr, unsigned rank)
+{
+    unsigned r;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
+    return r;
+}
+// all threads of all CTAs of the cluster (release / acquire)
+__device__ __forceinline__ void cluster_sync()
+{
+    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void mbar_expect_tx_cluster(unsigned bar_cluster, unsigned bytes)
+{
+    asm volatile("mbarrier.arrive.expect_tx.release.cluster.shared::cluster.b64 _, [%0], %1;" :: "r"(bar_cluster), "r"(bytes) : "memory");
+}
+// releases this thread's earlier writes (st_shared_cluster included) to whoever waits on the barrier
+__device__ __forceinline__ void mbar_arrive_cluster(unsigned bar_cluster)
+{
+    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" :: "r"(bar_cluster) : "memory");
+}
+// mbar_wait with cluster-scope acquire: for barriers other CTAs of the cluster arrive on
+__device__ __forceinline__ void mbar_wait_cluster(unsigned bar, unsigned parity)
+{
+    unsigned done = 0;
+    while (!done)
+        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
+                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+}
+__device__ __forceinline__ void st_shared_cluster_v4(unsigned addr_cluster, float4 v)
+{
+    asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" :: "r"(addr_cluster), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
+                 : "memory");
+}
+// TMA loads of a CTA pair: destination in this CTA's shared memory, completion on a barrier of either CTA
+__device__ __forceinline__ void tma_load_2d_pair(unsigned dst, const CUtensorMap *map, int c0, int c1, unsigned bar_cluster)
+{
+    asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
+                 :: "r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar_cluster) : "memory");
+}
+__device__ __forceinline__ void tma_load_4d_pair(unsigned dst, const CUtensorMap *map, int c0, int c1, int c2, int c3,
+                                                 unsigned bar_cluster)
+{
+    asm volatile("cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
+                 :: "r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(bar_cluster) : "memory");
+}
+// umma_f16_masked for the pair (M = 256): bit i of mask word w set = row 32w + i of the 256-row D is not written
+__device__ __forceinline__ void umma_f16_masked_pair(unsigned d_tmem, uint64_t a, uint64_t b, unsigned idesc, unsigned accumulate,
+                                                     unsigned mask)
+{
+    asm volatile("{ .reg .pred p; setp.ne.b32 p, %4, 0; tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, "
+                 "{%5, %5, %5, %5, %5, %5, %5, %5}, p; }"
+                 :: "r"(d_tmem), "l"(a), "l"(b), "r"(idesc), "r"(accumulate), "r"(mask) : "memory");
+}
+// arrive on the barrier at shared address `bar` in BOTH CTAs of the pair once the pair MMAs issued before complete
+__device__ __forceinline__ void umma_commit_pair(unsigned bar)
+{
+    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+                 :: "r"(bar), "h"((unsigned short)3) : "memory");
+}
+// tmem_alloc / tmem_dealloc for a pair: one warp of EACH CTA calls them, the columns are the same in both
+__device__ __forceinline__ void tmem_alloc_pair(unsigned dst, unsigned cols)
+{
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(dst), "r"(cols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc_pair(unsigned tmem, unsigned cols)
+{
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(cols) : "memory");
+}
+
 }  // namespace msw

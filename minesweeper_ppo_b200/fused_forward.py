@@ -1,5 +1,5 @@
 """Inference-only forward of `CNNResidualPolicy` for rollouts (SURVEY section 8, row f4): at the medium
-config's shape every convolution is a tcgen05 kernel with GroupNorm / ReLU / Dropout2d / the fp32 residual add
+config's shape (96 channels) and the package's default shape (128 channels) every convolution is a tcgen05 kernel with GroupNorm / ReLU / Dropout2d / the fp32 residual add
 fused into its epilogue (msw_conv3x3_gn); other shapes use fp16 NHWC library convolutions with ONE fused kernel
 (msw_gn_act) between them instead of the eager GroupNorm / ReLU / Dropout2d / residual-add / dtype-cast kernels.
 
@@ -96,18 +96,20 @@ def conv3x3(x16: torch.Tensor, taps16: torch.Tensor) -> torch.Tensor:
 
 
 def to_p8(x: torch.Tensor) -> torch.Tensor:
-    """fp32 [N, 96, 16, 16] (any memory format) -> the private "P8" order of the fused trunk's residual stream:
-    [N][tile 2][channel third 3][8-channel chunk 4][pixel 128][8] (msw_conv_tc.cu).  Test / tooling helper."""
+    """fp32 [N, C, 16, 16] (C = 96 or 128, any memory format) -> the private "P8" order of the fused trunk's
+    residual stream: [N][tile 2][32-channel slice C/32][8-channel chunk 4][pixel 128][8] (msw_conv_tc.cu; the
+    slices are the epilogue's warpgroups).  Test / tooling helper."""
     n, c, h, w = x.shape
-    assert (c, h, w) == (96, 16, 16)
-    t = x.permute(0, 2, 3, 1).reshape(n, 2, 128, 3, 4, 8)          # [N][tile][pixel][third][chunk][8]
+    assert c in (96, 128) and (h, w) == (16, 16)
+    t = x.permute(0, 2, 3, 1).reshape(n, 2, 128, c // 32, 4, 8)    # [N][tile][pixel][slice][chunk][8]
     return t.permute(0, 1, 3, 4, 2, 5).contiguous()
 
 
 def from_p8(t: torch.Tensor) -> torch.Tensor:
-    """Inverse of `to_p8`: -> fp32 [N, 96, 16, 16] (channels_last storage)."""
+    """Inverse of `to_p8`: -> fp32 [N, C, 16, 16] (channels_last storage); C from the tensor's size."""
     n = t.shape[0]
-    x = t.reshape(n, 2, 3, 4, 128, 8).permute(0, 1, 4, 2, 3, 5).reshape(n, 16, 16, 96)
+    c = t.numel() // (n * 256)
+    x = t.reshape(n, 2, c // 32, 4, 128, 8).permute(0, 1, 4, 2, 3, 5).reshape(n, 16, 16, c)
     return x.permute(0, 3, 1, 2)
 
 
@@ -129,8 +131,9 @@ def conv3x3_gn(x16: torch.Tensor, taps16: torch.Tensor, norm: torch.nn.GroupNorm
         raise ValueError("conv3x3_gn: residual must be a contiguous fp32 tensor in P8 order")
     dev = x16.device
     y16 = torch.empty((N, C, H, W), dtype=torch.float16, device=dev, memory_format=torch.channels_last)
-    y32 = torch.empty((N, 2, 3, 4, 128, 8), dtype=torch.float32, device=dev) if (want32 and not want_pool) else None
-    pool4 = torch.empty((N, 4, C), dtype=torch.float32, device=dev) if want_pool else None
+    y32 = torch.empty((N, 2, C // 32, 4, 128, 8), dtype=torch.float32, device=dev) if (want32 and not want_pool) else None
+    # pooled partial sums: per row quarter (C = 96: one CTA per board), per tile and row quarter (C = 128: a CTA pair)
+    pool4 = torch.empty((N, 8 if C == 128 else 4, C), dtype=torch.float32, device=dev) if want_pool else None
     with torch.cuda.device(dev):
         rc = L.msw_conv3x3_gn(x16.data_ptr(), taps16.data_ptr(), conv_bias.data_ptr(),
                               None if res32 is None else res32.data_ptr(), norm.weight.data_ptr(), norm.bias.data_ptr(),
@@ -149,8 +152,8 @@ class FusedRolloutForward:
     """Callable with the module's `(obs, return_mine)` signature, for use under torch.no_grad().
 
     Two shape classes, chosen once at construction (no run-time switches):
-      * the medium config's shape (96 channels, 6 groups, 16x16 boards, <= 16 observation planes): every
-        convolution runs on tcgen05 with GroupNorm / ReLU / Dropout2d / the fp32 residual add / the value head's
+      * the medium config's shape (96 channels, 6 groups) and the package's default shape (128 channels, 8 groups;
+        each convolution on a CTA pair), on 16x16 boards with <= 16 observation planes: every convolution runs on tcgen05 with GroupNorm / ReLU / Dropout2d / the fp32 residual add / the value head's
         average pool fused into its epilogue (msw_pack_obs16 -> 11 x msw_conv3x3_gn -> msw_cell_heads); the fp32
         residual stream lives in the kernels' private P8 order and no library convolution is on the path;
       * any other CNNResidualPolicy shape: library (cuDNN) fp16 NHWC convolutions with the fused GroupNorm kernel
@@ -168,7 +171,7 @@ class FusedRolloutForward:
         self.model, self.seed, self.calls = model, int(seed), 0
         self.sample_id_base = int(sample_id_base)     # global index of row 0 (env shard offset): keys the Dropout2d stream
         self.epoch: Optional[torch.Tensor] = None     # device uint32 counter mixed into the dropout RNG (graph replays)
-        self.tc_trunk = C == 96 and G == 6 and model.stem[0].in_channels <= 16 and len(model.residual_stack) >= 1
+        self.tc_trunk = (C, G) in ((96, 6), (128, 8)) and model.stem[0].in_channels <= 16 and len(model.residual_stack) >= 1
         # grid cap of the persistent conv kernels (0 = one CTA per SM): a collector that runs two populations on two
         # streams gives each half the SMs, so an HBM-bound residual layer of one runs beside an MMA-bound layer of the other
         self.max_ctas = int(max_ctas)
@@ -247,7 +250,7 @@ class FusedRolloutForward:
         return float(blk.dropout.p) if (self.model.training and isinstance(blk.dropout, torch.nn.Dropout2d)) else 0.0
 
     def _trunk_tc(self, obs: torch.Tensor, cid: int):
-        """Medium-config shape: 11 msw_conv3x3_gn launches; returns (a16 NHWC, pooled fp32 [N, C])."""
+        """tcgen05 shapes: 1 + 2 * blocks msw_conv3x3_gn launches; returns (a16 NHWC, pooled fp32 [N, C])."""
         m = self.model
         base, max_ctas = self.sample_id_base, self.max_ctas
         nb, cin, hh, ww = obs.shape
@@ -295,8 +298,8 @@ class FusedRolloutForward:
             FusedRolloutForward._warned.add(key)
             import sys
             print(f"[minesweeper_ppo_b200] FusedRolloutForward: shape C={key[0]} G={key[1]} obs={key[2]} is outside the "
-                  "tcgen05 trunk (96 channels, 6 groups, 16x16 boards): convolutions run in cuDNN with the fused "
-                  "GroupNorm kernel between them", file=sys.stderr, flush=True)
+                  "tcgen05 trunk (96 channels and 6 groups or 128 channels and 8 groups, 16x16 boards): convolutions "
+                  "run in cuDNN with the fused GroupNorm kernel between them", file=sys.stderr, flush=True)
         if self.stem16 is not None and obs.dtype == torch.float32 and obs.is_contiguous():
             nb, cin, hh, ww = obs.shape
             x = torch.empty((nb, 16, hh, ww), dtype=torch.float16, device=obs.device, memory_format=torch.channels_last)
