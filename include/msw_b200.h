@@ -353,6 +353,27 @@ int msw_conv3x3_gn(const void *x16, const void *w_taps16, const float *conv_bias
                    uint64_t seed, uint64_t call_id, const uint32_t *epoch, int64_t sample_id_base, int32_t max_ctas,
                    void *stream);
 
+/* The whole rollout forward of the three-convolution baseline policy (policy.CNNPolicy, build_model("cnn"):
+ * conv 3x3 -> ReLU -> GroupNorm(4, 32) -> conv 3x3 -> ReLU -> GroupNorm(8, 64) -> conv 3x3 -> ReLU, then the 1x1
+ * policy and mine heads and the value head's average pool) on 16x16 boards in one persistent tcgen05 launch, with
+ * the roundings of the fp16 autocast forward (train_rl.py:222-227): each convolution accumulates in fp32, adds its
+ * bias and rounds once to fp16; GroupNorm runs in fp32 on the fp16 ReLU output and is rounded to fp16 as the next
+ * convolution's input.
+ * x16: fp16 NHWC [n][16][16][16] (msw_pack_obs16's layout: observation planes, missing channels zero).
+ * wK_taps16: fp16 [9][Cout][Cin], tap = ky*3 + kx of the module's weight (conv1's input channels padded to 16 with
+ * zeros).  bK, gammaK, betaK: fp32 conv biases and GroupNorm affine.  wp16 / wm16: fp16 [64] weights of the 1x1
+ * policy / mine heads, bp16 / bm16 their fp16 biases (one value each).
+ * Writes fp16 logits16 [n][256] and mine16 [n][256] (the heads, fp32 sums over the 64 channels) and pooled16
+ * [n][64] (the mean over the board of the fp16 feature map, summed in a fixed order).
+ * Only H = W = 16, Cin = 16, widths C1 / C2 / C3 = 32 / 64 / 64 and groups G1 / G2 = 4 / 8; anything else is
+ * MSW_ERR_BAD_SHAPE.  x16, the taps, the fp32 vectors and wp16 / wm16 must be 16-byte aligned. */
+int msw_cnn_forward(const void *x16, const void *w1_taps16, const float *b1, const float *gamma1, const float *beta1,
+                    const void *w2_taps16, const float *b2, const float *gamma2, const float *beta2,
+                    const void *w3_taps16, const float *b3, const void *wp16, const void *bp16, const void *wm16,
+                    const void *bm16, void *logits16, void *mine16, void *pooled16, int64_t n, int32_t H, int32_t W,
+                    int32_t Cin, int32_t C1, int32_t G1, int32_t C2, int32_t G2, int32_t C3, float eps1, float eps2,
+                    void *stream);
+
 /* Backward of msw_gn_act for the training forward.  save_mean / save_rstd
  * ([n][G]) and save_mask ([n][HW][C/8], bit k = channel 8j+k passed ReLU and
  * Dropout2d) come from the forward call (all three nullable there, given

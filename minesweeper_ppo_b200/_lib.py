@@ -79,6 +79,7 @@ SIGNATURES = {
                               C.c_void_p]),
     "msw_conv3x3_gn": (C.c_int, [C.c_void_p] * 9 + [C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float,
                                  C.c_float, C.c_uint64, C.c_uint64, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
+    "msw_cnn_forward": (C.c_int, [C.c_void_p] * 18 + [C.c_int64] + [C.c_int32] * 8 + [C.c_float, C.c_float, C.c_void_p]),
     "msw_gn_act_bwd": (C.c_int, [C.c_void_p] * 13 + [C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_void_p]),
     "msw_late_start": (C.c_int, [_P(EnvDesc), _P(State), C.c_int64, C.c_void_p, C.c_uint64, C.c_float, C.c_int32,
                                  C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),

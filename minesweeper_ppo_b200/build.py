@@ -16,7 +16,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 INCLUDE = os.path.join(os.path.dirname(PKG), "include")
 LIB = os.path.join(PKG, "libmsw_b200.so")
-SOURCES = ["msw_capi.cu", "msw_env.cu", "msw_gae.cu", "msw_sampler.cu", "msw_gn.cu", "msw_heads.cu", "msw_heads_tc.cu", "msw_conv_tc.cu", "msw_avoid.cu", "msw_eval.cu", "msw_host_expand.cpp"]
+SOURCES = ["msw_capi.cu", "msw_env.cu", "msw_gae.cu", "msw_sampler.cu", "msw_gn.cu", "msw_heads.cu", "msw_heads_tc.cu", "msw_conv_tc.cu", "msw_cnn_fwd.cu", "msw_avoid.cu", "msw_eval.cu", "msw_host_expand.cpp"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

@@ -1,4 +1,7 @@
-"""Inference-only forward of `CNNResidualPolicy` for rollouts (SURVEY section 8, row f4): at the medium
+"""Inference-only rollout forwards: `FusedRolloutForward` for `CNNResidualPolicy` and `FusedCnnForward` for the
+three-convolution baseline `CNNPolicy` (build_model("cnn")); `make_rollout_forward` picks one.
+
+`FusedRolloutForward` (SURVEY section 8, row f4): at the medium
 config's shape (96 channels) and the package's default shape (128 channels) every convolution is a tcgen05 kernel with GroupNorm / ReLU / Dropout2d / the fp32 residual add
 fused into its epilogue (msw_conv3x3_gn); other shapes use fp16 NHWC library convolutions with ONE fused kernel
 (msw_gn_act) between them instead of the eager GroupNorm / ReLU / Dropout2d / residual-add / dtype-cast kernels.
@@ -17,7 +20,7 @@ import torch
 import torch.nn.functional as F
 
 from . import _lib
-from .policy import CNNResidualPolicy
+from .policy import CNNPolicy, CNNResidualPolicy
 
 
 def gn_act(x16: torch.Tensor, norm: torch.nn.GroupNorm, *, conv_bias: Optional[torch.Tensor] = None,
@@ -333,3 +336,124 @@ class FusedRolloutForward:
         else:
             a16, pooled = self._trunk_library(obs, cid)
         return self._heads(a16, pooled, return_mine)
+
+
+def cnn_forward(x16: torch.Tensor, taps: Tuple[torch.Tensor, torch.Tensor, torch.Tensor], vecs: Tuple[torch.Tensor, ...],
+                heads16: torch.Tensor, head_bias16: torch.Tensor, eps: Tuple[float, float]
+                ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """msw_cnn_forward: x16 fp16 [N, 16, 16, 16] channels_last (msw_pack_obs16's layout); taps = the fp16 tap-major
+    weights [9, 32, 16], [9, 64, 32], [9, 64, 64]; vecs = fp32 (b1, gamma1, beta1, b2, gamma2, beta2, b3);
+    heads16 fp16 [2, 64] (policy, mine weights), head_bias16 fp16 [2].  Returns fp16 (logits [N, 256],
+    mine [N, 256], pooled [N, 64])."""
+    L = _lib.load()
+    N, cin, H, W = x16.shape
+    if x16.dtype != torch.float16 or not x16.is_contiguous(memory_format=torch.channels_last):
+        raise ValueError("cnn_forward: x must be fp16 channels_last")
+    dev = x16.device
+    logits = torch.empty((N, H * W), dtype=torch.float16, device=dev)
+    mine = torch.empty((N, H * W), dtype=torch.float16, device=dev)
+    pooled = torch.empty((N, taps[2].shape[1]), dtype=torch.float16, device=dev)
+    b1, g1, be1, b2, g2, be2, b3 = vecs
+    with torch.cuda.device(dev):
+        rc = L.msw_cnn_forward(x16.data_ptr(), taps[0].data_ptr(), b1.data_ptr(), g1.data_ptr(), be1.data_ptr(),
+                               taps[1].data_ptr(), b2.data_ptr(), g2.data_ptr(), be2.data_ptr(), taps[2].data_ptr(),
+                               b3.data_ptr(), heads16[0].data_ptr(), head_bias16[0:1].data_ptr(), heads16[1].data_ptr(),
+                               head_bias16[1:2].data_ptr(), logits.data_ptr(), mine.data_ptr(), pooled.data_ptr(), N, H, W,
+                               cin, taps[0].shape[1], 4, taps[1].shape[1], 8, taps[2].shape[1], float(eps[0]),
+                               float(eps[1]), torch.cuda.current_stream(dev).cuda_stream)
+    _lib.check(rc, "msw_cnn_forward")
+    return logits, mine, pooled
+
+
+class FusedCnnForward:
+    """Rollout forward of the three-convolution baseline `CNNPolicy` (build_model("cnn")), with the module's
+    `(obs, return_mine)` signature, for use under torch.no_grad().
+
+    On 16x16 boards with <= 16 observation planes (fp32, contiguous) the whole network up to the value MLP is one
+    msw_cnn_forward launch after msw_pack_obs16: the three convolutions, both GroupNorms, the 1x1 policy / mine heads
+    and the average pool, with the roundings of the fp16 autocast forward.  The value MLP (Linear -> ReLU -> Linear)
+    runs in torch fp16 on the pooled features.  Any other input runs the module itself under fp16 autocast.
+
+    The fp16 / fp32 parameter copies are allocated once and updated in place by `refresh()`, so their addresses are
+    stable and the forward can be captured in a CUDA graph.  Conv and head biases are rounded to fp16 first, as
+    autocast casts them.  `epoch` and `sample_id_base` are set by the collector like on `FusedRolloutForward`;
+    this network has no dropout, so nothing reads them."""
+
+    def __init__(self, model: CNNPolicy, seed: int = 0, sample_id_base: int = 0):
+        if not isinstance(model, CNNPolicy):
+            raise TypeError("FusedCnnForward supports CNNPolicy only")
+        self.model, self.seed = model, int(seed)
+        self.sample_id_base = int(sample_id_base)
+        self.epoch: Optional[torch.Tensor] = None
+        self.cin = model.backbone[0].in_channels
+        self._w = None
+        self.refresh()
+
+    @staticmethod
+    def supports(model) -> bool:
+        return isinstance(model, CNNPolicy) and model.backbone[0].in_channels <= 16
+
+    @torch.no_grad()
+    def refresh(self) -> None:
+        m = self.model
+        conv = (m.backbone[0], m.backbone[3], m.backbone[6])
+        norm = (m.backbone[2], m.backbone[5])
+        if self._w is None:
+            dev = conv[0].weight.device
+            self.taps = tuple(torch.zeros((9, c.out_channels, 16 if k == 0 else c.in_channels), dtype=torch.float16, device=dev)
+                              for k, c in enumerate(conv))
+            self.vecs = tuple(torch.empty((n,), dtype=torch.float32, device=dev) for n in (32, 32, 32, 64, 64, 64, 64))
+            self.heads16 = torch.empty((2, 64), dtype=torch.float16, device=dev)
+            self.head_bias16 = torch.empty((2,), dtype=torch.float16, device=dev)
+            v1, v2 = m.value_head[2], m.value_head[4]
+            self.value = [(torch.empty_like(l.weight, dtype=torch.float16), torch.empty_like(l.bias, dtype=torch.float16))
+                          for l in (v1, v2)]
+            self._w = True
+        for t, c in zip(self.taps, conv):
+            t[:, :, :c.in_channels].copy_(c.weight.permute(2, 3, 0, 1).reshape(9, c.out_channels, c.in_channels))
+        b1, g1, be1, b2, g2, be2, b3 = self.vecs
+        for dst, c in ((b1, conv[0]), (b2, conv[1]), (b3, conv[2])):
+            dst.copy_(c.bias.to(torch.float16))
+        g1.copy_(norm[0].weight); be1.copy_(norm[0].bias)
+        g2.copy_(norm[1].weight); be2.copy_(norm[1].bias)
+        self.heads16[0].copy_(m.policy_head.weight.reshape(-1)); self.heads16[1].copy_(m.mine_head.weight.reshape(-1))
+        self.head_bias16[0:1].copy_(m.policy_head.bias); self.head_bias16[1:2].copy_(m.mine_head.bias)
+        for (w, b), l in zip(self.value, (m.value_head[2], m.value_head[4])):
+            w.copy_(l.weight)
+            b.copy_(l.bias)
+
+    def fused_input(self, obs: torch.Tensor) -> bool:
+        return (obs.is_cuda and obs.dim() == 4 and obs.dtype == torch.float32 and obs.is_contiguous()
+                and obs.shape[1] == self.cin and tuple(obs.shape[2:]) == (16, 16))
+
+    @torch.no_grad()
+    def __call__(self, obs: torch.Tensor, return_mine: bool = False):
+        if not self.fused_input(obs):
+            with torch.autocast("cuda", dtype=torch.float16):
+                return self.model(obs, return_mine=return_mine)
+        nb, cin, hh, ww = obs.shape
+        x = torch.empty((nb, 16, hh, ww), dtype=torch.float16, device=obs.device, memory_format=torch.channels_last)
+        with torch.cuda.device(obs.device):
+            _lib.check(_lib.load().msw_pack_obs16(obs.data_ptr(), x.data_ptr(), nb, cin, hh * ww,
+                                                  torch.cuda.current_stream(obs.device).cuda_stream), "msw_pack_obs16")
+        norm = (self.model.backbone[2], self.model.backbone[5])
+        logits, mine, pooled = cnn_forward(x, self.taps, self.vecs, self.heads16, self.head_bias16,
+                                           (norm[0].eps, norm[1].eps))
+        v = F.relu_(F.linear(pooled, *self.value[0]))
+        value = F.linear(v, *self.value[1]).squeeze(-1)
+        if not return_mine:
+            return logits, value
+        return logits, value, mine.reshape(nb, 1, hh, ww)
+
+
+def supports_fused(model) -> bool:
+    """True when `make_rollout_forward` has a hand-written forward for `model` (the collector's fused path and
+    graph capture)."""
+    return FusedRolloutForward.supports(model) or FusedCnnForward.supports(model)
+
+
+def make_rollout_forward(model, seed: int = 0, sample_id_base: int = 0):
+    """The rollout forward for `model`: FusedCnnForward for a CNNPolicy, FusedRolloutForward otherwise."""
+    if isinstance(model, CNNPolicy):
+        return FusedCnnForward(model, seed=seed, sample_id_base=sample_id_base)
+    return FusedRolloutForward(model, seed=seed, sample_id_base=sample_id_base)

@@ -22,7 +22,7 @@ import torch.nn as nn
 from . import _lib
 from .buffers import CompactRolloutBuffer, RolloutBuffer
 from .env import StepOut, VecMinesweeper
-from .fused_forward import FusedRolloutForward
+from .fused_forward import make_rollout_forward, supports_fused
 
 _DTYPE_CODE = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
 
@@ -82,7 +82,7 @@ class RolloutCollector:
         self.actions32 = torch.empty((N,), dtype=torch.int32, device=dev)
         self.sample_seed = int(sample_seed)
         self.rollouts_done = 0
-        self.fused = bool(fused)          # use FusedRolloutForward when the model supports it
+        self.fused = bool(fused)          # use the hand-written forward (make_rollout_forward) when the model has one
         self._fused_fwd = None
         # graph=True: the WHOLE rollout (reset, T x (forward, sample, step), bootstrap forward, weight
         # refresh) is captured once into a CUDA graph and replayed -- one launch per rollout instead of
@@ -103,15 +103,16 @@ class RolloutCollector:
 
     @staticmethod
     def can_graph(model: nn.Module) -> bool:
-        """graph=True needs the fused forward, i.e. a CNNResidualPolicy with 8 | channels-per-group."""
-        return FusedRolloutForward.supports(model)
+        """graph=True needs a fused forward: a CNNResidualPolicy with 8 | channels-per-group, or a CNNPolicy with
+        <= 16 input planes."""
+        return supports_fused(model)
 
     @torch.no_grad()
     def collect(self, model: nn.Module, autocast: bool = True) -> Tuple[RolloutBuffer, Dict]:
         if not self.use_graph:
             return self._collect(model, autocast)
-        if not (self.fused and autocast and FusedRolloutForward.supports(model)):
-            raise ValueError("graph=True needs the fused forward (CNNResidualPolicy, fused=True, CUDA autocast)")
+        if not (self.fused and autocast and supports_fused(model)):
+            raise ValueError("graph=True needs the fused forward (CNNResidualPolicy or CNNPolicy, fused=True, CUDA autocast)")
         key = self._graph_key(model, autocast)
         if self._graph is None or self._graph_key_captured != key:
             side = torch.cuda.Stream(device=self.vec.device)
@@ -142,9 +143,9 @@ class RolloutCollector:
         ctx = (lambda: torch.autocast(device_type="cuda", dtype=torch.float16)) if autocast else nullcontext
         base_step = self.rollouts_done * (T + 1)
         fwd = model
-        if self.fused and autocast and FusedRolloutForward.supports(model):
+        if self.fused and autocast and supports_fused(model):
             if self._fused_fwd is None or self._fused_fwd.model is not model:
-                self._fused_fwd = FusedRolloutForward(model, seed=self.sample_seed, sample_id_base=vec._desc.env_id_base)
+                self._fused_fwd = make_rollout_forward(model, seed=self.sample_seed, sample_id_base=vec._desc.env_id_base)
                 self._fused_fwd.epoch = self._epoch
             self._fused_fwd.refresh()                         # weights may have been updated since
             fwd, ctx = self._fused_fwd, nullcontext
