@@ -48,8 +48,8 @@ def is_stale() -> bool:
 
 
 def build_dev(out_path: str) -> str:
-    """Development build for tools/ only: the same sources with -DMSW_DEV_KNOBS (launch-shape sweeps, epilogue
-    ablation switches), written to `out_path` -- never to the product library's path."""
+    """Development build for tools/ only: the same sources with -DMSW_DEV_KNOBS (launch-shape sweeps), written to
+    `out_path` -- never to the product library's path."""
     srcs = [os.path.join(CSRC, s) for s in SOURCES]
     cmd = [_nvcc(), *[f for f in NVCC_FLAGS if f not in ("-Xptxas", "-v")], "-DMSW_DEV_KNOBS", "-I", INCLUDE, "-o", out_path, *srcs]
     env = dict(os.environ)

@@ -14,9 +14,8 @@
 //
 // All 27 weight taps stay resident in shared memory (119,808 B), and a board's activations never leave it: only
 // the 16-channel observation (msw_pack_obs16's fp16 NHWC layout) comes in and only the logits, mine logits and
-// pooled features go out.  Every convolution is msw_conv_tc.cu's scheme: per 128-pixel tile (8 image rows) nine
-// shifted-descriptor taps accumulate into one TMEM accumulator, and the disable-output-lane mask switches off the
-// rows whose horizontal neighbour is off the board.  A board's activation is stored with a zero halo row above and
+// pooled features go out.  Every convolution is msw_conv.cuh's conv3x3_mmas, once per 128-pixel tile (8 image
+// rows).  A board's activation is stored with a zero halo row above and
 // below (18 rows x 16 px, K-major, swizzled), so the vertical padding is those rows: the TMA box of the observation
 // starts at y = -1 and the tensor map zero-fills rows -1 and 16; the epilogues write the next layer's operand into
 // rows 1..16 and keep rows 0 and 17 zero.
@@ -50,6 +49,7 @@
 // epilogue.
 //
 #include "../../include/msw_b200.h"
+#include "msw_conv.cuh"
 #include "msw_error.h"
 #include "msw_sm100.cuh"
 
@@ -87,13 +87,6 @@ struct CnnParams {
     float eps1, eps2;
 };
 
-__device__ __forceinline__ float cnn_warp_sum(float v)           // fixed shuffle tree: deterministic
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-
 // 16 bytes of a read-only parameter vector.  volatile: the compiler would otherwise hoist the (loop-invariant)
 // bias / affine / head-weight loads out of the board loop and keep ~300 values live across it, spilling.
 __device__ __forceinline__ uint4 cnn_ld16(const void *p)
@@ -117,24 +110,8 @@ __device__ __forceinline__ void cnn_conv_mmas(unsigned d0, unsigned a, unsigned 
     // occupy ~250 registers
     asm volatile("" : "+r"(d0), "+r"(a), "+r"(w));
 #pragma unroll
-    for (int t = 0; t < 2; ++t) {
-        unsigned accumulate = 0u;
-#pragma unroll
-        for (int dy = 0; dy < 3; ++dy)
-#pragma unroll
-            for (int o = 0; o < 3; ++o) {
-                const int dxi = o == 0 ? 1 : o == 1 ? 0 : 2;               // the unmasked centre tap first
-                const int tap = dy * 3 + dxi;
-                const unsigned mask = dxi == 0 ? 0x00010001u : dxi == 2 ? 0x80008000u : 0u;
-                const unsigned sa = a + (unsigned)(((t * 8 + dy) * cnn::HW_W + dxi - 1) * (int)ROW);
-#pragma unroll
-                for (int k = 0; k < KS; ++k) {
-                    umma_f16_masked(d0 + 64u * t, umma_desc<ROW>(sa) + 2u * k, umma_desc<ROW>(w + tap * wtap) + 2u * k,
-                                    idesc, accumulate, mask);
-                    accumulate = 1u;
-                }
-            }
-    }
+    for (int t = 0; t < 2; ++t)
+        conv3x3_mmas<ROW, KS, 0u, 0, false>(d0 + 64u * t, a + (unsigned)(t * 8 * cnn::HW_W * (int)ROW), 0u, w, 0u, wtap, 0u, idesc);
 }
 
 // 16 accumulator columns of this thread's pixel (TMEM address `taddr`, channels c0 .. c0 + 15, `bias` = &b[c0])
@@ -169,11 +146,12 @@ __device__ __forceinline__ void cnn_group_partial(const uint32_t *h4, float *st,
         s1 += d0 + d1;
         s2 = fmaf(d0, d0, fmaf(d1, d1, s2));
     }
-    s1 = cnn_warp_sum(s1);
-    s2 = cnn_warp_sum(s2);
+    s1 = warp_sum(s1);
+    s2 = warp_sum(s2);
     if (lane == 0) {
-        st[0] = shift + s1 * (1.0f / 256.0f);
-        st[1] = s2 - s1 * s1 * (1.0f / 256.0f);
+        const float2 ms = mean_m2<256>(shift, s1, s2);
+        st[0] = ms.x;
+        st[1] = ms.y;
     }
 }
 
@@ -185,10 +163,7 @@ __device__ __forceinline__ float2 cnn_group_stats(const float *stat, int g, floa
 #pragma unroll
     for (int w = 0; w < 8; ++w) {
         const float2 pw = *reinterpret_cast<const float2 *>(stat + (w * 8 + g) * 2);
-        const float nn = na + 256.0f, delta = pw.x - mg, r = 256.0f / nn;
-        mg = fmaf(delta, r, mg);
-        m2 += pw.y + delta * delta * (na * r);
-        na = nn;
+        chan_step(na, mg, m2, 256.0f, pw.x, pw.y);
     }
     return make_float2(mg, rsqrtf(m2 * (1.0f / 2048.0f) + eps));
 }

@@ -42,6 +42,19 @@ __device__ __forceinline__ void philox4x32_10(uint32_t k0, uint32_t k1, uint32_t
     out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
 }
 
+// Dropout2d's draw for (global board gb, 8-channel chunk): channel 8 * chunk + k is dropped when
+// dropout2d_u16(w, k) < (uint32_t)(p * 65536).  Keyed by the GLOBAL board, so masks do not depend on sharding;
+// call id and the nullable device epoch (added per graph replay) give every forward fresh masks.
+__device__ __forceinline__ void dropout2d_draw(uint32_t k0, uint32_t k1, long long gb, uint32_t chunk, uint32_t call_lo,
+                                               uint32_t call_hi, const uint32_t *epoch, uint32_t (&w)[4])
+{
+    philox4x32_10(k0, k1 ^ 0x44524f50u, (uint32_t)gb, (uint32_t)(gb >> 32) ^ chunk, call_lo, call_hi + (epoch ? *epoch : 0u), w);
+}
+__device__ __forceinline__ uint32_t dropout2d_u16(const uint32_t (&w)[4], int k)
+{
+    return (w[k >> 1] >> (16 * (k & 1))) & 0xFFFFu;
+}
+
 // Window shifts.  win_shl: bit j of the result is flat bit (32*lane + j - s);
 // win_shr: flat bit (32*lane + j + s).  0 <= s <= 33; for s == 33 (W == 32 only)
 // the one bit that would come from two lanes away belongs to a cell the column

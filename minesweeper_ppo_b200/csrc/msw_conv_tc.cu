@@ -1,29 +1,20 @@
-// msw_conv_tc.cu -- 3x3 "same" convolution of the policy trunk (96 -> 96 channels on 16x16 boards, and the stem's
-// 16 -> 96; fp16 NHWC in, fp32 accumulate, fp16 NHWC out) on the 5th-generation tensor cores, plain
-// (conv3x3_tc_kernel<false>: no bias, it is folded into msw_gn_act) or with GroupNorm / ReLU / Dropout2d /
-// residual add (and the value head's average pool) fused into the epilogue (conv3x3_tc_kernel<true>).
-// 128 -> 128 channels (and the stem's 16 -> 128) run on conv3x3_pair_kernel below: one board per CTA pair.
+// msw_conv_tc.cu -- 3x3 "same" convolution of the policy trunk on 16x16 boards (fp16 NHWC in, fp32 accumulate, fp16
+// NHWC out) on the 5th-generation tensor cores, plain (GN = false: no bias, it is folded into msw_gn_act) or with
+// GroupNorm / ReLU / Dropout2d / residual add (and the value head's average pool) fused into the epilogue (GN = true).
+//   * 96 -> 96 channels and the stem's 16 -> 96: conv3x3_tc_kernel, one board per CTA;
+//   * 128 -> 128 channels and the stem's 16 -> 128: conv3x3_pair_kernel below, one board per CTA pair.
+// The shifted-descriptor / edge-mask scheme of the nine taps, the GroupNorm statistics, the pooled-sum butterfly and
+// the P8 order of the fp32 residual stream are in msw_conv.cuh; the mbarrier / TMA / tcgen05 wrappers in msw_sm100.cuh.
 //
-// out[y][x][co] = sum_{dy,dx,ci} in[y+dy][x+dx][ci] * w[co][ci][dy][dx] is computed as nine shifted GEMMs
-// per 128-pixel tile (8 image rows of one board) that all accumulate into ONE TMEM accumulator.  The tile's
-// input rows y0-1 .. y0+8 sit in shared memory as one linear [160 pixel][96 ch] block (a single 4-D TMA box;
-// rows above / below the board are zero-filled by the tensor map), and a tap is nothing but a different
-// shared-memory descriptor on that block:
-//   * the A operand of tap (dy, dx) starts (dy+1) * 16 + dx pixels into the block.  The swizzle is a function
-//     of the absolute shared-memory address (measured: descriptors whose start is shifted by whole 128- or
-//     64-byte rows give exact results with the matrix base offset left at 0), so no second copy and no im2col;
-//   * a horizontal shift drags the neighbouring image row's edge pixel into the rows with x = 0 (dx = -1) or
-//     x = 15 (dx = +1); those rows of D are switched off for that tap with tcgen05.mma's disable-output-lane
-//     mask, which is exactly the zero padding.  The first tap issued is the unmasked centre column, so every
-//     row of the accumulator is initialised.
-// All nine [96 x 96] weight taps stay resident in shared memory (162 KB, loaded once per persistent CTA);
-// the activation streams through a 2-stage ring.  K = 96 = one 64-channel block (128-byte swizzle) + one
-// 32-channel block (64-byte swizzle).  Roles: warp 0 TMA producer, warp 1 MMA issuer (54 tcgen05.mma of
-// 128 x 96 x 16 per tile into a ring of four 96-column accumulators), warp 2 TMEM allocation, warps 4-15
-// epilogue (thread = pixel, each warpgroup a third of the channels).  The mbarrier / TMA / tcgen05 wrappers are in
-// msw_sm100.cuh.
+// conv3x3_tc_kernel: all nine [96 x 96] weight taps stay resident in shared memory (162 KB, loaded once per persistent
+// CTA); the activation streams through a 2-stage ring of [10 rows x 16 px x 96 ch] blocks (a single 4-D TMA box; rows
+// above / below the board are zero-filled by the tensor map).  K = 96 = one 64-channel block (128-byte swizzle) + one
+// 32-channel block (64-byte swizzle).  Roles: warp 0 TMA producer, warp 1 MMA issuer (54 tcgen05.mma of 128 x 96 x 16
+// per tile into a ring of four 96-column accumulators), warp 2 TMEM allocation, warps 4-15 epilogue (thread = pixel,
+// each warpgroup a third of the channels).
 #include "../../include/msw_b200.h"
 #include "msw_common.cuh"
+#include "msw_conv.cuh"
 #include "msw_error.h"
 #include "msw_sm100.cuh"
 
@@ -32,14 +23,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
-#include <stdlib.h>
-
-// Ablation switches for tools/convgn_ablation.py: compiled in only with -DMSW_DEV_KNOBS (the product library has none).
-#ifdef MSW_DEV_KNOBS
-#define MSW_DBG(bit) ((dbg & (bit)) != 0)
-#else
-#define MSW_DBG(bit) false
-#endif
 
 namespace msw {
 
@@ -71,16 +54,10 @@ struct Cfg {
 };
 }  // namespace cv
 
-// What the fused GroupNorm epilogue needs (conv3x3_tc_kernel<true>); same meaning as msw_gn_act's arguments.
-//
-// The fp32 residual stream (res32 in, y32 out) is private to this kernel family, so it lives in HBM in the order
-// the epilogue touches it -- "P8": [board][tile 2][channel third 3][8-channel chunk 4][pixel 128][8 floats].  A
-// thread (= pixel) owns one 32-byte chunk per (third, chunk); the 32 lanes of a warp are 32 consecutive pixels,
-// so every 256-bit load / store instruction of a warp covers 1 KB of consecutive addresses (8 full lines)
-// instead of one line per lane as the pixel-major NHWC order would (32 lines per instruction: the epilogue was
-// LSU-bound at 690 us per layer with it, against 240 us of MMAs).
+// What the fused GroupNorm epilogue needs (GN = true); same meaning as msw_gn_act's arguments.  The fp32 residual
+// stream (res32 in, y32 out) is private to this kernel family, so it is kept in the P8 order of msw_conv.cuh.
 struct ConvGnParams {
-    const float *cbias, *gamma, *beta;   // [96]
+    const float *cbias, *gamma, *beta;   // [C]
     const float *res32;                  // nullable, P8 order
     float *y32;                          // nullable, P8 order
     float *pool4;                        // nullable [n][4][96]: per row-quarter sums of the fp32 output (value head's avg pool)
@@ -89,29 +66,6 @@ struct ConvGnParams {
     const uint32_t *epoch;               // nullable
     long long sample_base;               // global index of board 0 (Dropout2d stream is keyed by the global board)
 };
-
-// float offset of (board, tile, third, chunk, pixel-in-tile) in the P8 order
-__device__ __forceinline__ long long cv_p8(long long board, int half, int third, int c4, int pp)
-{
-    return ((((board * 2 + half) * 3 + third) * 4 + c4) * 128 + pp) * 8;
-}
-
-__device__ __forceinline__ void cv_st256(void *p, const uint32_t (&v)[8])
-{
-    asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
-                 :: "l"(p), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]) : "memory");
-}
-__device__ __forceinline__ void cv_ld256(const void *p, uint32_t (&v)[8])
-{
-    asm volatile("ld.global.v8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]) : "l"(p));
-}
-__device__ __forceinline__ float cv_warp_sum(float v)          // fixed shuffle tree: deterministic
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
 
 // GN = false: out = conv(x) (fp16).  GN = true: out = relu(GroupNorm(conv(x) + bias) [+ res]) [* Dropout2d], the
 // whole inter-convolution step of msw_gn_act fused into the epilogue (6 groups of 16 channels; statistics over
@@ -122,7 +76,7 @@ template <bool GN, int CIN, int EPI>
 __global__ void __launch_bounds__(cv::THREADS, 1)
 conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_constant__ CUtensorMap map_a1,
                   const __grid_constant__ CUtensorMap map_w0, const __grid_constant__ CUtensorMap map_w1,
-                  __half *__restrict__ out, long long boards, int dbg, const __grid_constant__ ConvGnParams gp)
+                  __half *__restrict__ out, long long boards, const __grid_constant__ ConvGnParams gp)
 {
     using namespace cv;
     using K = Cfg<CIN>;
@@ -185,31 +139,7 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
             tcgen05_fence_after();
             const unsigned a0 = base + OFF_A + s * A_STAGE, a1 = a0 + A0_BYTES, d = tmem + acc * C;
             if (elect_one()) {            // the whole warp runs the loop and the waits; one elected lane issues
-            unsigned accumulate = 0u;
-            if (!MSW_DBG(8))
-#pragma unroll
-            for (int dy = 0; dy < 3; ++dy)
-#pragma unroll
-                for (int o = 0; o < 3; ++o) {
-                    const int dxi = o == 0 ? 1 : o == 1 ? 0 : 2;           // the unmasked centre tap first
-                    const int tap = dy * 3 + dxi;
-                    // rows of D whose horizontal neighbour is off the board: x = 0 for dx = -1, x = 15 for dx = +1
-                    const unsigned mask = dxi == 0 ? 0x00010001u : dxi == 2 ? 0x80008000u : 0u;
-                    const unsigned sa0 = a0 + (unsigned)((dy * HW_W + dxi - 1) * (int)K::ROW0);
-                    const unsigned sa1 = a1 + (unsigned)((dy * HW_W + dxi - 1) * (int)K::ROW1);
-#pragma unroll
-                    for (int k = 0; k < K::KS0; ++k) {                       // first channel block, 16 channels (32 bytes) per step
-                        umma_f16_masked(d, umma_desc<K::ROW0>(sa0) + 2u * k, umma_desc<K::ROW0>(base + OFF_W0 + tap * W0_TAP) + 2u * k,
-                                        idesc, accumulate, mask);
-                        accumulate = 1u;
-                    }
-                    if constexpr (K::KS1 > 0) {
-#pragma unroll
-                        for (int k = 0; k < K::KS1; ++k)                     // second channel block
-                            umma_f16_masked(d, umma_desc<K::ROW1>(sa1) + 2u * k,
-                                            umma_desc<K::ROW1>(base + OFF_W1 + tap * W1_TAP) + 2u * k, idesc, 1u, mask);
-                    }
-                }
+            conv3x3_mmas<K::ROW0, K::KS0, K::ROW1, K::KS1, false>(d, a0, a1, base + OFF_W0, base + OFF_W1, W0_TAP, W1_TAP, idesc);
             umma_commit(empty(s));           // the smem stage is free once these MMAs have read it
             umma_commit(tfull(acc));         // ... and the accumulator is complete
             }
@@ -225,33 +155,15 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
             const unsigned acc = it % ACC, aph = (it / ACC) & 1u;
             mbar_wait(tfull(acc), aph);
             tcgen05_fence_after();
-            uint32_t v[32];
-            {
-                uint32_t lo[16], hi[16];
-                const unsigned taddr = tmem + ((unsigned)(q * 32) << 16) + acc * C + third * 32;
-                tmem_ld16(taddr, lo);
-                tmem_ld16(taddr + 16, hi);
-                tmem_wait_ld();
-#pragma unroll
-                for (int j = 0; j < 16; ++j) { v[j] = lo[j]; v[16 + j] = hi[j]; }
-            }
+            uint32_t lo[16], hi[16];
+            const unsigned taddr = tmem + ((unsigned)(q * 32) << 16) + acc * C + third * 32;
+            tmem_ld16(taddr, lo);
+            tmem_ld16(taddr + 16, hi);
+            tmem_wait_ld();
             tcgen05_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(tempty(acc));       // the accumulator is in registers: release it
-            if (MSW_DBG(1)) continue;
-            __half *dst = out + (board * 256 + (it & 1u) * 128 + q * 32 + lane) * (long long)C + third * 32;
-#pragma unroll
-            for (int c0 = 0; c0 < 32; c0 += 16) {
-                uint32_t packed[8];
-#pragma unroll
-                for (int k = 0; k < 8; ++k) {
-                    const __half2 hh = __floats2half2_rn(__uint_as_float(v[c0 + 2 * k]), __uint_as_float(v[c0 + 2 * k + 1]));
-                    packed[k] = *reinterpret_cast<const uint32_t *>(&hh);
-                }
-                // one 256-bit store per lane: the lanes of a warp write to 32 different 128-byte lines either way
-                // (pixels are 192 B apart), so the LSU cost is per instruction, not per byte
-                cv_st256(dst + c0, packed);
-            }
+            store_half32(out + (board * 256 + (it & 1u) * 128 + q * 32 + lane) * (long long)C + third * 32, lo, hi);
         }
         } else {
         // ---- fused GroupNorm epilogue.  Thread = pixel, its 32 channels = groups 2*third and 2*third + 1.
@@ -273,22 +185,16 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
             float sc = gp.drop_scale;
             if (EPI == 0 && te < C && gp.drop_p > 0.0f) {
                 uint32_t w[4];
-                const long long gb = gp.sample_base + board;
-                philox4x32_10(gp.k0, gp.k1 ^ 0x44524f50u, (uint32_t)gb, (uint32_t)(gb >> 32) ^ (uint32_t)(te >> 3), gp.call_lo,
-                              gp.call_hi + (gp.epoch ? *gp.epoch : 0u), w);
-                const int k = te & 7;
-                const uint32_t u16 = (w[k >> 1] >> (16 * (k & 1))) & 0xFFFFu;
-                if (u16 < thresh) sc = 0.0f;
+                dropout2d_draw(gp.k0, gp.k1, gp.sample_base + board, (uint32_t)(te >> 3), gp.call_lo, gp.call_hi, gp.epoch, w);
+                if (dropout2d_u16(w, te & 7) < thresh) sc = 0.0f;
             }
             uint32_t h[2][16];                       // fp16-rounded conv output of both tiles (the reference's rounding point)
-            // One-pass statistics of v = x + bias, shifted by a value of the warp's own data (no cancellation in
-            // S2 - S1^2/n): per thread S1 = sum (v - shift), S2 = sum (v - shift)^2 for its two groups.
-            float shift0 = 0.0f, shift1 = 0.0f, s1a = 0.0f, s2a = 0.0f, s1b = 0.0f, s2b = 0.0f;
+            GnSums sums = {};
 #pragma unroll
             for (int half = 0; half < 2; ++half) {
                 const unsigned it = 2u * bi + half, acc = it % ACC, aph = (it / ACC) & 1u;
                 if (EPI != 0)     // the 16 KB of residual stream this warpgroup will read for this tile: one line per thread on its way to L2
-                    asm volatile("prefetch.global.L2 [%0];" :: "l"(gp.res32 + cv_p8(board, half, third, 0, 0) + (q * 32 + lane) * 32));
+                    asm volatile("prefetch.global.L2 [%0];" :: "l"(gp.res32 + p8_offset<3>(board, half, third, 0, 0) + (q * 32 + lane) * 32));
                 mbar_wait(tfull(acc), aph);
                 tcgen05_fence_after();
                 uint32_t lo[16], hi[16];
@@ -299,38 +205,18 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
                 tcgen05_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(tempty(acc));
-                if (MSW_DBG(16)) continue;
-#pragma unroll
-                for (int jj = 0; jj < 16; ++jj) {
-                    const uint32_t *src = jj < 8 ? lo : hi;
-                    const __half2 hh = __floats2half2_rn(__uint_as_float(src[(2 * jj) & 15]), __uint_as_float(src[(2 * jj + 1) & 15]));
-                    h[half][jj] = *reinterpret_cast<const uint32_t *>(&hh);
-                    const float2 f = __half22float2(hh), cb = cb2[jj];
-                    const float v0 = f.x + cb.x, v1 = f.y + cb.y;
-                    if (half == 0 && jj == 0) shift0 = __shfl_sync(0xffffffffu, v0, 0);
-                    if (half == 0 && jj == 8) shift1 = __shfl_sync(0xffffffffu, v0, 0);
-                    if (jj < 8) {
-                        const float d0 = v0 - shift0, d1 = v1 - shift0;
-                        s1a += d0 + d1;
-                        s2a = fmaf(d0, d0, fmaf(d1, d1, s2a));
-                    } else {
-                        const float d0 = v0 - shift1, d1 = v1 - shift1;
-                        s1b += d0 + d1;
-                        s2b = fmaf(d0, d0, fmaf(d1, d1, s2b));
-                    }
-                }
+                gn_accumulate32(lo, hi, cb2, half == 0, h[half], sums);
             }
-            if (MSW_DBG(16)) continue;
             // the warp's (mean, M2) over its 1,024 values per group; the board's statistics are merged from the four
-            // row-owning warps of a channel third in a fixed order (Chan et al.)
-            s1a = cv_warp_sum(s1a); s2a = cv_warp_sum(s2a);
-            s1b = cv_warp_sum(s1b); s2b = cv_warp_sum(s2b);
+            // row-owning warps of a channel third in a fixed order
+            const float s1a = warp_sum(sums.s1[0]), s2a = warp_sum(sums.s2[0]), s1b = warp_sum(sums.s1[1]), s2b = warp_sum(sums.s2[1]);
             if (lane == 0) {
+                const float2 st0 = mean_m2<1024>(sums.shift[0], s1a, s2a), st1 = mean_m2<1024>(sums.shift[1], s1b, s2b);
                 float *dst = s_part + (par * 12 + we) * 4;
-                dst[0] = shift0 + s1a * (1.0f / 1024.0f); dst[1] = s2a - s1a * s1a * (1.0f / 1024.0f);
-                dst[2] = shift1 + s1b * (1.0f / 1024.0f); dst[3] = s2b - s1b * s1b * (1.0f / 1024.0f);
+                dst[0] = st0.x; dst[1] = st0.y;
+                dst[2] = st1.x; dst[3] = st1.y;
             }
-            if (!MSW_DBG(2)) asm volatile("bar.sync 1, 384;" ::: "memory");
+            asm volatile("bar.sync 1, 384;" ::: "memory");
             if (te < C) {
                 // one thread per channel folds statistics, affine, conv bias and the Dropout2d scale into y = a*x + b
                 const int c = te, gsel = (c >> 4) & 1, w4 = (c >> 5) * 4;
@@ -338,23 +224,19 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
 #pragma unroll
                 for (int qq = 0; qq < 4; ++qq) {
                     const float *src = s_part + (par * 12 + w4 + qq) * 4 + 2 * gsel;
-                    const float nn = na + 1024.0f, delta = src[0] - mg, w = 1024.0f / nn;
-                    mg = fmaf(delta, w, mg);
-                    m2 += src[1] + delta * delta * (na * w);
-                    na = nn;
+                    chan_step(na, mg, m2, 1024.0f, src[0], src[1]);
                 }
-                const float rg = rsqrtf(m2 * (1.0f / 4096.0f) + gp.eps);       // biased variance, eps as torch
-                const float a = gp.gamma[c] * rg;
-                s_ab[(par * 2 + 0) * C + c] = a * sc;
-                s_ab[(par * 2 + 1) * C + c] = fmaf(s_cb[c] - mg, a, gp.beta[c]) * sc;
+                const float2 ab = gn_fold<4096>(mg, m2, gp.eps, gp.gamma[c], gp.beta[c], s_cb[c], sc);
+                s_ab[(par * 2 + 0) * C + c] = ab.x;
+                s_ab[(par * 2 + 1) * C + c] = ab.y;
             }
-            if (!MSW_DBG(2)) asm volatile("bar.sync 1, 384;" ::: "memory");
+            asm volatile("bar.sync 1, 384;" ::: "memory");
             // ---- normalise, (+ residual), ReLU, store: chunk by chunk (8 channels), both tiles per chunk
             const float4 *a4 = reinterpret_cast<const float4 *>(s_ab + (par * 2 + 0) * C + cbase);
             const float4 *b4 = reinterpret_cast<const float4 *>(s_ab + (par * 2 + 1) * C + cbase);
             const int pp = q * 32 + lane;
             uint32_t rnext[8];                       // residual values of the next (chunk, tile): loaded one step ahead
-            if (EPI != 0) cv_ld256(gp.res32 + cv_p8(board, 0, third, 0, pp), rnext);
+            if (EPI != 0) ld256(gp.res32 + p8_offset<3>(board, 0, third, 0, pp), rnext);
 #pragma unroll
             for (int c0 = 0; c0 < 32; c0 += 8) {
                 const float4 aa0 = a4[c0 >> 2], aa1 = a4[(c0 >> 2) + 1], bb0 = b4[c0 >> 2], bb1 = b4[(c0 >> 2) + 1];
@@ -367,8 +249,8 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
                     if (EPI != 0) {
 #pragma unroll
                         for (int k = 0; k < 8; ++k) rr[k] = rnext[k];
-                        if (half == 0) cv_ld256(gp.res32 + cv_p8(board, 1, third, c0 >> 3, pp), rnext);
-                        else if (c0 < 24) cv_ld256(gp.res32 + cv_p8(board, 0, third, (c0 >> 3) + 1, pp), rnext);
+                        if (half == 0) ld256(gp.res32 + p8_offset<3>(board, 1, third, c0 >> 3, pp), rnext);
+                        else if (c0 < 24) ld256(gp.res32 + p8_offset<3>(board, 0, third, (c0 >> 3) + 1, pp), rnext);
                     }
                     uint32_t o[8];
 #pragma unroll
@@ -384,29 +266,17 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
                             ps[j + 1] = half == 0 ? v1 : ps[j + 1] + v1;
                         }
                     }
-                    if (EPI != 2 && gp.y32 && !MSW_DBG(1)) cv_st256(gp.y32 + cv_p8(board, half, third, c0 >> 3, pp), o);
+                    if (EPI != 2 && gp.y32) st256(gp.y32 + p8_offset<3>(board, half, third, c0 >> 3, pp), o);
 #pragma unroll
                     for (int k = 0; k < 4; ++k) {
                         const __half2 hh = __floats2half2_rn(__uint_as_float(o[2 * k]), __uint_as_float(o[2 * k + 1]));
                         h[half][(c0 >> 1) + k] = *reinterpret_cast<const uint32_t *>(&hh);     // reuse the slot for the output
                     }
                 }
-                if (EPI == 2) {
-                    // warp sum of 8 channels over the 32 lanes in 9 shuffles (fixed butterfly: deterministic): each
-                    // step halves the number of channels a lane carries; lane L ends with channel bit4*4 + bit3*2 + bit2
-                    const bool b4s = lane & 16, b3s = lane & 8, b2s = lane & 4;
-                    float a1[4], a2[2], a3;
-#pragma unroll
-                    for (int i = 0; i < 4; ++i)
-                        a1[i] = (b4s ? ps[4 + i] : ps[i]) + __shfl_xor_sync(0xffffffffu, b4s ? ps[i] : ps[4 + i], 16);
-#pragma unroll
-                    for (int i = 0; i < 2; ++i)
-                        a2[i] = (b3s ? a1[2 + i] : a1[i]) + __shfl_xor_sync(0xffffffffu, b3s ? a1[i] : a1[2 + i], 8);
-                    a3 = (b2s ? a2[1] : a2[0]) + __shfl_xor_sync(0xffffffffu, b2s ? a2[0] : a2[1], 4);
-                    a3 += __shfl_xor_sync(0xffffffffu, a3, 2);
-                    a3 += __shfl_xor_sync(0xffffffffu, a3, 1);
-                    if ((lane & 3) == 0)
-                        gp.pool4[(board * 4 + q) * C + cbase + c0 + (b4s ? 4 : 0) + (b3s ? 2 : 0) + (b2s ? 1 : 0)] = a3;
+                if (EPI == 2) {                      // the warp's sum of these 8 channels over its 32 pixels
+                    int ch;
+                    const float sum = pool8_butterfly(ps, lane, ch);
+                    if ((lane & 3) == 0) gp.pool4[(board * 4 + q) * C + cbase + c0 + ch] = sum;
                 }
             }
 #pragma unroll
@@ -417,7 +287,7 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
                     uint32_t packed[8];
 #pragma unroll
                     for (int k = 0; k < 8; ++k) packed[k] = h[half][(c0 >> 1) + k];
-                    if (!MSW_DBG(1)) cv_st256(out + px * C + cbase + c0, packed);
+                    st256(out + px * C + cbase + c0, packed);
                 }
             }
         }
@@ -440,9 +310,9 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
 // board (image rows 8r .. 8r + 7, i.e. input rows 8r - 1 .. 8r + 8: the same 4-D TMA box as above).  The leader
 // (rank 0) issues one cta_group::2 MMA per tap and k-step for both tiles (9 taps x 8 k-steps = 72 per board); A
 // rows 128 .. 255 are the peer's tile, B's 64 + 64 rows the two weight halves, and each CTA's TMEM receives its own
-// 128 pixels x all 128 output channels.  Taps, shifted descriptors and the disable-output-lane masks are those of
-// conv3x3_tc_kernel, the mask covering the 256 rows of the pair.  K = 128 = two 64-channel blocks (128-byte rows,
-// 128-byte swizzle; both through the same tensor map); the stem (CIN = 16) is as above.
+// 128 pixels x all 128 output channels.  The taps are msw_conv.cuh's conv3x3_mmas in its pair form.  K = 128 = two
+// 64-channel blocks (128-byte rows, 128-byte swizzle; both through the same tensor map); the stem (CIN = 16) is as
+// above.
 //
 // GroupNorm statistics of a board span both tiles.  Every epilogue warp writes its (mean, M2) of its two groups
 // into its own CTA's exchange area AND the partner's (st.shared::cluster), then arrives on the partner's xfull
@@ -460,7 +330,7 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
 // Roles: warp 0 TMA producer (both CTAs), warp 1 MMA issuer (leader), warp 2 TMEM allocation (both), warps 4-19
 // epilogue (thread = pixel of the CTA's tile, warpgroup g = channels [32g, 32g + 32): groups 2g and 2g + 1).
 namespace cvp {
-constexpr int C = 128, HALF = 64, HW_W = 16, TILE_PX = 128, PX_IN = 160;
+constexpr int C = 128, HALF = 64, TILE_PX = 128, PX_IN = 160;
 constexpr int THREADS = 640, EPI_WARPS = 16, STAGES = 2, ACC = 4, TMEM_COLS = 512;    // 4 x 128 accumulator columns
 
 template <int CIN>
@@ -485,12 +355,6 @@ struct Cfg {
     static_assert(SMEM_BYTES <= 232448, "shared memory of one CTA");
 };
 }  // namespace cvp
-
-// float offset of (board, tile, quarter, chunk, pixel-in-tile) in the C = 128 P8 order
-__device__ __forceinline__ long long cvp_p8(long long board, int tile, int quarter, int c4, int pp)
-{
-    return ((((board * 2 + tile) * 4 + quarter) * 4 + c4) * 128 + pp) * 8;
-}
 
 // GN / CIN / EPI as conv3x3_tc_kernel; pool4 is [n][tile 2 x row quarter 4][128].
 template <bool GN, int CIN, int EPI>
@@ -567,29 +431,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_con
             tcgen05_fence_after();
             const unsigned a0 = base + OFF_A + s * A_STAGE, a1 = a0 + A0_BYTES, d = tmem + acc * C;
             if (elect_one()) {
-            unsigned accumulate = 0u;
-#pragma unroll
-            for (int dy = 0; dy < 3; ++dy)
-#pragma unroll
-                for (int o = 0; o < 3; ++o) {
-                    const int dxi = o == 0 ? 1 : o == 1 ? 0 : 2;           // the unmasked centre tap first
-                    const int tap = dy * 3 + dxi;
-                    const unsigned mask = dxi == 0 ? 0x00010001u : dxi == 2 ? 0x80008000u : 0u;
-                    const unsigned sa0 = a0 + (unsigned)((dy * HW_W + dxi - 1) * (int)K::ROW0);
-                    const unsigned sa1 = a1 + (unsigned)((dy * HW_W + dxi - 1) * (int)K::ROW1);
-#pragma unroll
-                    for (int k = 0; k < K::KS0; ++k) {
-                        umma_f16_masked_pair(d, umma_desc<K::ROW0>(sa0) + 2u * k,
-                                             umma_desc<K::ROW0>(base + K::OFF_W0 + tap * W0_TAP) + 2u * k, idesc, accumulate, mask);
-                        accumulate = 1u;
-                    }
-                    if constexpr (K::KS1 > 0) {
-#pragma unroll
-                        for (int k = 0; k < K::KS1; ++k)
-                            umma_f16_masked_pair(d, umma_desc<K::ROW1>(sa1) + 2u * k,
-                                                 umma_desc<K::ROW1>(base + K::OFF_W1 + tap * W1_TAP) + 2u * k, idesc, 1u, mask);
-                    }
-                }
+            conv3x3_mmas<K::ROW0, K::KS0, K::ROW1, K::KS1, true>(d, a0, a1, base + K::OFF_W0, base + K::OFF_W1, W0_TAP, W1_TAP, idesc);
             umma_commit_pair(empty(s));          // both CTAs' stage s is free once these MMAs have read it
             umma_commit_pair(tfull(acc));        // ... and both halves of the accumulator are complete
             }
@@ -612,18 +454,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_con
             tcgen05_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive_cluster(mapa_shared(tempty(acc), 0u));
-            __half *dst = out + (board * 256 + rank * 128 + pp) * (long long)C + cbase;
-#pragma unroll
-            for (int c0 = 0; c0 < 32; c0 += 16) {
-                const uint32_t *src = c0 == 0 ? lo : hi;
-                uint32_t packed[8];
-#pragma unroll
-                for (int k = 0; k < 8; ++k) {
-                    const __half2 hh = __floats2half2_rn(__uint_as_float(src[2 * k]), __uint_as_float(src[2 * k + 1]));
-                    packed[k] = *reinterpret_cast<const uint32_t *>(&hh);
-                }
-                cv_st256(dst + c0, packed);
-            }
+            store_half32(out + (board * 256 + rank * 128 + pp) * (long long)C + cbase, lo, hi);
         }
         } else {
         float *s_x = reinterpret_cast<float *>(smem_pair + K::OFF_X);    // [parity][tile][warp][mean0, M2_0, mean1, M2_1]
@@ -641,15 +472,11 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_con
             float sc = gp.drop_scale;            // Dropout2d: msw_gn_act's stream, keyed by global board and 8-channel chunk
             if (EPI == 0 && te < C && gp.drop_p > 0.0f) {
                 uint32_t w[4];
-                const long long gb = gp.sample_base + board;
-                philox4x32_10(gp.k0, gp.k1 ^ 0x44524f50u, (uint32_t)gb, (uint32_t)(gb >> 32) ^ (uint32_t)(te >> 3), gp.call_lo,
-                              gp.call_hi + (gp.epoch ? *gp.epoch : 0u), w);
-                const int k = te & 7;
-                const uint32_t u16 = (w[k >> 1] >> (16 * (k & 1))) & 0xFFFFu;
-                if (u16 < thresh) sc = 0.0f;
+                dropout2d_draw(gp.k0, gp.k1, gp.sample_base + board, (uint32_t)(te >> 3), gp.call_lo, gp.call_hi, gp.epoch, w);
+                if (dropout2d_u16(w, te & 7) < thresh) sc = 0.0f;
             }
             if (EPI != 0)     // the 16 KB of residual stream this warpgroup reads for this tile: one line per thread
-                asm volatile("prefetch.global.L2 [%0];" :: "l"(gp.res32 + cvp_p8(board, (int)rank, wg, 0, 0) + pp * 32));
+                asm volatile("prefetch.global.L2 [%0];" :: "l"(gp.res32 + p8_offset<4>(board, (int)rank, wg, 0, 0) + pp * 32));
             mbar_wait(tfull(acc), aph);
             tcgen05_fence_after();
             uint32_t lo[16], hi[16];
@@ -661,32 +488,13 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_con
             __syncwarp();
             if (lane == 0) mbar_arrive_cluster(mapa_shared(tempty(acc), 0u));
             uint32_t h[16];                      // fp16-rounded conv output (the reference's rounding point)
-            float shift0 = 0.0f, shift1 = 0.0f, s1a = 0.0f, s2a = 0.0f, s1b = 0.0f, s2b = 0.0f;
-#pragma unroll
-            for (int jj = 0; jj < 16; ++jj) {
-                const uint32_t *src = jj < 8 ? lo : hi;
-                const __half2 hh = __floats2half2_rn(__uint_as_float(src[(2 * jj) & 15]), __uint_as_float(src[(2 * jj + 1) & 15]));
-                h[jj] = *reinterpret_cast<const uint32_t *>(&hh);
-                const float2 f = __half22float2(hh), cb = cb2[jj];
-                const float v0 = f.x + cb.x, v1 = f.y + cb.y;
-                if (jj == 0) shift0 = __shfl_sync(0xffffffffu, v0, 0);
-                if (jj == 8) shift1 = __shfl_sync(0xffffffffu, v0, 0);
-                if (jj < 8) {
-                    const float d0 = v0 - shift0, d1 = v1 - shift0;
-                    s1a += d0 + d1;
-                    s2a = fmaf(d0, d0, fmaf(d1, d1, s2a));
-                } else {
-                    const float d0 = v0 - shift1, d1 = v1 - shift1;
-                    s1b += d0 + d1;
-                    s2b = fmaf(d0, d0, fmaf(d1, d1, s2b));
-                }
-            }
+            GnSums sums = {};
+            gn_accumulate32(lo, hi, cb2, true, h, sums);
             // the warp's (mean, M2) of its 512 values per group, into both CTAs' exchange areas
-            s1a = cv_warp_sum(s1a); s2a = cv_warp_sum(s2a);
-            s1b = cv_warp_sum(s1b); s2b = cv_warp_sum(s2b);
+            const float s1a = warp_sum(sums.s1[0]), s2a = warp_sum(sums.s2[0]), s1b = warp_sum(sums.s1[1]), s2b = warp_sum(sums.s2[1]);
             if (lane == 0) {
-                const float4 st = make_float4(shift0 + s1a * (1.0f / 512.0f), s2a - s1a * s1a * (1.0f / 512.0f),
-                                              shift1 + s1b * (1.0f / 512.0f), s2b - s1b * s1b * (1.0f / 512.0f));
+                const float2 st0 = mean_m2<512>(sums.shift[0], s1a, s2a), st1 = mean_m2<512>(sums.shift[1], s1b, s2b);
+                const float4 st = make_float4(st0.x, st0.y, st1.x, st1.y);
                 const unsigned slot = ((par * 2 + rank) * EPI_WARPS + we) * 16u;
                 *reinterpret_cast<float4 *>(smem_pair + K::OFF_X + slot) = st;
                 st_shared_cluster_v4(x_peer + slot, st);
@@ -704,22 +512,18 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_con
 #pragma unroll
                     for (int qq = 0; qq < 4; ++qq) {
                         const float *src = s_x + ((par * 2 + t) * EPI_WARPS + w4 + qq) * 4 + 2 * gsel;
-                        const float nn = na + 512.0f, delta = src[0] - mg, w = 512.0f / nn;
-                        mg = fmaf(delta, w, mg);
-                        m2 += src[1] + delta * delta * (na * w);
-                        na = nn;
+                        chan_step(na, mg, m2, 512.0f, src[0], src[1]);
                     }
-                const float rg = rsqrtf(m2 * (1.0f / 4096.0f) + gp.eps);
-                const float a = gp.gamma[c] * rg;
-                s_ab[c] = a * sc;
-                s_ab[C + c] = fmaf(s_cb[c] - mg, a, gp.beta[c]) * sc;
+                const float2 ab = gn_fold<4096>(mg, m2, gp.eps, gp.gamma[c], gp.beta[c], s_cb[c], sc);
+                s_ab[c] = ab.x;
+                s_ab[C + c] = ab.y;
             }
             asm volatile("bar.sync 1, 512;" ::: "memory");
             // ---- normalise, (+ residual), ReLU, store: 8 channels at a time
             const float4 *a4 = reinterpret_cast<const float4 *>(s_ab + cbase);
             const float4 *b4 = reinterpret_cast<const float4 *>(s_ab + C + cbase);
             uint32_t rnext[8];
-            if (EPI != 0) cv_ld256(gp.res32 + cvp_p8(board, (int)rank, wg, 0, pp), rnext);
+            if (EPI != 0) ld256(gp.res32 + p8_offset<4>(board, (int)rank, wg, 0, pp), rnext);
 #pragma unroll
             for (int c0 = 0; c0 < 32; c0 += 8) {
                 const float4 aa0 = a4[c0 >> 2], aa1 = a4[(c0 >> 2) + 1], bb0 = b4[c0 >> 2], bb1 = b4[(c0 >> 2) + 1];
@@ -729,7 +533,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_con
                 if (EPI != 0) {
 #pragma unroll
                     for (int k = 0; k < 8; ++k) rr[k] = rnext[k];
-                    if (c0 < 24) cv_ld256(gp.res32 + cvp_p8(board, (int)rank, wg, (c0 >> 3) + 1, pp), rnext);
+                    if (c0 < 24) ld256(gp.res32 + p8_offset<4>(board, (int)rank, wg, (c0 >> 3) + 1, pp), rnext);
                 }
                 uint32_t o[8];
 #pragma unroll
@@ -740,29 +544,19 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_con
                     o[j] = __float_as_uint(fmaxf(v0, 0.0f));
                     o[j + 1] = __float_as_uint(fmaxf(v1, 0.0f));
                 }
-                if (EPI != 2 && gp.y32) cv_st256(gp.y32 + cvp_p8(board, (int)rank, wg, c0 >> 3, pp), o);
+                if (EPI != 2 && gp.y32) st256(gp.y32 + p8_offset<4>(board, (int)rank, wg, c0 >> 3, pp), o);
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
                     const __half2 hh = __floats2half2_rn(__uint_as_float(o[2 * k]), __uint_as_float(o[2 * k + 1]));
                     h[(c0 >> 1) + k] = *reinterpret_cast<const uint32_t *>(&hh);
                 }
-                if (EPI == 2) {
-                    // warp sum of 8 channels over the 32 lanes (pixels), the fixed butterfly of conv3x3_tc_kernel
-                    const bool b4s = lane & 16, b3s = lane & 8, b2s = lane & 4;
-                    float a1[4], a2[2], a3;
+                if (EPI == 2) {                      // the warp's sum of these 8 channels over its 32 pixels
+                    float ps[8];
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const float lo4 = __uint_as_float(o[i]), hi4 = __uint_as_float(o[4 + i]);
-                        a1[i] = (b4s ? hi4 : lo4) + __shfl_xor_sync(0xffffffffu, b4s ? lo4 : hi4, 16);
-                    }
-#pragma unroll
-                    for (int i = 0; i < 2; ++i)
-                        a2[i] = (b3s ? a1[2 + i] : a1[i]) + __shfl_xor_sync(0xffffffffu, b3s ? a1[i] : a1[2 + i], 8);
-                    a3 = (b2s ? a2[1] : a2[0]) + __shfl_xor_sync(0xffffffffu, b2s ? a2[0] : a2[1], 4);
-                    a3 += __shfl_xor_sync(0xffffffffu, a3, 2);
-                    a3 += __shfl_xor_sync(0xffffffffu, a3, 1);
-                    if ((lane & 3) == 0)
-                        gp.pool4[(board * 8 + rank * 4 + q) * C + cbase + c0 + (b4s ? 4 : 0) + (b3s ? 2 : 0) + (b2s ? 1 : 0)] = a3;
+                    for (int k = 0; k < 8; ++k) ps[k] = __uint_as_float(o[k]);
+                    int ch;
+                    const float sum = pool8_butterfly(ps, lane, ch);
+                    if ((lane & 3) == 0) gp.pool4[(board * 8 + rank * 4 + q) * C + cbase + c0 + ch] = sum;
                 }
             }
             __half *dst = out + (board * 256 + rank * 128 + pp) * (long long)C + cbase;
@@ -771,7 +565,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_con
                 uint32_t packed[8];
 #pragma unroll
                 for (int k = 0; k < 8; ++k) packed[k] = h[(c0 >> 1) + k];
-                cv_st256(dst + c0, packed);
+                st256(dst + c0, packed);
             }
         }
         }
@@ -787,39 +581,27 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_con
 
 }  // namespace msw
 
-template <bool GN, int CIN, int EPI>
-static int conv_launch_t(const CUtensorMap &ma0, const CUtensorMap &ma1, const CUtensorMap &mw0, const CUtensorMap &mw1, void *y16,
-                         int64_t n, int dbg, const msw::ConvGnParams &gp, int max_ctas, cudaStream_t stream)
+// Launch of either family with the kernel for <GN, stem, EPI>: conv3x3_tc_kernel (C = 96, one CTA per board) or, for
+// `pair`, conv3x3_pair_kernel (C = 128) in clusters of 2, one board per cluster at a time, at most one cluster per two
+// SMs (the grid cap is rounded down to whole pairs).
+template <bool GN, bool STEM, int EPI>
+static int conv_launch_t(bool pair, const CUtensorMap &ma0, const CUtensorMap &ma1, const CUtensorMap &mw0, const CUtensorMap &mw1,
+                         void *y16, int64_t n, const msw::ConvGnParams &gp, int max_ctas, cudaStream_t stream)
 {
     using namespace msw;
-    using K = cv::Cfg<CIN>;
-    MSW_SET_MAX_SMEM((conv3x3_tc_kernel<GN, CIN, EPI>), K::SMEM_BYTES);
+    constexpr int CIN96 = STEM ? 16 : 96, CIN128 = STEM ? 16 : 128;
+    const unsigned smem = pair ? cvp::Cfg<CIN128>::SMEM_BYTES : cv::Cfg<CIN96>::SMEM_BYTES;
+    if (pair) MSW_SET_MAX_SMEM((conv3x3_pair_kernel<GN, CIN128, EPI>), smem);
+    else MSW_SET_MAX_SMEM((conv3x3_tc_kernel<GN, CIN96, EPI>), smem);
     int sms = sm_count();
     if (max_ctas > 0 && max_ctas < sms) sms = max_ctas;             // caller shares the GPU with a concurrent launch
-    const long long grid = n < sms ? n : sms;                       // persistent: whole boards per CTA
-    conv3x3_tc_kernel<GN, CIN, EPI><<<(unsigned)grid, cv::THREADS, K::SMEM_BYTES, stream>>>(ma0, ma1, mw0, mw1, (__half *)y16,
-                                                                                       (long long)n, dbg, gp);
-    MSW_CUDA_TRY(cudaGetLastError());
-    return MSW_OK;
-}
-
-// The CTA-pair kernel: clusters of 2, one board per cluster at a time, at most one cluster per two SMs (the
-// launch's grid cap is rounded down to an even count).
-template <bool GN, int CIN, int EPI>
-static int conv_pair_launch_t(const CUtensorMap &ma0, const CUtensorMap &ma1, const CUtensorMap &mw0, const CUtensorMap &mw1,
-                              void *y16, int64_t n, const msw::ConvGnParams &gp, int max_ctas, cudaStream_t stream)
-{
-    using namespace msw;
-    using K = cvp::Cfg<CIN>;
-    MSW_SET_MAX_SMEM((conv3x3_pair_kernel<GN, CIN, EPI>), K::SMEM_BYTES);
-    int sms = sm_count();
-    if (max_ctas > 0 && max_ctas < sms) sms = max_ctas;
-    const long long pairs_max = sms / 2 > 0 ? sms / 2 : 1;
-    const long long pairs = n < pairs_max ? n : pairs_max;
+    // persistent: whole boards per CTA (per CTA pair)
+    const long long units_max = pair ? (sms / 2 > 0 ? sms / 2 : 1) : sms;
+    const long long units = n < units_max ? n : units_max;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(2 * pairs), 1, 1);
-    cfg.blockDim = dim3(cvp::THREADS, 1, 1);
-    cfg.dynamicSmemBytes = K::SMEM_BYTES;
+    cfg.gridDim = dim3((unsigned)(pair ? 2 * units : units), 1, 1);
+    cfg.blockDim = dim3(pair ? cvp::THREADS : cv::THREADS, 1, 1);
+    cfg.dynamicSmemBytes = smem;
     cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
@@ -827,8 +609,9 @@ static int conv_pair_launch_t(const CUtensorMap &ma0, const CUtensorMap &ma1, co
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    MSW_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv3x3_pair_kernel<GN, CIN, EPI>, ma0, ma1, mw0, mw1, (__half *)y16, (long long)n, gp));
+    cfg.numAttrs = pair ? 1 : 0;
+    MSW_CUDA_TRY(cudaLaunchKernelEx(&cfg, pair ? conv3x3_pair_kernel<GN, CIN128, EPI> : conv3x3_tc_kernel<GN, CIN96, EPI>, ma0, ma1,
+                                    mw0, mw1, (__half *)y16, (long long)n, gp));
     MSW_CUDA_TRY(cudaGetLastError());
     return MSW_OK;
 }
@@ -880,29 +663,16 @@ static int conv_launch(const char *who, const void *x16, const void *w_taps16, v
             return fail(MSW_ERR_ARG, "%s: weight tensor map failed (%d, %d)", who, (int)r0, (int)r1);
         if (Cin != 96) mw1 = mw0;
     }
-#ifdef MSW_DEV_KNOBS
-    const char *dbg_env = getenv("MSW_CONV_DBG");          // tools/convgn_ablation.py only
-    const int dbg = dbg_env ? atoi(dbg_env) : 0;
-#else
-    const int dbg = 0;
-#endif
     const ConvGnParams none = {};
     const ConvGnParams &gp = gn ? *gn : none;
+    const bool stem = Cin == 16;
     cudaStream_t st = (cudaStream_t)stream;
-    if (pair) {
-        if (!gn) return Cin == 128 ? conv_pair_launch_t<false, 128, 0>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st)
-                                   : conv_pair_launch_t<false, 16, 0>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
-        if (Cin == 16) return conv_pair_launch_t<true, 16, 0>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
-        if (!gp.res32) return conv_pair_launch_t<true, 128, 0>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
-        return gp.pool4 ? conv_pair_launch_t<true, 128, 2>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st)
-                        : conv_pair_launch_t<true, 128, 1>(ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
-    }
-    if (!gn) return Cin == 96 ? conv_launch_t<false, 96, 0>(ma0, ma1, mw0, mw1, y16, n, dbg, gp, max_ctas, st)
-                              : conv_launch_t<false, 16, 0>(ma0, ma1, mw0, mw1, y16, n, dbg, gp, max_ctas, st);
-    if (Cin == 16) return conv_launch_t<true, 16, 0>(ma0, ma1, mw0, mw1, y16, n, dbg, gp, max_ctas, st);          // the stem has no residual
-    if (!gp.res32) return conv_launch_t<true, 96, 0>(ma0, ma1, mw0, mw1, y16, n, dbg, gp, max_ctas, st);
-    return gp.pool4 ? conv_launch_t<true, 96, 2>(ma0, ma1, mw0, mw1, y16, n, dbg, gp, max_ctas, st)
-                    : conv_launch_t<true, 96, 1>(ma0, ma1, mw0, mw1, y16, n, dbg, gp, max_ctas, st);
+    if (!gn) return stem ? conv_launch_t<false, true, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st)
+                         : conv_launch_t<false, false, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
+    if (stem) return conv_launch_t<true, true, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);      // the stem has no residual
+    if (!gp.res32) return conv_launch_t<true, false, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
+    return gp.pool4 ? conv_launch_t<true, false, 2>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st)
+                    : conv_launch_t<true, false, 1>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
 }
 
 extern "C" int msw_conv3x3(const void *x16, const void *w_taps16, void *y16, int64_t n, int32_t H, int32_t W,

@@ -167,9 +167,7 @@ __global__ void __launch_bounds__(256, 4) gn_act_kernel(const GnParams p, long l
             float a[8], b[8];
             uint32_t kept = 0xFFu;                                    // channels that survive Dropout2d
             uint32_t w[4] = {0u, 0u, 0u, 0u};
-            if (p.drop_p > 0.0f)
-                philox4x32_10(p.k0, p.k1 ^ 0x44524f50u, (uint32_t)(n + p.sample_base),
-                              (uint32_t)((n + p.sample_base) >> 32) ^ (uint32_t)j, p.call_lo, p.call_hi + (p.epoch ? *p.epoch : 0u), w);
+            if (p.drop_p > 0.0f) dropout2d_draw(p.k0, p.k1, n + p.sample_base, (uint32_t)j, p.call_lo, p.call_hi, p.epoch, w);
             const uint32_t thresh = (uint32_t)(p.drop_p * 65536.0f);
 #pragma unroll
             for (int k = 0; k < 8; ++k) {
@@ -179,7 +177,7 @@ __global__ void __launch_bounds__(256, 4) gn_act_kernel(const GnParams p, long l
                 if (p.drop_p > 0.0f) {
                     // relu(z)*s == relu(z*s) for s >= 0, so the mask/scale folds into the affine when no
                     // residual is added (Dropout2d follows ReLU only on that path, cnn_residual.py:20-21)
-                    const uint32_t u16 = (w[k >> 1] >> (16 * (k & 1))) & 0xFFFFu;
+                    const uint32_t u16 = dropout2d_u16(w, k);
                     const float sc = (u16 < thresh) ? 0.0f : p.drop_scale;
                     if (u16 < thresh) kept &= ~(1u << k);
                     a[k] *= sc;

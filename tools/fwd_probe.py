@@ -1,10 +1,6 @@
 """Development: time the fused rollout forward at C3 size and list its kernels (torch profiler)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-if "--dev" in sys.argv:            # the -DMSW_DEV_KNOBS build (tools/convgn_ablation.py builds it): MSW_CONV_PAIR / MSW_CONV_DBG apply
-    sys.argv.remove("--dev")
-    from minesweeper_ppo_b200 import _lib
-    _lib.LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_dev", "libmsw_b200_dev.so")
 import torch
 import minesweeper_ppo_b200 as m
 from minesweeper_ppo_b200.fused_forward import FusedRolloutForward
