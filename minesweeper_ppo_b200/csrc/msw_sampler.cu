@@ -99,11 +99,15 @@ masked_sample_kernel(const T *__restrict__ logits, uint8_t *__restrict__ mask, l
     // `epoch` (device counter, nullable) lets a captured CUDA graph draw fresh numbers on every replay
     const uint32_t hi = step_hi + (epoch ? *epoch : 0u);
     philox4x32_10(k0, k1 ^ 0x53414d50u, (uint32_t)rid, (uint32_t)(rid >> 32), step_lo, hi, w);
-    const float u = ((float)(w[0] >> 8) + 0.5f) * (1.0f / 16777216.0f);   // (0,1), 24 bits
+    // (0, 1], 24 bits: once w0 >> 8 >= 2^23 the half is lost to rounding, so w0 >> 8 == 0xFFFFFF gives exactly 1
+    const float u = ((float)(w[0] >> 8) + 0.5f) * (1.0f / 16777216.0f);
     const float target = u * total;
 
-    // first lane whose running total exceeds the target; rounding can leave none -> last non-empty lane
-    const unsigned over = __ballot_sync(FULL, incl > target);
+    // first lane with mass whose running total exceeds the target.  The float32 scan is not monotone across lanes:
+    // an empty lane's `incl` can round one ulp above the lanes before it (or above `total`), and a target in that
+    // gap must not land there -- its first cell is masked, or past the row when 32 does not divide A.
+    // Rounding can leave no such lane (u == 1 among them) -> last non-empty lane.
+    const unsigned over = __ballot_sync(FULL, incl > target && s > 0.0f);
     const unsigned nonempty = __ballot_sync(FULL, s > 0.0f);
     const int owner = over ? (__ffs(over) - 1) : (31 - __clz(nonempty | 1u));
     int action = 0;
