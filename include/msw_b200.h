@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define MSW_VERSION 1
+#define MSW_VERSION 2
 #define MSW_OBS_CHANNELS 10        /* env.py:79-85: revealed + one-hot counts 0..8 */
 #define MSW_MAX_CELLS 1024
 
@@ -343,15 +343,11 @@ int msw_conv3x3(const void *x16, const void *w_taps16, void *y16, int64_t n, int
  * KB (the pixel-major NHWC order costs one line per lane); only this function reads or writes that stream.
  * pool4 (nullable, with res32, instead of y32): fp32 [n][Q][C] partial sums of the fp32 output -- Q = 4 row
  * quarters (C = 96) or 8 = 2 tiles x 4 row quarters (C = 128) -- whose sum over Q / 256 is the
- * AdaptiveAvgPool2d(1) of the value head (cnn_residual.py:65).
- * max_ctas: 0 = one persistent CTA per SM; k > 0 caps the grid (C = 128: rounded down to an even count, one
- * 2-CTA cluster per board at a time) so that two launches on different streams can
- * share the GPU (FusedRolloutForward overlaps an HBM-bound residual layer with an MMA-bound one that way). */
+ * AdaptiveAvgPool2d(1) of the value head (cnn_residual.py:65). */
 int msw_conv3x3_gn(const void *x16, const void *w_taps16, const float *conv_bias, const float *res32,
                    const float *gamma, const float *beta, void *y16, float *y32, float *pool4, int64_t n,
                    int32_t H, int32_t W, int32_t Cin, int32_t C, int32_t G, float eps, float drop_p,
-                   uint64_t seed, uint64_t call_id, const uint32_t *epoch, int64_t sample_id_base, int32_t max_ctas,
-                   void *stream);
+                   uint64_t seed, uint64_t call_id, const uint32_t *epoch, int64_t sample_id_base, void *stream);
 
 /* The whole rollout forward of the three-convolution baseline policy (policy.CNNPolicy, build_model("cnn"):
  * conv 3x3 -> ReLU -> GroupNorm(4, 32) -> conv 3x3 -> ReLU -> GroupNorm(8, 64) -> conv 3x3 -> ReLU, then the 1x1

@@ -47,20 +47,6 @@ def is_stale() -> bool:
     return any(os.path.getmtime(d) > t for d in _deps())
 
 
-def build_dev(out_path: str) -> str:
-    """Development build for tools/ only: the same sources with -DMSW_DEV_KNOBS (launch-shape sweeps), written to
-    `out_path` -- never to the product library's path."""
-    srcs = [os.path.join(CSRC, s) for s in SOURCES]
-    cmd = [_nvcc(), *[f for f in NVCC_FLAGS if f not in ("-Xptxas", "-v")], "-DMSW_DEV_KNOBS", "-I", INCLUDE, "-o", out_path, *srcs]
-    env = dict(os.environ)
-    env.pop("CC", None), env.pop("CXX", None)
-    r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, env=env)
-    if r.returncode != 0:
-        print(r.stdout)
-        raise RuntimeError(f"nvcc failed ({r.returncode})")
-    return out_path
-
-
 def build(force: bool = False, verbose: bool = False) -> str:
     if not force and not is_stale():
         return LIB

@@ -4,11 +4,8 @@
 #include "msw_error.h"
 #include "msw_sm100.cuh"
 
-#include <execinfo.h>
-#include <signal.h>
 #include <stdarg.h>
 #include <stdio.h>
-#include <unistd.h>
 
 namespace msw {
 
@@ -83,16 +80,3 @@ extern "C" int msw_words_per_board(int32_t H, int32_t W)
     if (H < 1 || W < 1 || W > 32 || (long long)H * W > MSW_MAX_CELLS) return 0;
     return (H * W + 31) / 32;
 }
-
-// Development aid (not part of the ABI in include/msw_b200.h): print a native backtrace on SIGSEGV.
-static void msw_segv_handler(int sig)
-{
-    void *frames[64];
-    const int n = backtrace(frames, 64);
-    const char msg[] = "\n[msw] SIGSEGV, native backtrace:\n";
-    if (write(2, msg, sizeof(msg) - 1) < 0) {}
-    backtrace_symbols_fd(frames, n, 2);
-    signal(sig, SIG_DFL);
-    raise(sig);
-}
-extern "C" void msw_debug_segv_backtrace(void) { signal(SIGSEGV, msw_segv_handler); }

@@ -583,18 +583,17 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_con
 
 // Launch of either family with the kernel for <GN, stem, EPI>: conv3x3_tc_kernel (C = 96, one CTA per board) or, for
 // `pair`, conv3x3_pair_kernel (C = 128) in clusters of 2, one board per cluster at a time, at most one cluster per two
-// SMs (the grid cap is rounded down to whole pairs).
+// SMs.
 template <bool GN, bool STEM, int EPI>
 static int conv_launch_t(bool pair, const CUtensorMap &ma0, const CUtensorMap &ma1, const CUtensorMap &mw0, const CUtensorMap &mw1,
-                         void *y16, int64_t n, const msw::ConvGnParams &gp, int max_ctas, cudaStream_t stream)
+                         void *y16, int64_t n, const msw::ConvGnParams &gp, cudaStream_t stream)
 {
     using namespace msw;
     constexpr int CIN96 = STEM ? 16 : 96, CIN128 = STEM ? 16 : 128;
     const unsigned smem = pair ? cvp::Cfg<CIN128>::SMEM_BYTES : cv::Cfg<CIN96>::SMEM_BYTES;
     if (pair) MSW_SET_MAX_SMEM((conv3x3_pair_kernel<GN, CIN128, EPI>), smem);
     else MSW_SET_MAX_SMEM((conv3x3_tc_kernel<GN, CIN96, EPI>), smem);
-    int sms = sm_count();
-    if (max_ctas > 0 && max_ctas < sms) sms = max_ctas;             // caller shares the GPU with a concurrent launch
+    const int sms = sm_count();
     // persistent: whole boards per CTA (per CTA pair)
     const long long units_max = pair ? (sms / 2 > 0 ? sms / 2 : 1) : sms;
     const long long units = n < units_max ? n : units_max;
@@ -619,7 +618,7 @@ static int conv_launch_t(bool pair, const CUtensorMap &ma0, const CUtensorMap &m
 // Shared host side of msw_conv3x3 / msw_conv3x3_gn: argument checks, the four tensor maps, the launch.
 // C = 96 (Cin 96 or 16): conv3x3_tc_kernel, one CTA per board; C = 128 (Cin 128 or 16): conv3x3_pair_kernel.
 static int conv_launch(const char *who, const void *x16, const void *w_taps16, void *y16, int64_t n, int32_t H, int32_t W,
-                       int32_t Cin, int32_t C, const msw::ConvGnParams *gn, int max_ctas, void *stream)
+                       int32_t Cin, int32_t C, const msw::ConvGnParams *gn, void *stream)
 {
     using namespace msw;
     if (!x16 || !w_taps16 || !y16) return fail(MSW_ERR_NULL, "%s: NULL pointer", who);
@@ -667,25 +666,24 @@ static int conv_launch(const char *who, const void *x16, const void *w_taps16, v
     const ConvGnParams &gp = gn ? *gn : none;
     const bool stem = Cin == 16;
     cudaStream_t st = (cudaStream_t)stream;
-    if (!gn) return stem ? conv_launch_t<false, true, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st)
-                         : conv_launch_t<false, false, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
-    if (stem) return conv_launch_t<true, true, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);      // the stem has no residual
-    if (!gp.res32) return conv_launch_t<true, false, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
-    return gp.pool4 ? conv_launch_t<true, false, 2>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st)
-                    : conv_launch_t<true, false, 1>(pair, ma0, ma1, mw0, mw1, y16, n, gp, max_ctas, st);
+    if (!gn) return stem ? conv_launch_t<false, true, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, st)
+                         : conv_launch_t<false, false, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, st);
+    if (stem) return conv_launch_t<true, true, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, st);      // the stem has no residual
+    if (!gp.res32) return conv_launch_t<true, false, 0>(pair, ma0, ma1, mw0, mw1, y16, n, gp, st);
+    return gp.pool4 ? conv_launch_t<true, false, 2>(pair, ma0, ma1, mw0, mw1, y16, n, gp, st)
+                    : conv_launch_t<true, false, 1>(pair, ma0, ma1, mw0, mw1, y16, n, gp, st);
 }
 
 extern "C" int msw_conv3x3(const void *x16, const void *w_taps16, void *y16, int64_t n, int32_t H, int32_t W,
                            int32_t Cin, int32_t C, void *stream)
 {
-    return conv_launch("msw_conv3x3", x16, w_taps16, y16, n, H, W, Cin, C, nullptr, 0, stream);
+    return conv_launch("msw_conv3x3", x16, w_taps16, y16, n, H, W, Cin, C, nullptr, stream);
 }
 
 extern "C" int msw_conv3x3_gn(const void *x16, const void *w_taps16, const float *conv_bias, const float *res32,
                               const float *gamma, const float *beta, void *y16, float *y32, float *pool4, int64_t n,
                               int32_t H, int32_t W, int32_t Cin, int32_t C, int32_t G, float eps, float drop_p,
-                              uint64_t seed, uint64_t call_id, const uint32_t *epoch, int64_t sample_id_base, int32_t max_ctas,
-                              void *stream)
+                              uint64_t seed, uint64_t call_id, const uint32_t *epoch, int64_t sample_id_base, void *stream)
 {
     using namespace msw;
     if (!conv_bias || !gamma || !beta) return fail(MSW_ERR_NULL, "msw_conv3x3_gn: NULL pointer");
@@ -704,5 +702,5 @@ extern "C" int msw_conv3x3_gn(const void *x16, const void *w_taps16, const float
     g.call_lo = (uint32_t)call_id; g.call_hi = (uint32_t)(call_id >> 32);
     g.epoch = epoch;
     g.sample_base = (long long)sample_id_base;
-    return conv_launch("msw_conv3x3_gn", x16, w_taps16, y16, n, H, W, Cin, C, &g, max_ctas, stream);
+    return conv_launch("msw_conv3x3_gn", x16, w_taps16, y16, n, H, W, Cin, C, &g, stream);
 }

@@ -16,7 +16,6 @@
 
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 #include <string.h>
 
 
@@ -891,31 +890,10 @@ static int set_encode_out(EnvParams &p, const msw_encode_out *out, bool require)
 // boards-per-warp rather than from the SM count:
 //   CTA = one warp (a slow board -- a deep flood fill, a board draw -- never holds other warps' slots),
 //   3 boards per warp with the next board's state prefetched (80 registers).
-// Sweeps: profiles/r01_sweep_launch_shape.txt, profiles/r01_sweep_*.txt.  The product library has ONE
-// shape; building with -DMSW_DEV_KNOBS (tools/ only) lets MSW_BLOCK / MSW_BPW override it for sweeps.
-struct LaunchShape { int block, bpw; };
+// Sweeps: profiles/r01_sweep_launch_shape.txt, profiles/r01_sweep_*.txt, profiles/r02ao_bpw_taper_sweep.txt.
+constexpr int ENV_BPW = 3;
 
-static inline LaunchShape launch_shape_cfg()
-{
-#ifdef MSW_DEV_KNOBS
-    static const LaunchShape c = [] {                 // initialised once, thread-safe (C++11 static init)
-        auto env_int = [](const char *name, int dflt) { const char *e = getenv(name); return e ? atoi(e) : dflt; };
-        LaunchShape v;
-        int blk = env_int("MSW_BLOCK", 32);
-        if (blk < 32) blk = 32;
-        if (blk > 256) blk = 256;
-        v.block = blk & ~31;
-        v.bpw = env_int("MSW_BPW", 3);
-        if (v.bpw < 1) v.bpw = 1;
-        return v;
-    }();
-    return c;
-#else
-    return LaunchShape{32, 3};
-#endif
-}
-
-// Fills the three launch segments of `q` and returns the grid.  Most warps walk `bpw` boards (next board's state
+// Fills the three launch segments of `q` and returns the grid of one-warp CTAs.  Most warps walk 3 boards (next board's state
 // prefetched); CTAs are handed out in index order, so the LAST CTAs get two boards, then one: when the grid runs
 // out of CTAs the SMs otherwise drain over a whole 3-board CTA lifetime (~18 us of a 110 us launch at C2) with
 // falling occupancy; tapered, they drain over one board time.  Fluid picture: with S resident warps, S/3 of the
@@ -923,28 +901,20 @@ static inline LaunchShape launch_shape_cfg()
 // one board time before the end; board times vary, and twice that share measured best
 // (profiles/r02an_taper_sweep.txt, C2 kernel: no taper 109.8 us, 1x 107.7, 1.5x 106.9, 2x 106.7, 3x 107.3 us =
 // 6.27 -> 6.45 TB/s; C4, a 1.7 ms launch: 1710 -> 1705 us).
-static inline int grid_for(EnvParams &q, int resident_warps_per_sm, int *block_out)
+static inline int grid_for(EnvParams &q, int resident_warps_per_sm)
 {
-    const LaunchShape c = launch_shape_cfg();
-    const int wpc = c.block / 32;
-    *block_out = c.block;
     const long long n = q.n;
-    long long taper_pct = 200;
-#ifdef MSW_DEV_KNOBS
-    if (const char *e = getenv("MSW_TAPER_PCT")) taper_pct = atoll(e);
-#endif
     const long long S = (long long)sm_count() * resident_warps_per_sm;
     long long n2 = 0, n1 = 0;                           // boards handled by 2-board and by 1-board warps
-    if (c.bpw >= 3 && n >= 8 * S && taper_pct > 0) {      // from eight waves on (measured at 18 and 148 waves)
-        n1 = S / 3 * taper_pct / 100;
+    if (n >= 8 * S) {                                   // from eight waves on (measured at 18 and 148 waves)
+        n1 = S / ENV_BPW * 2;
         n2 = 2 * n1;
     }
     q.seg_na = n - n2 - n1;
-    q.seg_wa = (q.seg_na + c.bpw - 1) / c.bpw;
+    q.seg_wa = (q.seg_na + ENV_BPW - 1) / ENV_BPW;
     q.seg_nb = q.seg_na + n2;
     q.seg_wb = (n2 + 1) / 2;
-    const long long warps = q.seg_wa + q.seg_wb + n1;
-    long long blocks = (warps + wpc - 1) / wpc;
+    long long blocks = q.seg_wa + q.seg_wb + n1;       // one warp per CTA
     if (blocks < 1) blocks = 1;
     if (blocks > 0x7fffffffLL) blocks = 0x7fffffffLL;
     return (int)blocks;
@@ -953,12 +923,12 @@ static inline int grid_for(EnvParams &q, int resident_warps_per_sm, int *block_o
 // Step launches use the next-board-prefetch instantiation (80 registers); reset / encode the plain one.
 // (Prefetch at 64 registers, no prefetch at 64 and at 48 registers were measured slower and dropped.)
 template <int MODE, int CW, int CHW>
-static void launch_shape(const EnvParams &p, int grid, int block, cudaStream_t s)
+static void launch_shape(const EnvParams &p, int grid, cudaStream_t s)
 {
     if (MODE != MODE_STEP)
-        env_kernel<MODE, CW, CHW, false, 4><<<grid, block, 0, s>>>(p);
+        env_kernel<MODE, CW, CHW, false, 4><<<grid, 32, 0, s>>>(p);
     else
-        env_kernel<MODE, CW, CHW, true, 3><<<grid, block, 0, s>>>(p);
+        env_kernel<MODE, CW, CHW, true, 3><<<grid, 32, 0, s>>>(p);
 }
 
 template <int MODE>
@@ -966,16 +936,15 @@ static int launch_env(const EnvParams &p_in, cudaStream_t s)
 {
     if (p_in.n == 0) return MSW_OK;
     EnvParams p = p_in;
-    int block = 256;
-    const int grid = grid_for(p, MODE == MODE_STEP ? 24 : 32, &block);     // 80 / 64 registers: 24 / 32 one-warp CTAs per SM
+    const int grid = grid_for(p, MODE == MODE_STEP ? 24 : 32);     // 80 / 64 registers: 24 / 32 one-warp CTAs per SM
     if (p.W == 16 && p.HW == 256)
-        launch_shape<MODE, 16, 256>(p, grid, block, s);       // BASELINE configs 1-3, 5
+        launch_shape<MODE, 16, 256>(p, grid, s);       // BASELINE configs 1-3, 5
     else if (p.W == 30 && p.HW == 480)
-        launch_shape<MODE, 30, 480>(p, grid, block, s);       // BASELINE config 4 (Expert, H=16 W=30)
+        launch_shape<MODE, 30, 480>(p, grid, s);       // BASELINE config 4 (Expert, H=16 W=30)
     else if (p.W == 16 && p.HW == 480)
-        launch_shape<MODE, 16, 480>(p, grid, block, s);       // Expert transposed (H=30 W=16)
+        launch_shape<MODE, 16, 480>(p, grid, s);       // Expert transposed (H=30 W=16)
     else
-        launch_shape<MODE, 0, 0>(p, grid, block, s);
+        launch_shape<MODE, 0, 0>(p, grid, s);
     MSW_CUDA_TRY(cudaGetLastError());
     return MSW_OK;
 }

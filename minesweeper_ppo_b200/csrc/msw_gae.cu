@@ -26,16 +26,17 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 namespace msw {
 
 constexpr int GAE_TC = 128;     // time rows per shared-memory chunk
 constexpr int GAE_THREADS = 256;
+// 32 env columns per CTA (one full 128-byte line per row).  16 columns -- twice the CTAs, so every SM
+// has work at N = 8,192 -- was measured slower (18.4 vs 14.3 us, half-line requests) and removed.
+constexpr int COLS = 32;
 
-// COLS env columns per CTA (16 or 32).  Thread t loads column t % COLS of rows t / COLS,
-// t / COLS + 256 / COLS, ...; the first COLS lanes of warp 0 walk the chains.
-template <int COLS>
+// Thread t loads column t % COLS of rows t / COLS, t / COLS + 256 / COLS, ...; the first COLS lanes of warp 0
+// walk the chains.
 __global__ void __launch_bounds__(GAE_THREADS)
 gae_kernel(const float *__restrict__ rewards, const float *__restrict__ values,
            const uint8_t *__restrict__ dones, const float *__restrict__ last_values,
@@ -329,24 +330,12 @@ extern "C" int msw_gae(const float *rewards, const float *values, const uint8_t 
         return fail(MSW_ERR_NULL, "msw_gae: NULL pointer");
     if (T < 0 || N < 0) return fail(MSW_ERR_BAD_SHAPE, "msw_gae: T=%lld N=%lld", (long long)T, (long long)N);
     if (T == 0 || N == 0) return MSW_OK;
-    // 32 columns per CTA (one full 128-byte line per row).  16 columns -- twice the CTAs, so every SM
-    // has work at N = 8,192 -- was measured slower (18.4 vs 14.3 us, half-line requests) and removed.
-    const int cols = 32;
-    const long long blocks = (N + cols - 1) / cols;
+    const long long blocks = (N + COLS - 1) / COLS;
     if (blocks > 0x7fffffffLL) return fail(MSW_ERR_BAD_SHAPE, "msw_gae: N too large");
     // TMA kernel where the tensor maps can be built (16-byte aligned bases and row pitches: N % 16 == 0, N bytes
-    // for dones); the plain-load kernel serves ragged N.  One kernel per shape class, no run-time switch
-    // (-DMSW_DEV_KNOBS: MSW_GAE_TMA=0 forces the plain kernel for tools/ measurements).
-#ifdef MSW_DEV_KNOBS
-    static const bool tma_on = [] {
-        const char *e = getenv("MSW_GAE_TMA");
-        return !(e && e[0] == '0');
-    }();
-#else
-    constexpr bool tma_on = true;
-#endif
+    // for dones); the plain-load kernel serves ragged N.  One kernel per shape class, no run-time switch.
     const uintptr_t bases = (uintptr_t)rewards | (uintptr_t)values | (uintptr_t)dones | (uintptr_t)advantages | (uintptr_t)returns;
-    if (tma_on && N % 16 == 0 && (bases & 15u) == 0 && T <= 0x7fffffffLL && tensor_map_encoder_available()) {
+    if (N % 16 == 0 && (bases & 15u) == 0 && T <= 0x7fffffffLL && tensor_map_encoder_available()) {
         CUtensorMap mr, mv, md, ma, mt;
         if (!make_map(&mr, rewards, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, T, N) ||
             !make_map(&mv, values, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, T, N) ||
@@ -369,12 +358,8 @@ extern "C" int msw_gae(const float *rewards, const float *values, const uint8_t 
         MSW_CUDA_TRY(cudaGetLastError());
         return MSW_OK;
     }
-#define MSW_GAE_LAUNCH(C)                                                                           \
-    gae_kernel<C><<<(unsigned)blocks, GAE_THREADS, 0, (cudaStream_t)stream>>>(                  \
-        rewards, values, dones, last_values, advantages, returns, T, N, gamma_f32, gamma_lam_f32, \
-        (int)last_values_prescaled)
-    MSW_GAE_LAUNCH(32);
-#undef MSW_GAE_LAUNCH
+    gae_kernel<<<(unsigned)blocks, GAE_THREADS, 0, (cudaStream_t)stream>>>(
+        rewards, values, dones, last_values, advantages, returns, T, N, gamma_f32, gamma_lam_f32, (int)last_values_prescaled);
     MSW_CUDA_TRY(cudaGetLastError());
     return MSW_OK;
 }

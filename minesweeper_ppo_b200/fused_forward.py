@@ -118,8 +118,8 @@ def from_p8(t: torch.Tensor) -> torch.Tensor:
 
 def conv3x3_gn(x16: torch.Tensor, taps16: torch.Tensor, norm: torch.nn.GroupNorm, conv_bias: torch.Tensor, *,
                res32: Optional[torch.Tensor] = None, drop_p: float = 0.0, want32: bool = False, want_pool: bool = False,
-               seed: int = 0, call_id: int = 0, epoch: Optional[torch.Tensor] = None, sample_id_base: int = 0,
-               max_ctas: int = 0) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+               seed: int = 0, call_id: int = 0, epoch: Optional[torch.Tensor] = None,
+               sample_id_base: int = 0) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
     """msw_conv3x3_gn: relu(GroupNorm(conv3x3(x16) + bias) [+ res32]) [* Dropout2d] in one launch.
     `res32` and the fp32 output are in the P8 order (`to_p8`); with `want_pool` the second result is instead
     the spatial mean of the fp32 output, fp32 [N, C] (the value head's AdaptiveAvgPool2d(1))."""
@@ -144,7 +144,7 @@ def conv3x3_gn(x16: torch.Tensor, taps16: torch.Tensor, norm: torch.nn.GroupNorm
                               None if pool4 is None else pool4.data_ptr(), N, H, W, Cin, C, norm.num_groups,
                               float(norm.eps), float(drop_p), int(seed) & 0xFFFFFFFFFFFFFFFF,
                               int(call_id) & 0xFFFFFFFFFFFFFFFF, None if epoch is None else epoch.data_ptr(),
-                              int(sample_id_base), int(max_ctas), torch.cuda.current_stream(dev).cuda_stream)
+                              int(sample_id_base), torch.cuda.current_stream(dev).cuda_stream)
     _lib.check(rc, "msw_conv3x3_gn")
     if want_pool:
         return y16, pool4.sum(dim=1) * (1.0 / (H * W))
@@ -164,7 +164,7 @@ class FusedRolloutForward:
 
     _warned = set()
 
-    def __init__(self, model: CNNResidualPolicy, seed: int = 0, sample_id_base: int = 0, max_ctas: int = 0):
+    def __init__(self, model: CNNResidualPolicy, seed: int = 0, sample_id_base: int = 0):
         if not isinstance(model, CNNResidualPolicy):
             raise TypeError("FusedRolloutForward supports CNNResidualPolicy only")
         C = model.stem[0].out_channels
@@ -175,9 +175,6 @@ class FusedRolloutForward:
         self.sample_id_base = int(sample_id_base)     # global index of row 0 (env shard offset): keys the Dropout2d stream
         self.epoch: Optional[torch.Tensor] = None     # device uint32 counter mixed into the dropout RNG (graph replays)
         self.tc_trunk = (C, G) in ((96, 6), (128, 8)) and model.stem[0].in_channels <= 16 and len(model.residual_stack) >= 1
-        # grid cap of the persistent conv kernels (0 = one CTA per SM): a collector that runs two populations on two
-        # streams gives each half the SMs, so an HBM-bound residual layer of one runs beside an MMA-bound layer of the other
-        self.max_ctas = int(max_ctas)
         self._w: List = []
         self.refresh()
 
@@ -255,25 +252,25 @@ class FusedRolloutForward:
     def _trunk_tc(self, obs: torch.Tensor, cid: int):
         """tcgen05 shapes: 1 + 2 * blocks msw_conv3x3_gn launches; returns (a16 NHWC, pooled fp32 [N, C])."""
         m = self.model
-        base, max_ctas = self.sample_id_base, self.max_ctas
+        base = self.sample_id_base
         nb, cin, hh, ww = obs.shape
         x = torch.empty((nb, 16, hh, ww), dtype=torch.float16, device=obs.device, memory_format=torch.channels_last)
         with torch.cuda.device(obs.device):
             _lib.check(_lib.load().msw_pack_obs16(obs.data_ptr(), x.data_ptr(), nb, cin, hh * ww,
                                                   torch.cuda.current_stream(obs.device).cuda_stream), "msw_pack_obs16")
-        a16, a32 = conv3x3_gn(x, self.stem_taps, m.stem[1], self.stem[1], want32=True, max_ctas=max_ctas)   # stem conv + GN + ReLU
+        a16, a32 = conv3x3_gn(x, self.stem_taps, m.stem[1], self.stem[1], want32=True)   # stem conv + GN + ReLU
         last = len(self.blocks) - 1
         pooled = None
         for k, (blk, ((_, b1), (_, b2))) in enumerate(zip(m.residual_stack, self.blocks)):
             # conv1 + GroupNorm + ReLU + Dropout2d
             t16, _ = conv3x3_gn(a16, self.taps[k][0], blk.norm1, b1, drop_p=self._drop_p(blk), seed=self.seed,
-                                call_id=cid + k, epoch=self.epoch, sample_id_base=base, max_ctas=max_ctas)
+                                call_id=cid + k, epoch=self.epoch, sample_id_base=base)
             # conv2 + GroupNorm + fp32 residual add + ReLU; the last block emits the value head's average pool
             # instead of a residual stream nobody reads
             if k == last:
-                a16, pooled = conv3x3_gn(t16, self.taps[k][1], blk.norm2, b2, res32=a32, want_pool=True, max_ctas=max_ctas)
+                a16, pooled = conv3x3_gn(t16, self.taps[k][1], blk.norm2, b2, res32=a32, want_pool=True)
             else:
-                a16, a32 = conv3x3_gn(t16, self.taps[k][1], blk.norm2, b2, res32=a32, want32=True, max_ctas=max_ctas)
+                a16, a32 = conv3x3_gn(t16, self.taps[k][1], blk.norm2, b2, res32=a32, want32=True)
         return a16, pooled
 
     def _heads(self, a16: torch.Tensor, pooled: torch.Tensor, return_mine: bool):

@@ -41,7 +41,7 @@ def test_binding_arity_matches_header():
 
 
 def test_host_side_calls_without_device(lib):
-    assert lib.msw_version() == 1
+    assert lib.msw_version() == 2
     assert lib.msw_words_per_board(16, 16) == 8 and lib.msw_words_per_board(16, 30) == 15
     assert lib.msw_words_per_board(32, 32) == 32 and lib.msw_words_per_board(33, 32) == 0
     assert lib.msw_words_per_board(16, 33) == 0

@@ -236,7 +236,7 @@ def test_conv3x3_gn_c128_outputs_stay_inside_their_windows(n):
     def call(res32, y32p, poolp, drop):
         return L.msw_conv3x3_gn(x.data_ptr(), taps.data_ptr(), bias.data_ptr(), res32, norm.weight.data_ptr(),
                                 norm.bias.data_ptr(), y16.data_ptr(), y32p, poolp, n, 16, 16, C, C, 8, 1e-5, drop,
-                                1, 2, None, 0, 0, st)
+                                1, 2, None, 0, st)
 
     assert call(None, y32.data_ptr(), None, 0.2) == 0                  # EPI 0 with Dropout2d, y32 out
     assert call(res.data_ptr(), y32.data_ptr(), None, 0.0) == 0        # EPI 1
@@ -260,7 +260,7 @@ def test_conv3x3_c128_shape_errors():
 
     def gn(H, cin, G):
         return L.msw_conv3x3_gn(x.data_ptr(), taps.data_ptr(), v.data_ptr(), None, v.data_ptr(), v.data_ptr(),
-                                y.data_ptr(), None, None, n, H, 16, cin, C, G, 1e-5, 0.0, 0, 0, None, 0, 0, st)
+                                y.data_ptr(), None, None, n, H, 16, cin, C, G, 1e-5, 0.0, 0, 0, None, 0, st)
 
     assert gn(16, C, 6) == 1
     assert gn(16, 96, 8) == 1

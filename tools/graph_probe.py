@@ -4,9 +4,6 @@ import os, sys, json, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 import minesweeper_ppo_b200 as m
-if os.environ.get("MSW_SEGV"):
-    from minesweeper_ppo_b200 import _lib
-    _lib.load().msw_debug_segv_backtrace()
 
 out = {}
 for N in [int(a) for a in sys.argv[1:]] or (128, 1024, 8192):
